@@ -3,9 +3,12 @@
 
     python bench.py --gpus N --steps K --warmup W                 (this repo's CUDA path)
     python bench.py --impl reference --gpus N --steps K --warmup W  (reference math on the host cores)
+    python bench.py ... --dump-outputs DIR                          (also save what the last timed step computed)
 
 One "step" = one pass of the hot path (reference train.py:140-152) over one synthetic 128^3 crop per GPU
 with the default Model() (in 2, out 3, base_filters 16).  Prints ONE JSON line (rank 0).  See DESIGN.md §4.
+
+The benchmark writes nothing into the source tree (no bytecode caches either): the tree may be read-only.
 """
 from __future__ import annotations
 
@@ -19,6 +22,7 @@ import sys
 import threading
 import time
 
+sys.dont_write_bytecode = True
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 PKG = "3d-brain-tumor-segmentation_b200"
@@ -361,6 +365,24 @@ def measure_tta(b3d, torch, dist, dev, model, world, reps=2):
             "mode": "replicas: flips dealt to ranks + 1 all-reduce" if world > 1 else "8 sequential forwards"}
 
 
+def dump_step_outputs(out_dir, out):
+    """What a caller of the timed training step receives from its last step, as DIR/<name>.npy: the loss, macro Dice
+    and micro Dice that train_step returns.  Weights and crops are seeded (synthdata), dropout hashes a fixed seed
+    with a step counter and run_b3d seeds the generator the VAE draws eps from: runs with the same arguments see the
+    same inputs, so two builds can be compared array by array.
+    The weights the step updates are not saved: the step is not bit-reproducible (float atomics in the pooling and
+    parameter-gradient reductions change 16-bit roundings), and Adam turns the resulting noise in near-zero gradients
+    into learning-rate-sized weight differences between runs of one build.  The returned values stay close: three
+    runs of one build with --steps 20 --warmup 5 on a B200 (1000 W limit) spread by 5e-5 relative in the loss and
+    2e-3 relative in both Dice scores."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in zip(("loss", "macro_dice", "micro_dice"), out):
+        t = t.detach().cpu()
+        np.save(os.path.join(out_dir, name + ".npy"), (t.double() if t.dtype == torch.float64 else t.float()).numpy())
+
+
 def run_b3d(args):
     import torch
     import torch.distributed as dist
@@ -375,7 +397,9 @@ def run_b3d(args):
     b3d = importlib.import_module(PKG)
     import synthdata as R               # seeded synthetic weights / inputs (neutral module: nothing under oracle/)
 
-    # ---- model, synthetic data (rank r uses seed + 100 r), optimizer
+    # ---- model, synthetic data (rank r uses seed + 100 r), optimizer.  The VAE draws eps from torch's default
+    # generators inside the step, and torch seeds those at random in every process: seed them like the crops.
+    torch.manual_seed(100 * rank)
     p = R.init_params(R.param_shapes(crop=CROP), dtype=torch.float32)
     x, y, _, _ = R.synth_batch((1,) + CROP, seed=100 * rank, dtype=torch.float32)
     xh, yh = x.pin_memory(), y.pin_memory()
@@ -416,6 +440,8 @@ def run_b3d(args):
         ms = timed(lambda: step(), args.steps)
     clocks = cs.summary()
     value = world * args.steps / (ms / 1e3)
+    if args.dump_outputs and rank == 0:        # before the end-to-end pass below trains the model further
+        dump_step_outputs(args.dump_outputs, step.out)
 
     # ---- end to end through the public API: pinned host inputs -> H2D -> step -> D2H of the loss
     loss_host = torch.empty(1).pin_memory()
@@ -521,12 +547,20 @@ def run_b3d(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed steps; --impl reference times fewer when its B3D_REF_BUDGET_S budget (200 s) runs out, "
+                         "and its JSON line reports the number it timed")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="b3d", choices=["b3d", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra-configs", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, save the loss and Dice scores the last step returned as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b3d":
+        ap.error("--dump-outputs saves the CUDA path's step (--impl b3d)")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -1,11 +1,11 @@
 """ORACLE / test infrastructure.  Generates tests/golden/*.npz by EXECUTING THE REFERENCE'S OWN FILES
-(/root/reference/{model.py,layers/*.py,util.py}) on oracle/tf_shim (see oracle/run_reference.py) in fp64.
-Run in the build container (needs /root/reference):   python -m oracle.make_golden
-The GPU box has no /root/reference: tests there read the committed fixtures.
+({model.py,layers/*.py,util.py} of the original project) on oracle/tf_shim (see oracle/run_reference.py) in fp64.
+Needs a checkout of the original project at oracle/_ref/ or at $B3D_REFERENCE:   python -m oracle.make_golden
+Without one, tests read the committed fixtures.
 
 Fixtures (small on purpose; weights/inputs are regenerated from seeds by oracle.ref_model):
   model_16.npz : full model, 16^3 crop, training call (dropout mask + eps injected), loss, dice,
-                 gradients of 12 representative tensors + L2 norms of all 260 gradients
+                 gradients of 14 representative tensors (the largest one sampled) + L2 norms of all 260 gradients
   gn_cases.npz : GroupNormalization.call on odd shapes (chunk boundary mid-slice, C/G = 1, 2, 4)
 """
 from __future__ import annotations
@@ -21,12 +21,16 @@ ROOT = os.path.dirname(HERE)
 sys.path.insert(0, ROOT)
 
 from oracle import ref_model as R  # noqa: E402
-from oracle.run_reference import ReferenceRunner, _import_reference  # noqa: E402
+from oracle.run_reference import REF, ReferenceRunner, _import_reference, available  # noqa: E402
 
 GRAD_KEYS = ["enc.L0.B0.conv1.kernel", "enc.L0.B0.gn2.gamma", "enc.L0.B0.spatial.kernel",
              "enc.L1.B1.dense_relu.kernel", "enc.L2.B2.ptwise.kernel", "enc.L3.B3.conv2.kernel",
              "enc.L0.down.conv.kernel", "dec.L0.up.conv.kernel", "dec.L1.block.gn1.beta", "dec.out.kernel",
              "vae.proj.kernel", "vae.unproj.bias", "vae.L0.block.conv2.bias", "vae.out.kernel"]
+# a larger gradient is stored as every GRAD_STRIDE-th element of its flattened array (prime: the sample runs
+# through every kernel tap and channel position)
+SAMPLE_ABOVE = 1 << 16
+GRAD_STRIDE = 17
 
 
 def model_case(crop, out):
@@ -46,7 +50,12 @@ def model_case(crop, out):
          "grad_names": np.array(sorted(nv)),
          "grad_norms": np.array([float(nv[k].grad.norm()) for k in sorted(nv)])}
     for k in GRAD_KEYS:
-        d["grad:" + k] = nv[k].grad.numpy().astype(np.float32)
+        g = nv[k].grad.numpy().astype(np.float32)
+        if g.size > SAMPLE_ABOVE:          # keeps the fixture file under 1 MB; its norm is in grad_norms
+            d["grad_sample:" + k] = np.ascontiguousarray(g.reshape(-1)[::GRAD_STRIDE])
+            d["grad_stride"] = np.int64(GRAD_STRIDE)
+        else:
+            d["grad:" + k] = g
     # inference call (VAE off) on the same weights
     yi = rr.forward(x, training=False, inference=True)[0]
     d["y_pred_inference"] = yi.detach().numpy().astype(np.float32)
@@ -75,6 +84,9 @@ def gn_cases(out):
 
 
 if __name__ == "__main__":
+    if not available():
+        sys.exit(f"make_golden: no checkout of the original project at {REF} (install it at oracle/_ref/ or set "
+                 "B3D_REFERENCE to its directory)")
     g = os.path.join(ROOT, "tests", "golden")
     os.makedirs(g, exist_ok=True)
     model_case((16, 16, 16), os.path.join(g, "model_16.npz"))

@@ -1,8 +1,8 @@
 """ORACLE / test infrastructure.  Imports the reference's OWN hot-path python files
-(/root/reference/{model.py,layers/*.py,util.py}) UNMODIFIED on top of oracle/tf_shim and runs
-them on this repo's synthetic weights/inputs.  Only usable where /root/reference exists
-(the build container); the GPU box uses the fixtures this produces (tests/golden/*.npz, written
-by oracle/make_golden.py).
+({model.py,layers/*.py,util.py} of the original project) UNMODIFIED on top of oracle/tf_shim and runs
+them on this repo's synthetic weights/inputs.  Only usable where a checkout of the original project is
+installed: at oracle/_ref/ (kept out of git), or wherever the environment variable B3D_REFERENCE names;
+elsewhere tests use the fixtures this produces (tests/golden/*.npz, written by oracle/make_golden.py).
 """
 from __future__ import annotations
 
@@ -13,7 +13,7 @@ import sys
 import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF = os.environ.get("B3D_REFERENCE", "/root/reference")
+REF = os.path.abspath(os.environ.get("B3D_REFERENCE") or os.path.join(HERE, "_ref"))
 
 
 def available() -> bool:
@@ -21,6 +21,9 @@ def available() -> bool:
 
 
 def _import_reference():
+    if not available():
+        raise RuntimeError(f"no checkout of the original project at {REF} (install it at oracle/_ref/ or set "
+                           "B3D_REFERENCE to its directory)")
     shim = os.path.join(HERE, "tf_shim")
     for p in (REF, shim):
         if p not in sys.path:
@@ -35,7 +38,7 @@ def _import_reference():
     assert "tf_shim" in tf.__file__, "real TensorFlow found?  the shim must shadow it"
     ref_model = importlib.import_module("model")
     ref_util = importlib.import_module("util")
-    assert ref_model.__file__.startswith(REF), ref_model.__file__
+    assert ref_model.__file__.startswith(REF + os.sep), ref_model.__file__
     return tf, ref_model, ref_util
 
 

@@ -81,6 +81,9 @@ def test_model_matches_reference_fixture_16(b3d, dev, mode):
     for k in g.files:
         if k.startswith("grad:"):
             assert rel(nv[k[5:]].grad, g[k]) < {"fp32": 2e-3, "tf32": 2e-1, "mixed": 5e-1}[mode], (k, rel(nv[k[5:]].grad, g[k]))
+        elif k.startswith("grad_sample:"):
+            got = nv[k[12:]].grad.reshape(-1)[::int(g["grad_stride"])]
+            assert rel(got, g[k]) < {"fp32": 2e-3, "tf32": 2e-1, "mixed": 5e-1}[mode], (k, rel(got, g[k]))
     assert yi[1] is None and yi[2] is None and yi[3] is None
     assert rel(yi[0], g["y_pred_inference"]) < otol
     agree = (yi[0].argmax(-1).cpu() == torch.from_numpy(g["y_pred_inference"]).argmax(-1)).float().mean()
