@@ -82,6 +82,7 @@ SIGNATURES = {
     "b3d_gn_channel_stats": "TTiv",
     "b3d_gn_channel_apply": "TTTTTifiv",
     "b3d_gn_channel_bwd": "TTTTTTTTTifiv",
+    "b3d_gn_channel_apply_slab": "TTTTTTifiLv",
     "b3d_relayout": "TTiv",
     "b3d_gn_stats_slab": "TTiLLv",
     "b3d_gn_apply_slab": "TTTTTifiLLv",

@@ -3,8 +3,10 @@
 // group g of a sample = channels [g*cg, (g+1)*cg) of every voxel — unlike the contiguous-chunk behaviour of the
 // channels_last path (norm.cu).  Same HBM-streaming structure: every thread owns a fixed quad of channels (block size
 // is a multiple of C/4), 128-bit accesses, register accumulators -> shared memory -> one atomic per CTA and value.
-// Also the NCDHW <-> NDHWC re-layout kernels the channels_first API surface needs at the model boundary.
+// Also the depth-slab apply (whole-volume statistics, fp32 and / or P16 twin output) of sharded inference, and the
+// NCDHW <-> NDHWC re-layout kernels the channels_first API surface needs at the model boundary.
 #include "common.cuh"
+#include "twin16.cuh"
 
 namespace b3d {
 
@@ -163,6 +165,61 @@ __global__ void gnc_bwd_apply_kernel(const float* __restrict__ dy, const float* 
   }
 }
 
+// ---- depth-slab form (slab.py): one rank's slab [1, Dl, H, W, C] normalised with the statistics of the WHOLE volume
+// (the all-reduced partial sums of gnc_stats_kernel over every slab; a group holds total_voxels * C/G values) ->
+// fp32 y and / or its P16 twin.  One thread = one 16-byte twin cell (8 channels of a voxel), kSlabIter cells per pass
+// loaded before any is stored; the block is a multiple of C/8 threads and every stride a multiple of C/8 cells, so a
+// thread keeps its channel octet over the grid-stride loop and its 8 scale / shift constants are computed once.
+constexpr int kSlabIter = 4;
+constexpr int kSlabMaxThreads = 512;    // C <= 4096
+
+template <bool RELU>
+__global__ void __launch_bounds__(kSlabMaxThreads)
+    gnc_apply_slab_kernel(const float* __restrict__ x, const double* __restrict__ stats,
+                          const float* __restrict__ gamma, const float* __restrict__ beta, float* __restrict__ y,
+                          Twin16 tw, long long ncells, int cg, double inv_n, float eps) {
+  pdl_trigger();
+  pdl_wait();
+  const unsigned nt = blockDim.x;
+  const long long cell0 = (long long)blockIdx.x * (kSlabIter * nt) + threadIdx.x;
+  const int c8 = (int)(threadIdx.x % tw.C8);
+  float a[8], c[8];
+#pragma unroll
+  for (int i = 0; i < 8; ++i) {
+    const int ch = c8 * 8 + i;
+    float mean, rstd;
+    group_moments(stats, ch / cg, inv_n, eps, mean, rstd);
+    a[i] = rstd * __ldg(gamma + ch);
+    c[i] = __ldg(beta + ch) - mean * a[i];
+  }
+  const long long pass = (long long)gridDim.x * kSlabIter * nt;      // cells
+  CellPos pos = cell_pos(tw, 0u, (unsigned long long)cell0 * 8, nt, (unsigned long long)(pass - (kSlabIter - 1) * nt));
+  for (long long k0 = cell0; k0 < ncells; k0 += pass) {
+    float in[kSlabIter][8];
+#pragma unroll
+    for (int k = 0; k < kSlabIter; ++k) {
+      const long long cell = k0 + (long long)k * nt;
+      if (cell < ncells) ld8(x + cell * 8, in[k]);
+    }
+#pragma unroll
+    for (int k = 0; k < kSlabIter; ++k) {
+      const long long cell = k0 + (long long)k * nt;
+      if (cell < ncells) {
+        float o[8];
+#pragma unroll
+        for (int i = 0; i < 8; ++i) {
+          const float t = fmaf(in[k][i], a[i], c[i]);
+          o[i] = RELU ? fmaxf(t, 0.f) : t;
+        }
+        if (y != nullptr) st8(y + cell * 8, o);
+        if (tw.p != nullptr) cell_store(tw, pos, o);
+      }
+      if (k < kSlabIter - 1) cell_step(tw, pos, pos.dr1, pos.dw1);
+      else cell_step(tw, pos, pos.dr2, pos.dw2);
+    }
+  }
+}
+
 // ---- NCDHW <-> NDHWC: [B, C, S] <-> [B, S, C] through 32x32 shared-memory tiles.
 // src [B, R, Cn] -> dst [B, Cn, R]; the voxel dimension (millions) always rides on gridDim.x
 __global__ void __launch_bounds__(256) transpose_kernel(const float* __restrict__ src, float* __restrict__ dst,
@@ -285,6 +342,61 @@ extern "C" int b3d_gn_channel_bwd(const DLTensor* dy_, const DLTensor* x_, const
   if (relu) B3D_GNC(true); else B3D_GNC(false);
 #undef B3D_GNC
   B3D_LAUNCH_CHECK("gn_channel_bwd");
+  return B3D_OK;
+}
+
+// One depth slab of sharded inference (slab.py): x / y / y16 = this rank's slab [1, Dl, H, W, C] (y16: its P16 twin
+// [1, Dl, H, C/8, W, 8]); stats = the all-reduced (sum x, sum x^2) of every channel group over the whole volume of
+// total_voxels voxels (total_voxels = the slab's own voxel count: the un-sharded apply).  y and y16 are each optional,
+// not both.
+extern "C" int b3d_gn_channel_apply_slab(const DLTensor* x_, const DLTensor* stats_, const DLTensor* gamma_,
+                                         const DLTensor* beta_, DLTensor* y_, DLTensor* y16_, int groups, float eps,
+                                         int relu, long long total_voxels, void* stream) {
+  TView x, y, st, ga, be;
+  B3D_TRY(view(x_, DT_F32, 5, false, "x", &x));
+  B3D_REQUIRE(x.shape[0] == 1, B3D_ERR_SHAPE, "gn_channel_apply (slab): batch 1");
+  B3D_REQUIRE(y_ != nullptr || y16_ != nullptr, B3D_ERR_ARG, "gn_channel_apply (slab): neither y nor y16 given");
+  const int C = (int)x.shape[4];
+  B3D_REQUIRE(groups >= 1 && C >= groups, B3D_ERR_SHAPE,
+              "Number of groups (%d) cannot be more than the number of channels (%d).", groups, C);
+  B3D_REQUIRE(C % groups == 0, B3D_ERR_SHAPE,
+              "Number of groups (%d) must be a multiple of the number of channels (%d).", groups, C);
+  B3D_REQUIRE(C % 8 == 0 && C / 8 <= kSlabMaxThreads && ((uintptr_t)x.p & 15) == 0, B3D_ERR_UNSUPPORTED,
+              "gn_channel_apply (slab): channels must be a multiple of 8, at most %d (C=%d)", 8 * kSlabMaxThreads, C);
+  const long long S = x.numel / C, ncells = x.numel / 8;
+  B3D_REQUIRE(S > 0 && total_voxels >= S, B3D_ERR_ARG,
+              "gn_channel_apply (slab): total_voxels (%lld) below the slab's %lld voxels", total_voxels, S);
+  B3D_REQUIRE(ncells < (1LL << 32), B3D_ERR_UNSUPPORTED, "gn_channel_apply (slab): slab too large");
+  y.p = nullptr;
+  if (y_ != nullptr) {
+    B3D_TRY(view(y_, DT_F32, -1, false, "y", &y));
+    B3D_REQUIRE(x.numel == y.numel && ((uintptr_t)y.p & 15) == 0, B3D_ERR_SHAPE,
+                "gn_channel_apply (slab): x/y size mismatch");
+  }
+  B3D_TRY(vecn(stats_, DT_F64, 2LL * groups, "stats", &st));
+  B3D_TRY(vecn(gamma_, DT_F32, C, "gamma", &ga));
+  B3D_TRY(vecn(beta_, DT_F32, C, "beta", &be));
+  // the cell position is advanced for y-only calls too, so its geometry is that of x
+  Twin16 tw;
+  tw.p = nullptr; tw.p2 = nullptr; tw.bf16 = 0;
+  tw.W = (unsigned)x.shape[3]; tw.C8 = (unsigned)(C / 8); tw.rows = (unsigned)(x.shape[1] * x.shape[2]);
+  if (y16_ != nullptr) B3D_TRY(twin_view(y16_, nullptr, x, &tw));
+  const int q = C / 8;
+  const int threads = q >= 256 ? q : (256 / q) * q;
+  long long blocks = (ncells + (long long)threads * kSlabIter - 1) / ((long long)threads * kSlabIter);
+  const long long cap = 8LL * sm_count();
+  if (blocks > cap) blocks = cap;
+  const double inv_n = 1.0 / ((double)total_voxels * (C / groups));
+  cudaStream_t s = (cudaStream_t)stream;
+  if (relu)
+    launch_pdl(gnc_apply_slab_kernel<true>, dim3((unsigned)blocks), threads, 0, s, (const float*)x.p,
+               (const double*)st.p, (const float*)ga.p, (const float*)be.p, (float*)y.p, tw, ncells, C / groups, inv_n,
+               eps);
+  else
+    launch_pdl(gnc_apply_slab_kernel<false>, dim3((unsigned)blocks), threads, 0, s, (const float*)x.p,
+               (const double*)st.p, (const float*)ga.p, (const float*)be.p, (float*)y.p, tw, ncells, C / groups, inv_n,
+               eps);
+  B3D_LAUNCH_CHECK("gn_channel_apply (slab)");
   return B3D_OK;
 }
 

@@ -882,8 +882,8 @@ class GroupNormChannelFn(Function):
 def group_norm(x, gamma, beta, stats=None, groups=8, eps=1e-5, relu=False, channel_mode=False, operand_only=False):
     ctx = _slab.current()
     if channel_mode:
-        if ctx is not None:
-            raise NotImplementedError("b3d: depth-slab inference is built for the channels_last GroupNorm semantics")
+        if ctx is not None:    # channel-group statistics of the WHOLE volume: partial sums + all-reduce
+            return ctx.group_norm_channel(x, gamma, beta, groups, eps, relu, operand_only)
         return GroupNormChannelFn.apply(x, gamma, beta, groups, eps, relu)
     if ctx is not None:        # chunk statistics of the WHOLE volume: partial sums + all-reduce
         return ctx.group_norm(x, gamma, beta, groups, eps, relu, stats, operand_only)

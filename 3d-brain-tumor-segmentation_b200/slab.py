@@ -12,6 +12,10 @@ its slab while a `SlabContext` reroutes the three operations whose result depend
   * GroupNormalization (group_norm.py:83-124): its "groups" are contiguous 1/G chunks of the WHOLE flat volume
       (SURVEY F1) and do not line up with slabs => every rank reduces partial (sum, sum^2) per global chunk
       (`b3d_gn_stats_slab`), one all-reduce of 2*G doubles, then `b3d_gn_apply_slab`.
+      A channels_first model's groups are true channel groups (a fixed set of channels over every voxel of the
+      volume): the slab's own `b3d_gn_channel_stats` are the partial sums, all-reduced the same way, then
+      `b3d_gn_channel_apply_slab`.  Such a model takes and returns NCDHW tensors, so the drivers below cut and
+      gather along dim 2 instead of dim 1.
   * channel squeeze-excitation (resnet.py:45-58): the global-average-pool sums from the pointwise conv's epilogue
       are all-reduced (F floats) and divided by the global voxel count.
 
@@ -66,9 +70,14 @@ class Comm:
         self.all_reduce_sum(a)
         self.all_reduce_sum(b)
 
-    def all_gather_cat(self, t: torch.Tensor, sizes: Sequence[int]) -> torch.Tensor:
-        """Concatenate the ranks' tensors (dim 1 extents `sizes`) on every rank."""
+    def all_gather_cat(self, t: torch.Tensor, sizes: Sequence[int], dim: int = 1) -> torch.Tensor:
+        """Concatenate the ranks' tensors (extents `sizes` along `dim`) on every rank."""
         raise NotImplementedError
+
+
+def _gather_parts(t: torch.Tensor, sizes: Sequence[int], dim: int) -> List[torch.Tensor]:
+    return [torch.empty(tuple(t.shape[:dim]) + (n,) + tuple(t.shape[dim + 1:]), dtype=t.dtype, device=t.device)
+            for n in sizes]
 
 
 class DistComm(Comm):
@@ -98,12 +107,12 @@ class DistComm(Comm):
         if self.world > 1:
             self.dist.all_reduce(t, op=self.dist.ReduceOp.SUM, group=self.group)
 
-    def all_gather_cat(self, t, sizes):
+    def all_gather_cat(self, t, sizes, dim=1):
         if self.world == 1:
             return t
-        parts = [torch.empty((t.shape[0], n) + tuple(t.shape[2:]), dtype=t.dtype, device=t.device) for n in sizes]
+        parts = _gather_parts(t, sizes, dim)
         self.dist.all_gather(parts, t.contiguous(), group=self.group)
-        return torch.cat(parts, dim=1)
+        return torch.cat(parts, dim=dim)
 
 
 class PeerComm(Comm):
@@ -166,12 +175,12 @@ class PeerComm(Comm):
         ops._call("b3d_peer_allreduce2", a, b, self.peers, self.rank, self.sym, self.epoch, self.aseq)
         self.aseq += 1
 
-    def all_gather_cat(self, t, sizes):
+    def all_gather_cat(self, t, sizes, dim=1):
         if self.world == 1:
             return t
-        parts = [torch.empty((t.shape[0], n) + tuple(t.shape[2:]), dtype=t.dtype, device=t.device) for n in sizes]
+        parts = _gather_parts(t, sizes, dim)
         self.dist.all_gather(parts, t.contiguous(), group=self.group)
-        return torch.cat(parts, dim=1)
+        return torch.cat(parts, dim=dim)
 
 
 class _ThreadShared:
@@ -213,11 +222,11 @@ class ThreadComm(Comm):
         sh.barrier.wait()
         t.copy_(total)
 
-    def all_gather_cat(self, t, sizes):
+    def all_gather_cat(self, t, sizes, dim=1):
         sh = self.sh
         sh.slots[self.rank] = t
         sh.barrier.wait()
-        out = torch.cat([sh.slots[r] for r in range(self.world)], dim=1)
+        out = torch.cat([sh.slots[r] for r in range(self.world)], dim=dim)
         sh.barrier.wait()
         return out
 
@@ -523,8 +532,37 @@ class SlabContext:
         ops._call("b3d_gn_apply_slab", x, stats, gamma, beta, y, groups, float(eps), int(relu), off, total)
         return y
 
+    def group_norm_channel(self, x, gamma, beta, groups, eps, relu, operand_only=False):
+        """GroupNormalization with true channel groups (channels_first models; ops.group_norm routes here): the
+        slab's channel-group sums are partial sums of the whole volume's, all-reduced in the next flush together
+        with the pointwise conv's pending pooling sums; outputs as in `group_norm`."""
+        from . import ops
+        x = ops.materialize(x)
+        ops._check(x)
+        stats = torch.empty((1, groups, 2), dtype=torch.float64, device=x.device)
+        ops._call("b3d_gn_channel_stats", x, stats, groups)     # raises the reference's ValueError on bad groups
+        self._pending.append(stats)
+        self.flush()
+        nvox = self.global_voxels(x)
+        if self.p16 is not None and ops.p16_ok(x.shape):
+            y16 = self.new_p16(x.shape, x)
+            y = None if operand_only else torch.empty_like(x)
+            ops._call("b3d_gn_channel_apply_slab", x, stats, gamma, beta, y, y16, groups, float(eps), int(relu), nvox)
+            if y is None:
+                return ops.virtual(x.shape, x, [y16], None)
+            ops._attach(y, y16, None)
+            return y
+        y = self.new_activation(x.shape, x)
+        ops._call("b3d_gn_channel_apply_slab", x, stats, gamma, beta, y, None, groups, float(eps), int(relu), nvox)
+        return y
+
 
 # ------------------------------------------------------------------------------------------ drivers
+def depth_axis(model) -> int:
+    """Dimension of the depth axis in the model's public tensors: 2 for a channels_first model (NCDHW), else 1."""
+    return 2 if getattr(model, "data_format", "channels_last") == "channels_first" else 1
+
+
 def slab_forward(model, x_local: torch.Tensor, ctx: SlabContext) -> torch.Tensor:
     """This rank's slab of `model(x, training=False, inference=True)[0]` (test.py:133)."""
     with torch.no_grad(), ctx:
@@ -532,15 +570,17 @@ def slab_forward(model, x_local: torch.Tensor, ctx: SlabContext) -> torch.Tensor
 
 
 def sharded_inference(model, x: torch.Tensor, comm: Comm, gather: bool = True, align: Optional[int] = None):
-    """x: the WHOLE padded volume [1, D, H, W, C] (every rank holds it, as after loading a case from disk);
-    each rank computes its depth slab; returns the whole prediction (gather=True) or (slab, (d0, d1))."""
+    """x: the WHOLE padded volume [1, D, H, W, C] ([1, C, D, H, W] for a channels_first model; every rank holds it,
+    as after loading a case from disk); each rank computes its depth slab; returns the whole prediction
+    (gather=True) or (slab, (d0, d1)), in the layout of x."""
     if align is None:
         align = 2 ** (len(model.encoder.levels) - 1)
-    ctx = SlabContext(comm, x.shape[1], align=align)
-    y = slab_forward(model, x[:, ctx.d0:ctx.d1].contiguous(), ctx)
+    ax = depth_axis(model)
+    ctx = SlabContext(comm, x.shape[ax], align=align)
+    y = slab_forward(model, x.narrow(ax, ctx.d0, ctx.local_depth).contiguous(), ctx)
     if not gather:
         return y, (ctx.d0, ctx.d1)
-    return comm.all_gather_cat(y, [b - a for a, b in ctx.bounds])
+    return comm.all_gather_cat(y, [b - a for a, b in ctx.bounds], dim=ax)
 
 
 class GraphedInference:
@@ -555,8 +595,9 @@ class GraphedInference:
         self.ctx = None
         if comm is not None:
             align = 2 ** (len(model.encoder.levels) - 1)
-            self.ctx = SlabContext(comm, depth if depth is not None else x_example.shape[1] * comm.world, align=align)
-            if self.ctx.local_depth != self.x.shape[1]:
+            ax = depth_axis(model)
+            self.ctx = SlabContext(comm, depth if depth is not None else x_example.shape[ax] * comm.world, align=align)
+            if self.ctx.local_depth != self.x.shape[ax]:
                 raise ValueError("GraphedInference: x_example must be this rank's slab")
         s = torch.cuda.Stream()
         s.wait_stream(torch.cuda.current_stream())
@@ -588,15 +629,16 @@ def run_virtual_ranks(model, x: torch.Tensor, world: int, align: Optional[int] =
     comms = ThreadComm.make(world)
     if align is None:
         align = 2 ** (len(model.encoder.levels) - 1)
-    bounds = slab_bounds(x.shape[1], world, align)
+    ax = depth_axis(model)
+    bounds = slab_bounds(x.shape[ax], world, align)
     outs, stats, errs = [None] * world, [None] * world, []
 
     def work(r):
         try:
             if x.is_cuda:
                 torch.cuda.set_device(x.device)
-            ctx = SlabContext(comms[r], x.shape[1], bounds)
-            outs[r] = slab_forward(model, x[:, bounds[r][0]:bounds[r][1]].contiguous(), ctx)
+            ctx = SlabContext(comms[r], x.shape[ax], bounds)
+            outs[r] = slab_forward(model, x.narrow(ax, bounds[r][0], bounds[r][1] - bounds[r][0]).contiguous(), ctx)
             stats[r] = ctx.stats
         except BaseException as e:     # noqa: BLE001 — release the other ranks, then re-raise in the caller
             errs.append(e)
@@ -610,4 +652,4 @@ def run_virtual_ranks(model, x: torch.Tensor, world: int, align: Optional[int] =
     if errs:
         real = [e for e in errs if not isinstance(e, threading.BrokenBarrierError)]
         raise (real or errs)[0]
-    return torch.cat(outs, dim=1), stats
+    return torch.cat(outs, dim=ax), stats

@@ -141,6 +141,12 @@ int b3d_gn_channel_apply(const DLTensor* x, const DLTensor* stats, const DLTenso
 int b3d_gn_channel_bwd(const DLTensor* dy, const DLTensor* x, const DLTensor* stats, const DLTensor* gamma,
                        const DLTensor* beta, DLTensor* dgamma, DLTensor* dbeta, DLTensor* csum, DLTensor* dx,
                        int groups, float eps, int relu, void* stream);
+/* Depth-slab form (sharded inference, slab.py): x = one slab [1, Dl, H, W, C]; stats fp64 [1, G, 2] = the all-reduced
+ * sums of every group over the whole volume of total_voxels voxels (the slabs' gn_channel_stats added up).  Writes the
+ * fp32 y and / or the P16 twin y16 [1, Dl, H, C/8, W, 8] (fp16 or bf16); each is nullable, not both.  C % 8 == 0. */
+int b3d_gn_channel_apply_slab(const DLTensor* x, const DLTensor* stats, const DLTensor* gamma, const DLTensor* beta,
+                              DLTensor* y, DLTensor* y16, int groups, float eps, int relu, long long total_voxels,
+                              void* stream);
 int b3d_relayout(const DLTensor* src, DLTensor* dst, int to_channels_last, void* stream);
 
 /* ---- ResnetBlock epilogue (resnet.py:121-137) --------------------------------------------------
