@@ -992,8 +992,8 @@ static int pad_cin(const ConvGeom& g) {
 }
 static int pad_cout(int c) { return (c + 15) / 16 * 16; }
 
-// kd-folded variant of the 3x3x3 kernel (TcCfg::FOLD): narrow output tiles with 16-bit operands.  Off by default
-// until it has been validated and timed on hardware (b3d_set_conv_kdfold); the packed weight layout depends on it.
+// kd-folded variant of the 3x3x3 kernel (TcCfg::FOLD): narrow output tiles with 16-bit operands.  On by default
+// (b3d_set_conv_kdfold switches it); the packed weight layout depends on it.
 static int g_kdfold = 1;
 static bool use_fold(const ConvGeom& g) {
   if (!g_kdfold || g.mode != CONV_S1 || g.k != 3 || operand_type(g) == OP_TF32) return false;
