@@ -82,19 +82,18 @@ int sm_count();
 // Both are no-ops in launches without the attribute / without a dependent.
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-// <<<grid, block, smem, s>>> with the programmatic-serialization attribute (B3D_PDL=0: plain launch).  Only for kernels
-// whose first statement is pdl_wait().
+// <<<grid, block, smem, s>>> with the programmatic-serialization attribute.  Only for kernels that read nothing the
+// previous kernel writes before their pdl_wait().
 template <typename... KArgs, typename... Args>
 inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t s,
                               Args&&... args) {
-  static const int pdl = [] { const char* e = getenv("B3D_PDL"); return (e == nullptr || e[0] != '0') ? 1 : 0; }();
   cudaLaunchConfig_t cfg;
   memset(&cfg, 0, sizeof(cfg));
   cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = s;
   cudaLaunchAttribute at[1];
   at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   at[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = at; cfg.numAttrs = pdl ? 1 : 0;
+  cfg.attrs = at; cfg.numAttrs = 1;
   return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
 }
 __device__ __forceinline__ float warp_sum(float v) {

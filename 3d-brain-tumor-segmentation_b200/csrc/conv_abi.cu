@@ -526,19 +526,6 @@ extern "C" int b3d_conv3d_dgrad_p16(const DLTensor* dy_, const DLTensor* w_, DLT
 // How the P16 weight gradient of a layer runs: 0 = not on this path (narrow layers, odd channel counts), 1 = straight
 // from the operands, 2 = needs a 16-bit scratch of numel(big tensor) elements (stride-2 family: space-to-depth copy),
 // 3 = needs a 16-bit scratch of numel(dy) elements (TS-mode kernel: voxel-transposed dy).  `w_sp` = W of dy.
-// kh-folded TS-mode weight gradient (conv_tc_wgrad_ts.cu).  OFF by default: correct (tests/test_gpu_p16.py runs it with
-// B3D_WGRAD_TSF=1) but SLOWER than the per-tap kernels on B200 — 128^3 16->16 355 vs 241 us, 128^3 32->16 830 vs 411 us,
-// 64^3 32->32 134 vs 89 us (profiles/r02e_wgrad_tsf.txt), with 8 or 9 issuing warps alike: a TS-mode MMA runs at the
-// pipe's peak from N = 32 up, so folding kh into N saves no pipe time (M = 128 rows are computed for 16-32 useful ones
-// either way), and its B operand with a 288-byte N-group stride is fetched at about half the rate of the plane-strided one.
-static bool wgrad_tsf_on() {
-  static int on = -1;
-  if (on < 0) {
-    const char* e = getenv("B3D_WGRAD_TSF");
-    on = (e != nullptr && e[0] != '0' && e[0] != 0) ? 1 : 0;
-  }
-  return on == 1;
-}
 // Data gradient of a stride-1 conv whose INPUT was a virtual channel concat: dx comes out as one compact tensor per
 // concatenated piece (dx0 .. dx3, channel counts multiples of 16 adding up to the layer's Cin) instead of one tensor the
 // framework would have to slice — and copy — afterwards.
@@ -642,8 +629,6 @@ extern "C" int b3d_conv3d_wgrad_p16_plan(int k, int stride, int transposed, int 
   WgradGeom wg;
   memset(&wg, 0, sizeof(wg));
   wg.k = k; wg.s = 1; wg.nA = cin; wg.nB = cout; wg.bigp = cin; wg.smallp = cout; wg.Ws = w_sp;
-  if (wgrad_tsf_on() && k == 3 && (cout == 16 || cout == 32) && cin % 16 == 0 && 3 * cin <= 440 && w_sp % 8 == 0)
-    return 3;               // kh-folded TS kernel (the per-source limits are checked at launch; else plan 1 is run)
   return (g_wgrad_ts && tc_wgrad_ts_supported(wg)) ? 3 : 1;
 }
 
@@ -769,19 +754,11 @@ extern "C" int b3d_conv3d_wgrad_p16(const DLTensor* x0_, const DLTensor* x1_, co
   if (plan == 3) {
     const long long need = (long long)dy.B * dy.D * dy.H * dy.W * cout;
     B3D_REQUIRE(scratch != nullptr && scratch_n >= need, B3D_ERR_ARG, "wgrad (P16, TS): scratch of %lld elements", need);
-    WgP16 ws;
-    memset(&ws, 0, sizeof(ws));
-    ws.n = src.n; ws.big_bf16 = 1;
-    for (int i = 0; i < src.n; ++i) { ws.big[i] = src.p[i]; ws.C[i] = src.C[i]; }
-    if (wgrad_tsf_on() && tc_wgrad_tsf_supported(wg, &ws)) {
-      B3D_TRY(launch_p16_t8(dy.p, scratch, (long long)dy.B * dy.D * dy.H, dy.W, dy.C8, s));
-      return launch_conv_wgrad_tsf(wg, ws, scratch, (float*)dw.p, s);
-    }
     if (src.n == 1 && g_wgrad_ts && tc_wgrad_ts_supported(wg)) {
       B3D_TRY(launch_p16_t8(dy.p, scratch, (long long)dy.B * dy.D * dy.H, dy.W, dy.C8, s));
       return launch_conv_wgrad_ts(wg, xf.p, scratch, (float*)dw.p, s, 1, 0);
     }
-    // neither TS form takes these sources: the plan-1 kernel below (the scratch stays unused)
+    // the TS kernel takes one source only: the plan-1 kernel below (the scratch stays unused)
   }
   if (transposed) { wp.n = 1; wp.big[0] = big.p; wp.C[0] = cbig; }
   return launch_conv_wgrad_tc(wg, big.p, sml.p, (float*)dw.p, s, 0, 0, 0, &wp);

@@ -134,9 +134,6 @@ int launch_conv_wgrad_ts(const WgradGeom& wg, const void* x_bf16, const void* dy
 bool tc_wgrad_kdf_supported(const WgradGeom& wg, const WgP16* p16);
 int launch_conv_wgrad_kdf(const WgradGeom& wg, float* dw, cudaStream_t s, const WgP16& p16,
                           const void* dres = nullptr, float* dw2 = nullptr);
-// kh-folded TS-mode weight gradient (conv_tc_wgrad_ts.cu): P16 sources (virtual concat), Cout 16 | 32
-bool tc_wgrad_tsf_supported(const WgradGeom& wg, const WgP16* p16);
-int launch_conv_wgrad_tsf(const WgradGeom& wg, const WgP16& src, const void* dyT_bf16, float* dw, cudaStream_t s);
 int launch_cast_bf16_t8(const float* src, void* dst, long long nvox, int C, float* colsum, cudaStream_t s);
 int launch_cast_stack_bf16(const float* src, void* dst, int B, int D, int H, int W, int Cn, long long pitch, int k,
                            int sgn, int nA, cudaStream_t s);

@@ -308,7 +308,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) conv_tc_kernel(const TcParams p
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
   pdl_trigger();
-  pdl_wait();          // everything above overlaps the tail of the previous kernel (B3D_PDL)
+  pdl_wait();          // everything above overlaps the tail of the previous kernel
 
   if (warp == kTmaWarp) {
     // ============ operand loader, TMA form: one elected thread fetches the halo of every K chunk as ONE 5-D box
@@ -1225,19 +1225,8 @@ static int launch_cfg(const ConvGeom& g, const TcProblem& q, const float* x, con
     p.bias = nullptr; p.stats = nullptr; p.gap = nullptr;
     p.y = ws; p.ws_slice = out_elems;
   }
-  {
-    // programmatic dependent launch (common.cuh): the CTAs' prologue overlaps the tail of the previous kernel;
-    // B3D_PDL=0 launches the plain way (A/B: 11.85 -> 11.6-11.8 ms per training step)
-    static const int pdl = [] { const char* e = getenv("B3D_PDL"); return (e == nullptr || e[0] != '0') ? 1 : 0; }();
-    cudaLaunchConfig_t cfg;
-    memset(&cfg, 0, sizeof(cfg));
-    cfg.gridDim = grid; cfg.blockDim = dim3(kTcThreads); cfg.dynamicSmemBytes = C::SMEM; cfg.stream = s;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = at; cfg.numAttrs = pdl ? 1 : 0;
-    B3D_TRY(cuda_ok(cudaLaunchKernelEx(&cfg, conv_tc_kernel<C>, p, maps), "launch conv_tc"));
-  }
+  // programmatic dependent launch (common.cuh): the CTAs' prologue overlaps the tail of the previous kernel
+  B3D_TRY(cuda_ok(launch_pdl(conv_tc_kernel<C>, grid, dim3(kTcThreads), C::SMEM, s, p, maps), "launch conv_tc"));
   B3D_LAUNCH_CHECK("conv_tc");
   if (p.ksplit > 1) {
     const int G = stats != nullptr ? (g.groups > 0 ? g.groups : 1) : 8;

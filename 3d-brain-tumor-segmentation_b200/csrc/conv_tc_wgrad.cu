@@ -417,10 +417,7 @@ struct KdfParams {
   int nsrc, cend8[4];
   int g, xbd;                      // an x box holds g planes x xbd depth slices (xbd = HD when one source covers the
                                    // tile's planes: the whole halo is ONE box; else one box per (depth slice, g planes))
-  int dbg;                         // timing experiments only (B3D_KDF_DBG): 1 no MMAs, 8 no final reduction
   int P;                           // channel planes (octets) of the tile: 4 (Cin = 32, M = 128) or 2 (Cin = 16, M = 64)
-  int ntg;                         // 1: a CTA holds all 9 (kh, kw) accumulators (always, since the final reduction is
-                                   // vectorised); 3: blockIdx.z = kh — measured slower, experiments only (B3D_KDF_NTG)
 };
 
 __global__ void __launch_bounds__(256, 1)
@@ -436,13 +433,11 @@ __global__ void __launch_bounds__(256, 1)
   const int P = prm.P;
   const int cbase = blockIdx.y * 8 * P;       // channel tile
   const int yplanes = prm.Cout / 8;
-  const int kh0 = prm.ntg == 3 ? (int)blockIdx.z : 0, nt = prm.ntg == 3 ? 3 : 9;   // this CTA's taps: (kh0 + t / 3, t % 3)
-  const int nkh = nt / 3;
 
   if (threadIdx.x == 0) {
     // one MMA-issuing warp per kh tap (a warp can issue a tcgen05.mma only every ~50 cycles: profiles/r01_umma_rate.txt)
-    for (int i = 0; i < prm.nstages; ++i) { mbar_init(smem_u32(&full[i]), 1); mbar_init(smem_u32(&empty[i]), nkh); }
-    mbar_init(smem_u32(done), nkh);
+    for (int i = 0; i < prm.nstages; ++i) { mbar_init(smem_u32(&full[i]), 1); mbar_init(smem_u32(&empty[i]), 3); }
+    mbar_init(smem_u32(done), 3);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
   if (warp == 2) {
@@ -485,7 +480,7 @@ __global__ void __launch_bounds__(256, 1)
           int si = 0;
           while (si + 1 < prm.nsrc && gp >= prm.cend8[si]) ++si;
           const int lp = gp - (si > 0 ? prm.cend8[si - 1] : 0);
-          tma_load_5d(xdst + (uint32_t)((d * P + p) * prm.pslice), &maps.x[si], 4 * w0, h0 - 1 + kh0, lp, d0 - 1 + d, b, fb);
+          tma_load_5d(xdst + (uint32_t)((d * P + p) * prm.pslice), &maps.x[si], 4 * w0, h0 - 1, lp, d0 - 1 + d, b, fb);
         } else {
           // dy three times, shifted by 1 - kw voxels along w (zero fill outside the volume): copy kw at in-tile voxel u
           // holds dy[u - (kw - 1)], the partner of x[u + (kd - 1, kh - 1, 0)]
@@ -497,7 +492,7 @@ __global__ void __launch_bounds__(256, 1)
       __syncwarp();
       if (++s == prm.nstages) { s = 0; ph ^= 1; }
     }
-  } else if (warp >= 1 && warp <= nkh) {
+  } else if (warp >= 1 && warp <= 3) {
     // warps 1..3: the MMAs of kh tap (warp - 1), each into its own accumulator block
     const int t = warp - 1;
     const bool leader = elect_one();
@@ -525,7 +520,7 @@ __global__ void __launch_bounds__(256, 1)
           for (int w8 = 0; w8 < prm.TW; w8 += 8) {
             const uint32_t ycell = (uint32_t)((d * prm.TH + h) * prm.TW + w8);
             const uint32_t xcell = (uint32_t)(d * P * slicec + h * prm.HW + w8);
-            if (leader && !(prm.dbg & 1)) {
+            if (leader) {
               tc_mma_bf16(tmem_base + t * 3 * prm.Cout, adesc0 + xcell + (uint32_t)(t * prm.HW), bdesc0 + ycell, idesc, acc);
               // pointwise conv: rows kd = 1 of the centre (kh = 1) A operand are x[u] itself
               if (prm.dw2 != nullptr && t == 1)
@@ -546,7 +541,7 @@ __global__ void __launch_bounds__(256, 1)
     const int kd = q;
     mbar_wait(smem_u32(done), 0);
     tc_fence_after();
-    const bool live = blockIdx.x < prm.ntiles && q < 3 && !(prm.dbg & 8);
+    const bool live = blockIdx.x < prm.ntiles && q < 3;
     // the (kd, tap) block of dw — rows ci of this tile x Cout — is contiguous: stage the warp's 32 rows through shared
     // memory (the stage buffers are free once `done` fired) and add it with 16-byte vector reductions, consecutive lanes
     // on consecutive addresses (row-per-lane scalar atomics are 32 sectors per instruction, 8 P Cout of them per tap);
@@ -555,8 +550,8 @@ __global__ void __launch_bounds__(256, 1)
     float* stg = reinterpret_cast<float*>(smem) + q * 32 * pitch;
     const int n4 = 8 * P * prm.Cout / 4;
 #pragma unroll 1
-    for (int tt = 0; tt < nt + (prm.dw2 != nullptr ? 1 : 0); ++tt) {
-      const int t = tt < nt ? (tt + (int)blockIdx.x) % nt : 9;      // 9: the pointwise accumulator (rows kd = 1 only)
+    for (int tt = 0; tt < 9 + (prm.dw2 != nullptr ? 1 : 0); ++tt) {
+      const int t = tt < 9 ? (tt + (int)blockIdx.x) % 9 : 9;        // 9: the pointwise accumulator (rows kd = 1 only)
       for (int j = 0; j < prm.Cout; j += 16) {
         float v[16];
         tc_ld16(tmem_base + ((uint32_t)(q * 32) << 16) + t * prm.Cout + j, v);
@@ -567,7 +562,7 @@ __global__ void __launch_bounds__(256, 1)
       __syncwarp();
       if (live && (t < 9 || kd == 1)) {
         float4* blk = reinterpret_cast<float4*>(
-            t < 9 ? prm.dw + ((size_t)(kd * 9 + kh0 * 3 + t) * prm.Cin + cbase) * prm.Cout : prm.dw2 + (size_t)cbase * prm.Cout);
+            t < 9 ? prm.dw + ((size_t)(kd * 9 + t) * prm.Cin + cbase) * prm.Cout : prm.dw2 + (size_t)cbase * prm.Cout);
         for (int e = lane; e < n4; e += 32) {
           const int r = (e * 4) / prm.Cout, c = (e * 4) % prm.Cout;
           atomicAdd(blk + e, *reinterpret_cast<const float4*>(stg + r * pitch + c));
@@ -585,13 +580,10 @@ __global__ void __launch_bounds__(256, 1)
 }
 
 bool tc_wgrad_kdf_supported(const WgradGeom& wg, const WgP16* p16) {
-  static const int on = [] { const char* e = getenv("B3D_WGRAD_KDF"); return (e == nullptr || e[0] != '0') ? 1 : 0; }();
-  if (!on || p16 == nullptr) return false;
-  // Cin = 16: M = 64 with 48 real rows (in place of the TS-mode kernel, B3D_WGRAD_KDF16=0 keeps that one); Cin = 64 /
-  // 96 / 128: one CTA row per 32-channel tile (B3D_WGRAD_KDF64=0 keeps the per-tap kernel)
-  static const int on16 = [] { const char* e = getenv("B3D_WGRAD_KDF16"); return (e == nullptr || e[0] != '0') ? 1 : 0; }();
-  static const int on64 = [] { const char* e = getenv("B3D_WGRAD_KDF64"); return (e == nullptr || e[0] != '0') ? 1 : 0; }();
-  const bool cin_ok = wg.nA == 32 || (wg.nA == 16 && on16) || (on64 && wg.nA % 32 == 0 && wg.nA <= 128);
+  if (p16 == nullptr) return false;
+  // Cin = 16: M = 64 with 48 real rows (in place of the TS-mode kernel); Cin = 64 / 96 / 128: one CTA row per
+  // 32-channel tile
+  const bool cin_ok = wg.nA == 16 || (wg.nA % 32 == 0 && wg.nA <= 128);
   if (!(wg.k == 3 && wg.s == 1 && cin_ok && (wg.nB == 16 || wg.nB == 32))) return false;
   if (wg.Ws % 8 != 0 || wg.Hs % 2 != 0) return false;
   for (int i = 0; i < p16->n; ++i)
@@ -607,24 +599,12 @@ int launch_conv_wgrad_kdf(const WgradGeom& wg, float* dw, cudaStream_t s, const 
   static const int cand[][3] = {{1, 4, 8}, {2, 4, 8}, {2, 4, 16}, {2, 8, 16}, {3, 8, 16}, {4, 8, 16}, {4, 8, 32}};
   KdfParams p;
   memset(&p, 0, sizeof(p));
-  // small volumes: split the kh taps over 3 CTA groups (fewer final atomics per CTA, all SMs still busy)
-  const long long vox = (long long)wg.B * wg.Ds * wg.Hs * wg.Ws;
-  static const int force_ntg = [] { const char* e = getenv("B3D_KDF_NTG"); return e ? atoi(e) : 0; }();
-  // kh groups over blockIdx.z (ntg = 3) measured slower everywhere once the final reduction was vectorised (64^3
-  // 32->32: 64 vs 36 us): kept for experiments only
-  const int ntg = force_ntg ? force_ntg : 1;
-  (void)vox;
-  p.ntg = ntg;
   const int budget = kWgSmem - 128;
   bool found = false;
-  // timing experiments only: B3D_KDF_TILE = candidate index, B3D_KDF_NS = stage count
-  static const int force_tile = [] { const char* e = getenv("B3D_KDF_TILE"); return e ? atoi(e) : -1; }();
-  static const int force_ns = [] { const char* e = getenv("B3D_KDF_NS"); return e ? atoi(e) : 0; }();
   for (int i = 0; i < (int)(sizeof(cand) / sizeof(cand[0])); ++i) {
-    if (force_tile >= 0 && i != force_tile) continue;
     const int TD = cand[i][0], TH = cand[i][1], TW = cand[i][2];
     if (found && (TD > wg.Ds * 2 || TH > wg.Hs * 2 || TW > wg.Ws * 2)) continue;
-    const int HD = TD + 2, HH = TH + (ntg == 3 ? 0 : 2), HW = TW;      // no w halo: the kw shifts are in the dy copies
+    const int HD = TD + 2, HH = TH + 2, HW = TW;      // no w halo: the kw shifts are in the dy copies
     if (4 * HW > 256) continue;
     const int pslice = ((HH * HW * 16 + 127) / 128) * 128;
     // the A operand spans 16 M groups (M = 128) from the LAST depth slice a K step starts in: 12 are real, the rest
@@ -632,7 +612,7 @@ int launch_conv_wgrad_kdf(const WgradGeom& wg, float* dw, cudaStream_t s, const 
     const long long xbytes = (((long long)HD * P * pslice + 127) / 128) * 128;
     const int py = TD * TH * TW * 16;
     const long long stage = ((xbytes + (dw2 != nullptr ? 4LL : 3LL) * (Cout / 8) * py + 127) / 128) * 128;
-    for (int ns = force_ns > 0 ? force_ns : 4; ns >= 2; --ns) {
+    for (int ns = 4; ns >= 2; --ns) {
       const long long last = (long long)(ns - 1) * stage;
       // last K step of the last stage: group 15 starts at (TD-1)*4 slices + 15 slices + h/w offset
       if (ns * stage <= budget && last + ((long long)(TD - 1) * P + 4 * P + 1) * pslice <= budget) {
@@ -645,12 +625,11 @@ int launch_conv_wgrad_kdf(const WgradGeom& wg, float* dw, cudaStream_t s, const 
   }
   B3D_REQUIRE(found, B3D_ERR_UNSUPPORTED, "wgrad (kd in M): no tile fits shared memory (Cin=%d Cout=%d)", Cin, Cout);
   p.dw = dw; p.dw2 = dw2; p.Cin = Cin; p.Cout = Cout; p.P = P;
-  B3D_REQUIRE((dw2 == nullptr) == (dres == nullptr) && (dw2 == nullptr || (ntg == 1 && ((uintptr_t)dw2 & 15) == 0)),
+  B3D_REQUIRE((dw2 == nullptr) == (dres == nullptr) && (dw2 == nullptr || ((uintptr_t)dw2 & 15) == 0),
               B3D_ERR_ARG, "wgrad (kd in M): pointwise operands");
-  { const char* e = getenv("B3D_KDF_DBG"); p.dbg = e ? atoi(e) : 0; }
   p.ntd = (wg.Ds + p.TD - 1) / p.TD; p.nth = (wg.Hs + p.TH - 1) / p.TH; p.ntw = (wg.Ws + p.TW - 1) / p.TW;
   p.ntiles = wg.B * p.ntd * p.nth * p.ntw;
-  int nsplit = sm_count() / (nmt * ntg);
+  int nsplit = sm_count() / nmt;
   if (nsplit < 1) nsplit = 1;
   if (nsplit > p.ntiles) nsplit = p.ntiles;
   p.nsplit = nsplit;
@@ -664,9 +643,7 @@ int launch_conv_wgrad_kdf(const WgradGeom& wg, float* dw, cudaStream_t s, const 
       while (b) { const int t = a % b; a = b; b = t; }
       g = a;
     }
-    static const int big = [] { const char* e = getenv("B3D_KDF_BIGBOX"); return (e == nullptr || e[0] != '0') ? 1 : 0; }();
-    if (!big) g = 1;
-    p.g = g; p.xbd = (g == P && big) ? p.HD : 1;
+    p.g = g; p.xbd = g == P ? p.HD : 1;
   }
   int cum = 0;
   for (int i = 0; i < p16.n; ++i) {
@@ -687,7 +664,7 @@ int launch_conv_wgrad_kdf(const WgradGeom& wg, float* dw, cudaStream_t s, const 
                     "cudaFuncSetAttribute(wgrad_kdf)"));
     attr = true;
   }
-  conv3_wgrad_kdf_kernel<<<dim3((unsigned)nsplit, (unsigned)nmt, (unsigned)ntg), 256, kWgSmem, s>>>(maps, p);
+  conv3_wgrad_kdf_kernel<<<dim3((unsigned)nsplit, (unsigned)nmt), 256, kWgSmem, s>>>(maps, p);
   B3D_LAUNCH_CHECK("conv3_wgrad_kdf");
   return B3D_OK;
 }

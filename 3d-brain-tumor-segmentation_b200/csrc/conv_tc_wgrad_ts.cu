@@ -285,258 +285,6 @@ int launch_conv_wgrad_ts(const WgradGeom& wg, const void* x, const void* dyT, fl
   return B3D_OK;
 }
 
-// ================================================================================================ kh-folded form
-// The TS kernel above still issues one MMA per tap (27 per K step of 16 voxels, N = Cin each), and at N <= 32 an MMA's
-// cost is dominated by its fixed part.  Here the three kh taps of a (kd, kw) pair are folded into N: the x halo of a
-// tile is fetched as ONE box per source in the order [d][h][plane][w] (a P16 row-of-planes, as in conv_tc.cu), so the
-// N groups (kh, channel octet) of the B operand lie at ONE constant stride — a plane row — and a single MMA with
-// N' = 3 Cin multiplies dyT with the rows h-1, h, h+1 of the halo:
-//     D_(kd,kw)[co][kh * Cin + ci] += sum_v dyT[co][v] * x[v + (kd-1, kh-1, kw-1)][ci]
-// 9 MMAs per K step instead of 27 (Cin = 16: N' = 48).  Several sources (a virtual channel concat) = one MMA per
-// (pair, source) into adjacent accumulator columns.  Accumulators: pairs_per_cta * 3 * Cin <= 448 columns, so Cin = 16
-// keeps all 9 pairs in one CTA, Cin <= 48 one kd (3 pairs), Cin <= 144 one pair (grid.y = 1 | 3 | 9 tap groups).
-struct TsfParams {
-  float* dw;
-  int Cin, Cout;                   // total input channels (all sources), output channels
-  int nsrc, sc8[4], xoff[4], acol[4], coff[4];   // per source: planes, halo offset in a stage (bytes), accumulator column
-                                                 // offset inside a pair block, first channel
-  int TD, TH, TW, HD, HH, HW;
-  int py, xbytes, stage_bytes, nstages;
-  int ntd, nth, ntw, ntiles, nsplit;
-  int D;
-};
-struct alignas(64) TsfMaps {
-  CUtensorMap x[4];
-  CUtensorMap y;
-};
-
-// 9 issuing warps: one (kd, kw) pair each when a CTA holds all nine — with 8, one warp would carry two of the nine
-// equal work items and every tile would wait for it
-constexpr int kTsfIssuers = 9;
-constexpr int kTsfThreads = (2 + kTsfIssuers) * 32;
-constexpr int kTsfAccCols = 512 - 8 * kTsfIssuers;     // 440: accumulators below, A tiles (8 columns per warp) above
-
-template <int TGW>
-__global__ void __launch_bounds__(kTsfThreads, 1)
-    conv3_wgrad_tsf_kernel(const __grid_constant__ TsfMaps maps, const TsfParams prm) {
-  extern __shared__ __align__(1024) uint8_t smem[];
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + kTsSmem - 128);
-  uint64_t* full = bars;        // [4]  TMA bytes
-  uint64_t* empty = bars + 4;   // [4]  one tcgen05.commit per issuing warp
-  uint64_t* done = bars + 8;    //      one tcgen05.commit per issuing warp
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 9);
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int tg = blockIdx.y;                 // tap group: TGW = 9: all | 3: kd = tg | 1: (kd, kw) = (tg / 3, tg % 3)
-  const int gkd = TGW == 9 ? 0 : (TGW == 3 ? tg : tg / 3), gkw = TGW == 1 ? tg % 3 : 0;
-  const int od = TGW == 9 ? -1 : gkd - 1, ow = TGW == 1 ? gkw - 1 : -1;
-
-  if (threadIdx.x == 0) {
-    for (int i = 0; i < prm.nstages; ++i) { mbar_init(smem_u32(&full[i]), 1); mbar_init(smem_u32(&empty[i]), kTsfIssuers); }
-    mbar_init(smem_u32(done), kTsfIssuers);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)),
-                 "r"(512));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-
-  if (warp == 1) {
-    if (lane == 0) {
-      int s = 0, ph = 0;
-      const uint32_t bytes = (uint32_t)(prm.xbytes + prm.py);
-      for (int tile = blockIdx.x; tile < prm.ntiles; tile += prm.nsplit) {
-        int t = tile;
-        const int wt = t % prm.ntw; t /= prm.ntw;
-        const int ht = t % prm.nth; t /= prm.nth;
-        const int dt = t % prm.ntd; t /= prm.ntd;
-        const int b = t;
-        const int w0 = wt * prm.TW, h0 = ht * prm.TH, d0 = dt * prm.TD;
-        mbar_wait(smem_u32(&empty[s]), ph ^ 1);
-        const uint32_t fb = smem_u32(&full[s]);
-        mbar_expect_tx(fb, bytes);
-        const uint32_t base = smem_u32(smem + (size_t)s * prm.stage_bytes);
-        for (int i = 0; i < prm.nsrc; ++i)
-          tma_load_5d(base + prm.xoff[i], &maps.x[i], 4 * (w0 + ow), 0, h0 - 1, d0 + od, b, fb);
-        tma_load_5d(base + (uint32_t)(prm.stage_bytes - prm.py - 512), &maps.y, 0, 0, w0 / 8, h0, b * prm.D + d0, fb);
-        if (++s == prm.nstages) { s = 0; ph ^= 1; }
-      }
-    }
-  } else if (warp >= 2) {
-    const int iw = warp - 2;
-    const bool leader = elect_one();
-    // D = f32, A = B = bf16, A K-major (TMEM), B MN-major, M = 128; N is set per source below
-    const uint32_t idesc0 = (1u << 4) | (1u << 7) | (1u << 10) | (1u << 16) | ((128u >> 4) << 24);
-    const uint32_t a_col = tmem_base + kTsfAccCols + iw * 8;
-    int s = 0, ph = 0;
-    uint32_t acc = 0;
-    const uint32_t smem_base = smem_u32(smem);
-    const int wblk = prm.TW / 8;
-    const int nq = TGW * prm.nsrc;                     // (pair, source) work items of this CTA; warp iw takes q = iw (mod 9)
-    const int yoff = prm.stage_bytes - prm.py - 512;   // dyT tile sits at the end of the stage (512 B of cp slack after it)
-    for (int tile = blockIdx.x; tile < prm.ntiles; tile += prm.nsplit) {
-      mbar_wait(smem_u32(&full[s]), ph);
-      tc_fence_after();
-      const uint32_t xaddr = smem_base + (uint32_t)s * (uint32_t)prm.stage_bytes;
-      const uint64_t adesc0 = make_desc(xaddr + (uint32_t)yoff, 0, 128);
-      for (int d = 0; d < prm.TD; ++d)
-        for (int h = 0; h < prm.TH; h += 2)
-          for (int wb = 0; wb < wblk; ++wb) {
-            const uint32_t ycell = (uint32_t)(((d * prm.TH + h) * wblk + wb) * prm.Cout);      // 16-byte cells
-            if (leader) {
-              tc_cp_32x128b(a_col, adesc0 + ycell);                                            // voxels of row h
-              tc_cp_32x128b(a_col + 4, adesc0 + ycell + (uint32_t)(wblk * prm.Cout));          // voxels of row h+1
-              for (int q = iw; q < nq; q += kTsfIssuers) {
-                const int pr = q / prm.nsrc, i = q - pr * prm.nsrc;
-                const int kdl = TGW == 9 ? pr / 3 : 0, kwl = TGW == 1 ? 0 : pr % 3;
-                const int c8 = prm.sc8[i];
-                const uint32_t rowc = (uint32_t)(c8 * prm.HW);                                 // halo row pitch (cells)
-                // B: K = 8 voxels along w (16 B apart) x 2 rows (LBO = row pitch); N groups = (kh, octet) at one plane row
-                const uint64_t bdesc = make_desc(xaddr + (uint32_t)prm.xoff[i], rowc * 16, (uint32_t)prm.HW * 16) +
-                                       (uint64_t)(((uint32_t)((d + kdl) * prm.HH + h)) * rowc + (uint32_t)(wb * 8 + kwl));
-                const uint32_t idesc = idesc0 | ((uint32_t)(3 * c8) << 17);
-                tc_mma_ts_bf16(tmem_base + (uint32_t)(pr * 3 * prm.Cin + prm.acol[i]), a_col, bdesc, idesc, acc);
-              }
-            }
-            acc = 1;
-          }
-      if (leader) tc_commit(smem_u32(&empty[s]));
-      __syncwarp();
-      if (++s == prm.nstages) { s = 0; ph ^= 1; }
-    }
-    if (leader) tc_commit(smem_u32(done));
-    __syncwarp();
-  } else {
-    // ---- warp 0: final reduction of this CTA's partial dw (accumulator row co = TMEM lane co)
-    mbar_wait(smem_u32(done), 0);
-    tc_fence_after();
-    const bool live = blockIdx.x < prm.ntiles && lane < prm.Cout;
-#pragma unroll 1
-    for (int pr = 0; pr < TGW; ++pr) {
-      const int kd = TGW == 9 ? pr / 3 : gkd, kw = TGW == 1 ? gkw : pr % 3;
-      for (int i = 0; i < prm.nsrc; ++i) {
-        const int Ci = 8 * prm.sc8[i];
-        for (int kh = 0; kh < 3; ++kh) {
-          const int tap = kd * 9 + kh * 3 + kw;
-          for (int j = 0; j < Ci; j += 16) {
-            float v[16];
-            tc_ld16(tmem_base + (uint32_t)(pr * 3 * prm.Cin + prm.acol[i] + kh * Ci + j), v);
-            if (live) {
-              float* dst = prm.dw + ((size_t)tap * prm.Cin + prm.coff[i] + j) * prm.Cout + lane;   // dw[tap][ci][co]
-#pragma unroll
-              for (int q = 0; q < 16; ++q) atomicAdd(dst + (size_t)q * prm.Cout, v[q]);
-            }
-          }
-        }
-      }
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 1) {
-    tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512));
-  }
-}
-
-// sources: bf16 P16 twins whose channels concatenate to the conv input (C_i % 16 == 0, 3 C_i <= 256); Cout 16 | 32
-bool tc_wgrad_tsf_supported(const WgradGeom& wg, const WgP16* p16) {
-  if (!(wg.k == 3 && wg.s == 1 && (wg.nB == 16 || wg.nB == 32) && wg.Ws % 8 == 0 && wg.Hs % 2 == 0)) return false;
-  if (p16 == nullptr || p16->n < 1 || 3 * wg.nA > kTsfAccCols) return false;
-  for (int i = 0; i < p16->n; ++i)
-    if (p16->C[i] % 16 != 0 || 3 * p16->C[i] > 256) return false;
-  return true;
-}
-
-int launch_conv_wgrad_tsf(const WgradGeom& wg, const WgP16& src, const void* dyT, float* dw, cudaStream_t s) {
-  B3D_REQUIRE(tc_wgrad_tsf_supported(wg, &src), B3D_ERR_UNSUPPORTED, "wgrad (TS, kh-folded): shape not supported");
-  B3D_REQUIRE((((uintptr_t)dyT | (uintptr_t)dw) & 15) == 0, B3D_ERR_LAYOUT, "wgrad (TS): alignment");
-  const int Cin = wg.nA, Cout = wg.nB;
-  const int TGW = 9 * 3 * Cin <= kTsfAccCols ? 9 : (3 * 3 * Cin <= kTsfAccCols ? 3 : 1);
-  const int ntg = 9 / TGW;
-  static const int cand[][3] = {{1, 4, 8}, {2, 4, 8}, {2, 4, 16}, {2, 8, 16}, {4, 8, 16}, {4, 8, 32}, {4, 16, 32}};
-  TsfParams p;
-  memset(&p, 0, sizeof(p));
-  p.nsrc = src.n;
-  int c8tot = 0;
-  for (int i = 0; i < src.n; ++i) { p.sc8[i] = src.C[i] / 8; p.coff[i] = 8 * c8tot; p.acol[i] = 3 * 8 * c8tot; c8tot += p.sc8[i]; }
-  B3D_REQUIRE(8 * c8tot == Cin, B3D_ERR_SHAPE, "wgrad (TS): sources do not add up to Cin");
-  const int budget = kTsSmem - 128;
-  bool found = false;
-  for (int i = 0; i < (int)(sizeof(cand) / sizeof(cand[0])); ++i) {
-    const int TD = cand[i][0], TH = cand[i][1], TW = cand[i][2];
-    if (found && (TD > wg.Ds * 2 || TH > wg.Hs * 2 || TW > wg.Ws * 2)) continue;
-    if (wg.B > 1 && wg.Ds % TD != 0) continue;      // dyT folds the batch into depth: tiles must not straddle samples
-    const int HD = TD + (TGW == 9 ? 2 : 0), HH = TH + 2, HW = TW + (TGW >= 3 ? 2 : 0);
-    if (4 * HW > 256) continue;
-    long long off = 0;
-    int xoff[4];
-    for (int q = 0; q < src.n; ++q) { xoff[q] = (int)off; off += (((long long)HD * HH * p.sc8[q] * HW * 16 + 127) / 128) * 128; }
-    const int py = TD * TH * TW * Cout * 2;
-    // the dyT tile sits at the end of the stage; the cp of its last K chunk reads 32 rows (512 B) even when Cout = 16
-    const long long stage = ((off + py + 512 + 127) / 128) * 128;
-    for (int ns = 3; ns >= 2; --ns)
-      if (ns * stage <= budget) {
-        p.TD = TD; p.TH = TH; p.TW = TW; p.HD = HD; p.HH = HH; p.HW = HW;
-        p.py = py; p.stage_bytes = (int)stage; p.nstages = ns;
-        p.xbytes = 0;
-        for (int q = 0; q < src.n; ++q) { p.xoff[q] = xoff[q]; p.xbytes += HD * HH * p.sc8[q] * HW * 16; }
-        found = true;
-        break;
-      }
-  }
-  B3D_REQUIRE(found, B3D_ERR_UNSUPPORTED, "wgrad (TS): no tile fits shared memory (Cin=%d Cout=%d)", Cin, Cout);
-  p.dw = dw; p.Cin = Cin; p.Cout = Cout; p.D = wg.Ds;
-  p.ntd = (wg.Ds + p.TD - 1) / p.TD; p.nth = (wg.Hs + p.TH - 1) / p.TH; p.ntw = (wg.Ws + p.TW - 1) / p.TW;
-  p.ntiles = wg.B * p.ntd * p.nth * p.ntw;
-  int nsplit = sm_count() / ntg;
-  if (nsplit < 1) nsplit = 1;
-  if (nsplit > p.ntiles) nsplit = p.ntiles;
-  p.nsplit = nsplit;
-  EncodeTiledFn enc = tma_encode_fn();
-  B3D_REQUIRE(enc != nullptr, B3D_ERR_CUDA, "cuTensorMapEncodeTiled entry point not available");
-  TsfMaps maps;
-  memset(&maps, 0, sizeof(maps));
-  for (int i = 0; i < src.n; ++i) {
-    B3D_REQUIRE(((uintptr_t)src.big[i] & 15) == 0, B3D_ERR_LAYOUT, "wgrad (TS): alignment");
-    B3D_TRY(make_p16_map(&maps.x[i], src.big[i], 1, wg.B, wg.Db, wg.Hb, wg.Wb, p.sc8[i], p.HW, p.sc8[i], p.HH, p.HD));
-  }
-  {
-    const int W8 = wg.Ws / 8;
-    const cuuint64_t dims[5] = {8, (cuuint64_t)Cout, (cuuint64_t)W8, (cuuint64_t)wg.Hs, (cuuint64_t)wg.Ds * wg.B};
-    const cuuint64_t st[4] = {16, (cuuint64_t)Cout * 16, (cuuint64_t)Cout * 16 * W8, (cuuint64_t)Cout * 16 * W8 * wg.Hs};
-    const cuuint32_t box[5] = {8, (cuuint32_t)Cout, (cuuint32_t)(p.TW / 8), (cuuint32_t)p.TH, (cuuint32_t)p.TD};
-    const cuuint32_t es[5] = {1, 1, 1, 1, 1};
-    const CUresult r = enc(&maps.y, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, (void*)dyT, dims, st, box, es,
-                           CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                           CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    B3D_REQUIRE(r == CUDA_SUCCESS, B3D_ERR_CUDA, "cuTensorMapEncodeTiled(dyT) failed (%d)", (int)r);
-  }
-  B3D_TRY(cuda_ok(cudaMemsetAsync(dw, 0, sizeof(float) * 27 * (size_t)Cin * Cout, s), "memset dw"));
-  dim3 grid((unsigned)nsplit, (unsigned)ntg, 1);
-#define LAUNCH(T)                                                                                               \
-  do {                                                                                                          \
-    static bool attr = false;                                                                                   \
-    if (!attr) {                                                                                                \
-      B3D_TRY(cuda_ok(cudaFuncSetAttribute(conv3_wgrad_tsf_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
-                                           kTsSmem), "cudaFuncSetAttribute(wgrad_tsf)"));                        \
-      attr = true;                                                                                              \
-    }                                                                                                           \
-    conv3_wgrad_tsf_kernel<T><<<grid, kTsfThreads, kTsSmem, s>>>(maps, p);                                       \
-  } while (0)
-  if (TGW == 9) LAUNCH(9);
-  else if (TGW == 3) LAUNCH(3);
-  else LAUNCH(1);
-#undef LAUNCH
-  B3D_LAUNCH_CHECK("conv3_wgrad_tsf");
-  return B3D_OK;
-}
-
 // fp32 [nvox][C] -> bf16 [nvox/8][C][8] (8 consecutive voxels = 8 consecutive w) + optional column sums (bias gradient)
 __global__ void __launch_bounds__(256)
     cast_bf16_t8_kernel(const float* __restrict__ src, uint4* __restrict__ dst, long long nblk, int C,

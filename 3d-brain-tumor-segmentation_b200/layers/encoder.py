@@ -100,7 +100,7 @@ class Encoder(Layer):
 
     @staticmethod
     def _can_dedup(cache):
-        return (ops.DEDUP["on"] and ops.FUSED["on"] and ops.twin_dtype(False) is not None
+        return (ops.FUSED["on"] and ops.twin_dtype(False) is not None
                 and all(ops.sources(t) is not None for t in cache))
 
     def get_config(self):

@@ -88,7 +88,7 @@ class ResnetBlock(Layer):
         `inputs` holds only [a_0, .., a_last]; the two convs reading it use their kernels with the duplicate's weight
         slice folded into the last source's (SURVEY F3; exact)."""
         g = self.groups if self._fused_stats else 0
-        box = {} if ops.SHARE_DGRAD["on"] else None      # the two data gradients w.r.t. `inputs` are summed in-kernel
+        box = {}                                          # the two data gradients w.r.t. `inputs` are summed in-kernel
         (conv1, norm1, _), (conv2, norm2, _) = self.convs
         kpt = ops.fold_dup(self.conv3d_ptwise.kernel, dup_first) if dup_first else None
         kc1 = ops.fold_dup(conv1.kernel, dup_first) if dup_first else None

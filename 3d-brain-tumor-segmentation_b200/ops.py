@@ -215,12 +215,6 @@ def _grad_done(p, direct):
 USE_TC = {"on": True}
 
 
-def _os_env_flag(name, default):
-    import os
-    v = os.environ.get(name)
-    return default if v is None else v not in ("0", "", "off", "false")
-
-
 # ---- P16 operand twins -------------------------------------------------------------------------------------------
 # Every tensor that feeds a tcgen05 conv exists as a 16-bit "P16" twin [B, D, H, C/8, W, 8] (csrc/p16.cu) written by the
 # kernel that PRODUCES it (GroupNorm apply, block epilogue, their backward kernels): fp16 for forward activations, bf16
@@ -229,23 +223,6 @@ def _os_env_flag(name, default):
 # is not materialised at all: the autograd-visible tensor is then a zero-stride placeholder of the logical shape
 # (`_b3d_virtual`) that carries the twin(s); `materialize()` rebuilds fp32 for the rare consumer that needs it.
 P16 = {"on": True}
-# the pointwise and the first 3x3x3 conv of a ResnetBlock read the same tensor: their data gradients are summed in the
-# second kernel's epilogue (Conv3dFn.backward, `grad_box`: accumulate = 1, 256-bit read-modify-write by 12 epilogue
-# warps) instead of an autograd add pass.  Speed-neutral on B200 (A/B on one box, 128^3 step: 14.58 ms with it, 14.62 ms
-# without; with the round-1 4-warp epilogue it cost 0.5 ms) and it takes 16 torch `add` launches off the path.
-# B3D_SHARE_DGRAD=0 switches it off.
-SHARE_DGRAD = {"on": _os_env_flag("B3D_SHARE_DGRAD", True)}
-# ... and, better, computed by ONE kernel: the pointwise conv's incoming gradient joins the 3x3x3 conv's as a further K
-# segment that is used at the centre tap only (b3d_conv3d_dgrad_p16_block) — no pointwise data-gradient launch at all.
-# Needs SHARE_DGRAD (the two convs find each other through the block's grad_box).  B3D_FUSE_BLOCK_DGRAD=0 for A/B runs.
-FUSE_BLOCK_DGRAD = {"on": _os_env_flag("B3D_FUSE_BLOCK_DGRAD", True)}
-# The same pair of convs shares its input in the weight-gradient pass too: where the 3x3x3 layer runs on the kd-in-M
-# kernel (csrc/conv_tc_wgrad.cu) the pointwise layer's dw is one more MMA per K step over the x tile already in shared
-# memory (b3d_conv3d_wgrad_p16_block) instead of a second pass over x.  B3D_FUSE_BLOCK_WGRAD=0 for A/B runs.
-FUSE_BLOCK_WGRAD = {"on": _os_env_flag("B3D_FUSE_BLOCK_WGRAD", True)}
-# SURVEY F3: the encoder's dense connections list the previous block output twice; inside a Model the duplicate is
-# dropped and its weight slice folded into the other one (ops.FoldDupFn) — exact.  B3D_DEDUP=0 for A/B runs
-DEDUP = {"on": _os_env_flag("B3D_DEDUP", True)}
 # inside a Model forward (`fused_scope`) layer outputs are consumed by convs only, so blocks / resampling layers emit
 # twin-only outputs and channel concatenation is virtual; outside (layers used on their own) outputs stay real fp32
 import threading as _threading
@@ -416,12 +393,6 @@ def set_kd_fold(on: bool) -> bool:
     return prev
 
 
-# A/B switch for measurements (bench.py, tools/): B3D_KD_FOLD=0 runs the unfolded 3x3x3 kernel everywhere
-import os as _os
-if _os.environ.get("B3D_KD_FOLD") is not None:
-    set_kd_fold(_os.environ["B3D_KD_FOLD"] not in ("0", "", "off", "false"))
-
-
 def get_conv_precision():
     v = lib.b3d_get_conv_precision()
     return (_PREC_INV[v & 15], _PREC_INV[v >> 4])
@@ -530,7 +501,7 @@ class Conv3dFn(Function):
             k, stride, int(transposed), Cin, Cout, od[2]) != 0)
         ctx.mb = y._b3d_mb = {"bias": bias, "f32_grad": f32_grad}
         if grad_box is not None and k == 1 and stride == 1 and not transposed:
-            # the block's pointwise conv: see FUSE_BLOCK_DGRAD / FUSE_BLOCK_WGRAD
+            # the block's pointwise conv: the 3x3x3 conv reading the same x may compute its dx and dw (backward below)
             grad_box["pw"] = {"mb": ctx.mb, "w": w, "srcs_w": ctx.srcs_w}
         outs = (y, stats, gap)
         ctx.mark_non_differentiable(*[t for t in (stats, gap) if t is not None])
@@ -583,10 +554,13 @@ class Conv3dFn(Function):
             # Two convs reading the same tensor (pointwise + first 3x3x3 of a ResnetBlock) share a `grad_box`: the first
             # data gradient to run writes a fresh buffer and hands it to autograd, the second ADDS into that buffer in
             # its epilogue (accumulate = 1) and returns no gradient — same sum, no separate add pass over the tensor.
+            # Better, where both run on tcgen05 with twins, ONE kernel computes both: the pointwise conv's incoming
+            # gradient joins the 3x3x3 conv's as a further K segment used at the centre tap only
+            # (b3d_conv3d_dgrad_p16_block) — no pointwise data-gradient launch at all.
             box, acc = ctx.grad_box, 0
             split = ctx.pieces is not None and ctx.gradbox is not None and tcd and dy16 is not None
             fused_pw = None
-            if (FUSE_BLOCK_DGRAD["on"] and box is not None and "pw" in box and "dx" not in box and k == 3 and stride == 1
+            if (box is not None and "pw" in box and "dx" not in box and k == 3 and stride == 1
                     and not transposed and tcd and dy16 is not None and box["pw"]["mb"] is not mb
                     and ctx.xshape[-1] % 16 == 0):
                 dres16 = box["pw"]["mb"].get("dy16")
@@ -647,8 +621,11 @@ class Conv3dFn(Function):
             if pwbox is not None and pwbox["mb"] is mb:
                 pwbox["done"] = True
             dw, dw_direct = _grad_target(pw)
+            # the same pair shares x in the weight-gradient pass too: where the 3x3x3 layer runs on the kd-in-M kernel
+            # (csrc/conv_tc_wgrad.cu) the pointwise layer's dw is one more MMA per K step over the x tile already in
+            # shared memory (b3d_conv3d_wgrad_p16_block) instead of a second pass over x
             fuse_w = None
-            if (FUSE_BLOCK_WGRAD["on"] and plan and dy16 is not None and pwbox is not None and pwbox["mb"] is not mb
+            if (plan and dy16 is not None and pwbox is not None and pwbox["mb"] is not mb
                     and not pwbox.get("done") and k == 3 and stride == 1 and not transposed
                     and pwbox["w"].requires_grad and _same_sources(pwbox.get("srcs_w"), srcs_w)):
                 dres16 = pwbox["mb"].get("dy16")

@@ -233,9 +233,6 @@ class ThreadComm(Comm):
 
 # ------------------------------------------------------------------------------------------ context
 _TLS = threading.local()
-# A/B switch: B3D_SLAB_P16=0 keeps fp32 activations between the layers of a slab (the round-1 form)
-import os as _os
-SLAB_P16 = {"on": _os.environ.get("B3D_SLAB_P16", "1") not in ("0", "", "off", "false")}
 
 
 def current() -> Optional["SlabContext"]:
@@ -269,7 +266,7 @@ class SlabContext:
             self.comm.begin_forward()
         self.p16 = None
         self._arena_used = 0
-        if ops.P16["on"] and ops.USE_TC["on"] and SLAB_P16["on"]:
+        if ops.P16["on"] and ops.USE_TC["on"]:
             self.p16 = ops._TWIN_DT.get(ops.get_conv_precision()[0])
         return self
 

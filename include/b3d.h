@@ -92,9 +92,8 @@ int b3d_conv3d_tc_supported(int k, int stride, int transposed, int dgrad, int a,
 int b3d_set_conv_precision(int fwd_op, int bwd_op);
 int b3d_get_conv_precision(void);
 /* kd-folded variant of the 3x3x3 tcgen05 kernel for output tiles of 16 / 32 channels (depth taps folded into the MMA
- * N dimension: 2-2.4x fewer small-N MMAs; csrc/conv_tc.cu).  Process-wide, default ON (B3D_KD_FOLD=0 in the environment
- * of a Python process switches it off at import, ops.py); changes the packed weight layout of those layers (re-pack
- * after switching).  Returns the previous setting. */
+ * N dimension: 2-2.4x fewer small-N MMAs; csrc/conv_tc.cu).  Process-wide, default ON; changes the packed weight
+ * layout of those layers (re-pack after switching).  Returns the previous setting. */
 int b3d_set_conv_kdfold(int on);
 long long b3d_conv3d_packed_elems(int k, int stride, int a, int b);
 int b3d_conv3d_pack_weights(const DLTensor* w, DLTensor* packed, int stride, int transposed, int dgrad,

@@ -11,13 +11,11 @@ fused into a kernel (GroupNorm chunk statistics, pooling sums) are checked again
 at 1e-6 of the sum of magnitudes, which separates them from the conv's rounding.
 
 Every case names the kernel it is meant to reach, and the profiler confirms it: `expect_conv` / `expect_wgrad` restate
-the host heuristics (N tile, kd folding, operand type, split-K, weight-gradient plan) including the B3D_* switches, so a
-changed heuristic fails here instead of silently moving a case onto another path.  Ids containing `large` are the
-real-size cases; `-k "not large"` is the quick subset."""
-import os
+the host heuristics (N tile, kd folding, operand type, split-K, weight-gradient plan), so a changed heuristic fails here
+instead of silently moving a case onto another path.  The quick forward / data-gradient cases run once more with kd
+folding off (`ops.set_kd_fold(False)`, ids ending in `-kd_fold_off`).  Ids containing `large` are the real-size cases;
+`-k "not large"` is the quick subset."""
 import re
-import subprocess
-import sys
 
 import pytest
 import torch
@@ -27,22 +25,9 @@ from oracle import ref_model as R
 
 pytestmark = pytest.mark.gpu
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 OPCODE = {"tf32": 0, "bf16": 1, "fp16": 2}
 TWIN = {"fp16": torch.float16, "bf16": torch.bfloat16}
 SEEN = []          # (case id, kernel names, worst per-element ratio, worst rel-L2): printed with -s
-
-
-def env_on(name, default):
-    v = os.environ.get(name)
-    return default if v is None else not (v == "" or v[0] == "0")
-
-
-def switches():
-    """The A/B switches read once per process by the library (csrc/conv_tc*.cu, conv_abi.cu) and by ops.py."""
-    return {"kdf": env_on("B3D_WGRAD_KDF", True), "kdf16": env_on("B3D_WGRAD_KDF16", True),
-            "kdf64": env_on("B3D_WGRAD_KDF64", True), "tsf": env_on("B3D_WGRAD_TSF", False),
-            "fold": os.environ.get("B3D_KD_FOLD", "1") not in ("0", "", "off", "false")}
 
 
 # ------------------------------------------------------------------------------------------------ fixtures / helpers
@@ -52,6 +37,20 @@ def env(b3d, dev):
     yield b3d
     b3d.ops.set_conv_precision("fp16", "bf16")
     b3d._lib.lib.b3d_set_wgrad_ts(1)
+
+
+@pytest.fixture
+def kd_fold(env, request):
+    """The kd-folding setting of the case (indirect parameter); the previous one is restored afterwards."""
+    prev = env.ops.set_kd_fold(request.param)
+    yield request.param
+    env.ops.set_kd_fold(prev)
+
+
+def with_fold_off(cases):
+    """(case, kd_fold) parameters: every case with kd folding on, the quick ones once more with it off."""
+    return ([pytest.param(c, True, id=c[0]) for c in cases] +
+            [pytest.param(c, False, id=c[0] + "-kd_fold_off") for c in cases if "large" not in c[0]])
 
 
 def sm_count():
@@ -120,11 +119,11 @@ def pad(c, m):
 
 
 def expect_conv(mode, k, gcin, gcout, op, B, out_sp, *, act=0, accumulate=0, contiguous=True, nyd=1, stats=False,
-                stat_total=0, sw=None):
+                stat_total=0, fold=True):
     """Kernel configuration the host picks (csrc/conv_tc.cu operand_type / pick_n / use_fold / dispatch_n and the
     split-K rule of launch_cfg) for a conv pass in gather terms: gcin = channels read, gcout = channels written.
-    mode: 's1' | 'down' (space-to-depth) | 'up' (depth-to-space).  Returns (TcCfg tuple, split-K?, operand type)."""
-    sw = sw or switches()
+    mode: 's1' | 'down' (space-to-depth) | 'up' (depth-to-space); fold = ops.set_kd_fold.  Returns (TcCfg tuple,
+    split-K?, operand type)."""
     if not (op != "tf32" and (gcin % 16 == 0 or (mode == "s1" and gcin < 8))):
         op = "tf32"
     ck = 8 if op == "tf32" else 16
@@ -136,7 +135,7 @@ def expect_conv(mode, k, gcin, gcout, op, B, out_sp, *, act=0, accumulate=0, con
     else:
         ks, hb, qcin, qcout, qd = 2, 1, gcin, 8 * gcout, (Do // 2, Ho // 2, Wo // 2)
     n = pick_n(qcout)
-    fold = sw["fold"] and mode == "s1" and k == 3 and op != "tf32" and n in (16, 32)
+    fold = fold and mode == "s1" and k == 3 and op != "tf32" and n in (16, 32)
     if fold:
         cfg = (n, 8 if n == 16 else 4, 1, 3, 1, OPCODE[op], 1)
     else:
@@ -163,27 +162,21 @@ def expect_conv(mode, k, gcin, gcout, op, B, out_sp, *, act=0, accumulate=0, con
     return cfg, split, op
 
 
-def expect_wgrad(pieces, cout, H, W, ts=True, sw=None):
+def expect_wgrad(pieces, cout, H, W, ts=True):
     """Weight-gradient kernel of a stride-1 3x3x3 layer on the P16 path (conv_abi.cu b3d_conv3d_wgrad_p16,
-    conv_tc_wgrad.cu tc_wgrad_kdf_supported, conv_tc_wgrad_ts.cu; ts = b3d_set_wgrad_ts): 'kdf' | 'tsf' | 'ts' | 'tc',
-    and the plan b3d_conv3d_wgrad_p16_plan reports (3: a scratch for the TS forms, else 1)."""
-    sw = sw or switches()
+    conv_tc_wgrad.cu tc_wgrad_kdf_supported, conv_tc_wgrad_ts.cu; ts = b3d_set_wgrad_ts): 'kdf' | 'ts' | 'tc',
+    and the plan b3d_conv3d_wgrad_p16_plan reports (3: a scratch for the TS kernel, else 1)."""
     cin = sum(pieces)
-    tsf_plan = sw["tsf"] and cout in (16, 32) and cin % 16 == 0 and 3 * cin <= 440 and W % 8 == 0
     ts_ok = ts and cin == 16 and cout in (16, 32) and W % 8 == 0
-    plan = 3 if tsf_plan or ts_ok else 1
-    cin_ok = cin == 32 or (cin == 16 and sw["kdf16"]) or (sw["kdf64"] and cin % 32 == 0 and cin <= 128)
-    if sw["kdf"] and cin_ok and cout in (16, 32) and W % 8 == 0 and H % 2 == 0:
+    plan = 3 if ts_ok else 1
+    if cin in (16, 32, 64, 96, 128) and cout in (16, 32) and W % 8 == 0 and H % 2 == 0:
         return "kdf", plan
-    if tsf_plan and H % 2 == 0 and all(c % 16 == 0 and 3 * c <= 256 for c in pieces):
-        return "tsf", plan
     if ts_ok and len(pieces) == 1:
         return "ts", plan
     return "tc", plan
 
 
-WGRAD_KERNEL = {"kdf": "conv3_wgrad_kdf_kernel", "tsf": "conv3_wgrad_tsf_kernel", "ts": "conv3_wgrad_ts_kernel",
-                "tc": "conv3_wgrad_tc_kernel"}
+WGRAD_KERNEL = {"kdf": "conv3_wgrad_kdf_kernel", "ts": "conv3_wgrad_ts_kernel", "tc": "conv3_wgrad_tc_kernel"}
 
 
 # ------------------------------------------------------------------------------------------------ forward, stride 1
@@ -222,8 +215,8 @@ FWD = [
 ]
 
 
-@pytest.mark.parametrize("case", FWD, ids=[c[0] for c in FWD])
-def test_fwd_path(env, dev, case):
+@pytest.mark.parametrize("case,kd_fold", with_fold_off(FWD), indirect=["kd_fold"])
+def test_fwd_path(env, dev, case, kd_fold):
     cid, B, sp, cins, cout, k, op, p16, act, acc, extra, want_stats, want_gap, mean = case
     ops, lib = env.ops, env._lib.lib
     cin = sum(cins)
@@ -244,7 +237,7 @@ def test_fwd_path(env, dev, case):
         y0, ybuf0 = y.clone(), ybuf.clone()
         wp = ops.pack_weights(w, False, 1, False)
         cfg_e, split_e, op_e = expect_conv("s1", k, cin, cout, op, B, sp, act=act, accumulate=acc,
-                                           contiguous=not extra, stats=want_stats)
+                                           contiguous=not extra, stats=want_stats, fold=kd_fold)
         if p16:
             tw = [ops.to_p16(t, TWIN[op]) for t in xs]
             call = lambda: ops._call("b3d_conv3d_fwd_p16", *(tw + [None] * (4 - len(tw))), w, bias, y, 1, 0, act, stats,
@@ -342,8 +335,8 @@ SLAB = [
 ]
 
 
-@pytest.mark.parametrize("case", SLAB, ids=[c[0] for c in SLAB])
-def test_slab_fwd_window(env, dev, case):
+@pytest.mark.parametrize("case,kd_fold", with_fold_off(SLAB), indirect=["kd_fold"])
+def test_slab_fwd_window(env, dev, case, kd_fold):
     cid, d0, d1, hb, ha, pz, sp, cin, cout = case
     ops = env.ops
     D, H, W = sp
@@ -363,7 +356,8 @@ def test_slab_fwd_window(env, dev, case):
     off = d0 * H * W
     _, kern = run_profiled(lambda: ops._call("b3d_conv3d_fwd_p16_slab", xt, None, None, None, w, bias, y, 1, 0, 0, hb, ha,
                                              stats, 8, off, D * H * W, gap, wp, pz))
-    cfg_e, split_e, op_e = expect_conv("s1", 3, cin, cout, "fp16", 1, (d1 - d0, H, W), stats=True, stat_total=D * H * W)
+    cfg_e, split_e, op_e = expect_conv("s1", 3, cin, cout, "fp16", 1, (d1 - d0, H, W), stats=True, stat_total=D * H * W,
+                                       fold=kd_fold)
     assert tc_cfgs(kern) == [cfg_e] and has(kern, "conv_finish_kernel") == split_e, (kern, cfg_e, split_e)
     xr, wr = K.round_act(x.double().cpu(), "fp16"), K.round_weight(w.double().cpu(), "fp16")
     full = K.conv_taps(xr, wr) + bias.double().cpu()
@@ -398,8 +392,8 @@ DGRAD = [
 ]
 
 
-@pytest.mark.parametrize("case", DGRAD, ids=[c[0] for c in DGRAD])
-def test_dgrad_path(env, dev, case):
+@pytest.mark.parametrize("case,kd_fold", with_fold_off(DGRAD), indirect=["kd_fold"])
+def test_dgrad_path(env, dev, case, kd_fold):
     cid, form, B, sp, pieces, cout, k, mean = case
     ops = env.ops
     cin = sum(pieces)
@@ -429,7 +423,7 @@ def test_dgrad_path(env, dev, case):
                                  wpd, wpp)
     _, kern = run_profiled(call)
     cfg_e, split_e, op_e = expect_conv("s1", k, cout, cin, "bf16", B, sp, accumulate=form == "split",
-                                       nyd=len(pieces) if form in ("split", "block") else 1)
+                                       nyd=len(pieces) if form in ("split", "block") else 1, fold=kd_fold)
     if form == "block":
         cfg_e = cfg_e[:3] + (3, 1) + cfg_e[5:]
     cfgs = tc_cfgs(kern)
@@ -481,7 +475,17 @@ WGRAD = [
     ("wgrad_kdf_96to32", 1, (4, 6, 8), [32, 16, 48], 32, True, False, 0.3),
     ("wgrad_kdf_128to16", 1, (4, 8, 8), [64, 64], 16, True, False, 0.0),
     ("wgrad_kdf_block_32to16", 2, (6, 10, 16), [16, 16], 16, True, True, 0.0),
+    # sources of 1 and 3 channel octets: no plane count shared with the 4-plane tile but 1, so one x box per
+    # (depth slice, plane)
+    ("wgrad_kdf_onebox_32to16", 1, (4, 8, 16), [8, 24], 16, True, False, 0.0),
+    # odd H keeps these off kd-in-M: the per-tap kernel, the TS-mode kernel for Cin = 16, and the fused block form
+    # refuses
     ("wgrad_hodd_ts_16to32", 2, (4, 7, 16), [16], 32, True, False, 0.0),
+    ("wgrad_hodd_ts_16to16", 2, (4, 7, 24), [16], 16, True, False, 0.5),
+    ("wgrad_hodd_tc_32to32", 1, (8, 9, 16), [32], 32, True, False, 0.0),
+    ("wgrad_hodd_tc_64to16", 2, (4, 7, 16), [32, 32], 16, True, False, 0.0),
+    ("wgrad_hodd_tc_96to32", 1, (4, 5, 8), [32, 16, 48], 32, True, False, 0.3),
+    ("wgrad_hodd_block_32to16", 2, (6, 9, 16), [16, 16], 16, True, True, 0.0),
     ("wgrad_w12_tc_16to16_ts_off", 1, (4, 8, 12), [16], 16, False, False, 0.0),
     ("wgrad_tc_ks3_64to64", 1, (6, 10, 16), [64], 64, True, False, 0.5),
     ("wgrad_tc_ks3_256to128", 1, (4, 8, 8), [256], 128, True, False, 0.0),
@@ -502,8 +506,7 @@ def test_wgrad_path(env, dev, case):
     dw = torch.full((3, 3, 3, cin, cout), float("nan"), device=dev)
     lib.b3d_set_wgrad_ts(int(ts))
     try:
-        sw = dict(switches())
-        kind, plan_e = expect_wgrad(pieces, cout, sp[1], sp[2], ts, sw)
+        kind, plan_e = expect_wgrad(pieces, cout, sp[1], sp[2], ts)
         kdf_ok = bool(lib.b3d_conv3d_wgrad_p16_block_ok(cin, cout, sp[1], sp[2]))
         assert kdf_ok == (kind == "kdf"), (cid, kind, kdf_ok)
         plan = lib.b3d_conv3d_wgrad_p16_plan(3, 1, 0, cin, cout, sp[2])
@@ -744,28 +747,3 @@ def test_block_epilogue_kernels_at_model_shapes(env, dev, shape, mean):
               K.check("dbias_h2", dbh, dh2_r.sum(dim=(0, 1, 2, 3)), None, None, 1e-5)]
     record(f"block epilogue {tuple(shape)} mean {mean}", kern, checks)
 
-
-# ------------------------------------------------------------------------------------------------ switch sweep
-SWEEP = [("B3D_WGRAD_KDF", "0", "wgrad"), ("B3D_WGRAD_KDF16", "0", "wgrad"), ("B3D_WGRAD_KDF64", "0", "wgrad"),
-         ("B3D_KDF_BIGBOX", "0", "wgrad"), ("B3D_WGRAD_TSF", "1", "wgrad"), ("B3D_KD_FOLD", "0", "fwd or dgrad or slab"),
-         ("B3D_PDL", "0", "fwd or dgrad or slab")]
-
-
-def test_switch_sweep(env, dev):
-    """The quick subset of the cases each B3D_* switch affects, rerun in a fresh process with the switch set (they are
-    read once per process): the expected kernels follow from `switches()`."""
-    fails = []
-    for var, val, sel in SWEEP:
-        e = dict(os.environ, **{var: val})
-        cmd = [sys.executable, "-m", "pytest", "-q", "-x", "-p", "no:cacheprovider", os.path.abspath(__file__),
-               "-k", f"({sel}) and not large and not switch_sweep"]
-        try:
-            r = subprocess.run(cmd, cwd=ROOT, env=e, capture_output=True, text=True, timeout=600)
-        except subprocess.TimeoutExpired:
-            fails.append(f"{var}={val}: timed out")
-            continue
-        tail = r.stdout.strip().splitlines()[-1:] if r.stdout else []
-        print(f"{var}={val}: rc {r.returncode} {tail}")
-        if r.returncode != 0:
-            fails.append(f"{var}={val}: rc {r.returncode}\n{r.stdout[-3000:]}\n{r.stderr[-2000:]}")
-    assert not fails, "\n".join(fails)

@@ -60,8 +60,8 @@ CONV_CASES = [
     ((8, 8, 16), [32, 32], 32, 3, 2, False),
     ((4, 8, 8), [32], 16, 3, 2, True),               # transposed
     ((4, 4, 8), [64, 64], 32, 3, 2, True),
-    # shapes of the kh-folded TS weight gradient (conv_tc_wgrad_ts.cu; off by default, B3D_WGRAD_TSF=1 in the environment
-    # of the test run selects it): all 9 (kd, kw) pairs per CTA | one kd | one pair; several sources
+    # weight gradients over several channel tiles and sources: Cin 48 on the per-tap kernel (conv3_wgrad_tc_kernel),
+    # Cin 16 / 64 / 96 with the depth taps folded into M
     ((8, 16, 8), [16], 32, 3, 1, False),
     ((6, 10, 24), [48], 16, 3, 1, False),            # 432 accumulator columns, partial tiles in d and h
     ((8, 8, 16), [64], 32, 3, 1, False),             # N' = 192, one pair per CTA
