@@ -122,7 +122,8 @@ def gn_chunk_scale(y: torch.Tensor, groups: int = 8) -> torch.Tensor:
 
 # --------------------------------------------------------------------------------------------------------- checker
 def rel_l2(got: torch.Tensor, ref: torch.Tensor) -> float:
-    g, r = got.detach().double().cpu(), ref.detach().double().cpu()
+    r = ref.detach().double()
+    g = got.detach().double().to(r.device)
     return float((g - r).norm() / (r.norm() + 1e-300))
 
 
@@ -140,14 +141,14 @@ def check(what: str, got: torch.Tensor, ref: torch.Tensor, A: Optional[torch.Ten
           rel_tol: float, tile: Optional[Sequence[int]] = None, labels: str = "bdhwc") -> Check:
     """rel-L2(got, ref) <= rel_tol and, when A is given, every element within
     C_BOUND*(n_acc + 4)*2^-23*A + 2^-23*|ref|.  `tile` (TD, TH, TW, N): extent of one CTA output tile, to name the tile
-    of the worst element in the message."""
-    g = got.detach().double().cpu()
-    r = ref.detach().double().cpu()
+    of the worst element in the message.  Evaluated on ref's device (a GPU reference is compared on the GPU)."""
+    r = ref.detach().double()
+    g = got.detach().double().to(r.device)
     assert g.shape == r.shape, (what, tuple(g.shape), tuple(r.shape))
     rel = rel_l2(g, r)
     err = (g - r).abs()
     if A is not None:
-        bound = C_BOUND * (n_acc + 4) * U32 * A.detach().double().cpu() + U32 * r.abs() + 1e-300
+        bound = C_BOUND * (n_acc + 4) * U32 * A.detach().double().to(r.device) + U32 * r.abs() + 1e-300
         q = err / bound
     else:
         q = err / (r.abs().max() + 1e-300)
@@ -180,3 +181,33 @@ def check_sums(what: str, got: torch.Tensor, ref: torch.Tensor, scale: torch.Ten
     msg = (f"{what}: worst |got - ref| / ({tol:.0e} * sum|terms|) = {ratio:.3f} at index {tuple(int(i) for i in idx)} "
            f"(got {float(g.reshape(-1)[flat]):.10g}, ref {float(r.reshape(-1)[flat]):.10g})")
     return Check(what, rel_l2(g, r), ratio, dict(enumerate(int(i) for i in idx)), ok, msg)
+
+
+def half_ulp(v: torch.Tensor, dtype: torch.dtype) -> torch.Tensor:
+    """Half the spacing of `dtype` (torch.float16 | torch.bfloat16) numbers at |v|: the largest error of rounding v to
+    nearest (subnormals included)."""
+    mant, tiny = {torch.float16: (10, 2.0 ** -24), torch.bfloat16: (7, 2.0 ** -133)}[dtype]
+    _, e = torch.frexp(v.double().abs())                   # |v| = m * 2^e, m in [0.5, 1)
+    return torch.clamp(torch.ldexp(torch.ones_like(v, dtype=torch.float64), e - 1 - mant), min=tiny) * 0.5
+
+
+def check_rounded(what: str, got: torch.Tensor, ref: torch.Tensor, dtype: torch.dtype, tol32: float = 1e-5,
+                  labels: str = "bdhwc") -> Check:
+    """A 16-bit output that exists only in its rounded form (a P16 twin written without its fp32 tensor), unpacked to
+    fp32, against the fp64 reference: every element within half a `dtype` ulp (at the larger of |got|, |ref|) plus
+    tol32 * max|ref| for the fp32 evaluation that was rounded.  A value taken from a neighbouring cell or chunk misses
+    this bound by orders of magnitude."""
+    r = ref.detach().double()
+    g = got.detach().double().to(r.device)
+    assert g.shape == r.shape, (what, tuple(g.shape), tuple(r.shape))
+    bound = half_ulp(torch.maximum(g.abs(), r.abs()), dtype) + tol32 * float(r.abs().max()) + 1e-300
+    q = (g - r).abs() / bound
+    flat = int(torch.argmax(torch.nan_to_num(q, nan=float("inf"))).item())
+    idx = np.unravel_index(flat, tuple(g.shape))
+    ratio = float(q.reshape(-1)[flat])
+    where = dict(zip(labels, (int(i) for i in idx)))
+    ok = bool(torch.isfinite(g).all()) and ratio <= 1.0
+    msg = (f"{what}: worst |got - ref| / (half {str(dtype)[6:]} ulp + {tol32:.0e} max|ref|) = {ratio:.3f} at "
+           + ", ".join(f"{k}={v}" for k, v in where.items())
+           + f" (got {float(g.reshape(-1)[flat]):.8g}, ref {float(r.reshape(-1)[flat]):.8g})")
+    return Check(what, rel_l2(g, r), ratio, where, ok, msg)

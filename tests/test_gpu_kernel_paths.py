@@ -14,7 +14,13 @@ Every case names the kernel it is meant to reach, and the profiler confirms it: 
 the host heuristics (N tile, kd folding, operand type, split-K, weight-gradient plan), so a changed heuristic fails here
 instead of silently moving a case onto another path.  The quick forward / data-gradient cases run once more with kd
 folding off (`ops.set_kd_fold(False)`, ids ending in `-kd_fold_off`).  Ids containing `large` are the real-size cases;
-`-k "not large"` is the quick subset."""
+`-k "not large"` is the quick subset.
+
+GroupNorm (chunk and channel form) and the block epilogue are checked output by output against fp64 at the model's
+shapes; the depth-slab forms on the windows sharded inference produces, against fp64 of the whole volume sliced, with
+their P16 twins held to the rounding of the fp32 values they were stored from (`test_slab_window_kernels`)."""
+import contextlib
+import math
 import re
 
 import pytest
@@ -62,20 +68,28 @@ def rnd(*shape, seed=0, scale=1.0, mean=0.0, dev="cuda"):
     return (torch.randn(*shape, generator=g) * scale + mean).to(dev)
 
 
-def run_profiled(fn):
-    """Run fn under torch.profiler (CUDA activities) and return (its result, the names of the CUDA kernels it ran)."""
+def run_profiled(fn, repeatable=True):
+    """Run fn under torch.profiler (CUDA activities) and return (its result, the names of the CUDA kernels it ran).
+    On a shared device CUPTI occasionally delivers no activity at all for a short profiled region; a trace without a
+    single CUDA event is then taken once more, if fn may run twice (`repeatable`: False for calls that accumulate into
+    their outputs)."""
     from torch.profiler import ProfilerActivity, profile
-    torch.cuda.synchronize()
-    with profile(activities=[ProfilerActivity.CUDA]) as prof:
-        out = fn()
+    for attempt in range(2 if repeatable else 1):
         torch.cuda.synchronize()
-    names = []
-    try:
-        for e in prof.profiler.kineto_results.events():
-            if "cuda" in str(e.device_type()).lower():
-                names.append(e.name())
-    except AttributeError:
-        names = [e.name for e in prof.events() if "cuda" in str(e.device_type).lower()]
+        with profile(activities=[ProfilerActivity.CUDA]) as prof:
+            out = fn()
+            torch.cuda.synchronize()
+        names = []
+        try:
+            for e in prof.profiler.kineto_results.events():
+                if "cuda" in str(e.device_type()).lower():
+                    names.append(e.name())
+        except AttributeError:
+            names = [e.name for e in prof.events() if "cuda" in str(e.device_type).lower()]
+        if names:
+            break
+        print("    torch.profiler recorded no CUDA activity" + ("; profiling the call again" if repeatable and not attempt
+                                                               else ""))
     kernels = [n for n in names if "kernel" in n]
     assert kernels, ("torch.profiler recorded no CUDA kernel for this case (CUPTI unavailable?): the kernel path "
                      f"cannot be verified; events seen: {names[:10]}")
@@ -245,7 +259,7 @@ def test_fwd_path(env, dev, case, kd_fold):
         else:
             x = torch.cat(xs, dim=-1).contiguous()
             call = lambda: ops._call("b3d_conv3d_fwd", x, w, bias, y, 1, 0, act, stats, 8, gap, acc, wp)
-        _, kern = run_profiled(call)
+        _, kern = run_profiled(call, repeatable=not acc)
     finally:
         ops.set_conv_precision("fp16", "bf16")
     cfgs = tc_cfgs(kern)
@@ -355,7 +369,7 @@ def test_slab_fwd_window(env, dev, case, kd_fold):
     gap = pre_g.clone() if pz else torch.empty(1, cout, device=dev)
     off = d0 * H * W
     _, kern = run_profiled(lambda: ops._call("b3d_conv3d_fwd_p16_slab", xt, None, None, None, w, bias, y, 1, 0, 0, hb, ha,
-                                             stats, 8, off, D * H * W, gap, wp, pz))
+                                             stats, 8, off, D * H * W, gap, wp, pz), repeatable=not pz)
     cfg_e, split_e, op_e = expect_conv("s1", 3, cin, cout, "fp16", 1, (d1 - d0, H, W), stats=True, stat_total=D * H * W,
                                        fold=kd_fold)
     assert tc_cfgs(kern) == [cfg_e] and has(kern, "conv_finish_kernel") == split_e, (kern, cfg_e, split_e)
@@ -421,7 +435,7 @@ def test_dgrad_path(env, dev, case, kd_fold):
         outs = [torch.full((B, *sp, c), float("nan"), device=dev) for c in pieces]
         call = lambda: ops._call("b3d_conv3d_dgrad_p16_block", dy16, dres16, w, wpw, *(outs + [None] * (4 - len(outs))),
                                  wpd, wpp)
-    _, kern = run_profiled(call)
+    _, kern = run_profiled(call, repeatable=form != "split")
     cfg_e, split_e, op_e = expect_conv("s1", k, cout, cin, "bf16", B, sp, accumulate=form == "split",
                                        nyd=len(pieces) if form in ("split", "block") else 1, fold=kd_fold)
     if form == "block":
@@ -615,45 +629,72 @@ GN_SHAPES = [("large_128c_16", (1, 128, 128, 128, 16)), ("large_64c_32_b2", (2, 
              ("fallback_c24", (1, 6, 10, 12, 24))]
 
 
-def _gn_ref(x, ga, be, dy, dx_kernel):
-    """fp64 GroupNorm + ReLU (the oracle) and its gradients (autograd), plus csum = per chunk (sum h, sum h*xhat) with
-    h = dy*[y > 0]*gamma_j, and xhat.
+def _gn_layout(shape, groups, channel, device):
+    """The element -> group and element -> affine-index maps of GroupNorm on NDHWC storage [B, D, H, W, C]:
+      * chunk form (channels_last, norm.cu / block.cu): group g of a sample is the g-th contiguous 1/G of its flat buffer,
+        and flat element e has the affine index g*C/G + (e % C) % (C/G) (SURVEY F1, ref_model.group_norm_chunk);
+      * channel form (channels_first, norm_channel.cu): group g is channels [g*C/G, (g+1)*C/G) of every voxel, and the
+        affine index is the channel.
+    Returns (per_group: [B, ...] -> [B, G] sums over each group, expand: [B, G] -> [B, ...], the affine index of every
+    element of a sample)."""
+    B, C = shape[0], shape[-1]
+    cg, n = C // groups, math.prod(shape[1:])
+    if channel:
+        per_group = lambda t: t.reshape(B, -1, groups, cg).sum((1, 3))
+        expand = lambda v: v[:, None, :, None].expand(B, n // C, groups, cg).reshape(shape)
+        j = torch.arange(C, device=device).expand(shape[1:])
+    else:
+        per_group = lambda t: t.reshape(B, groups, -1).sum(-1)
+        expand = lambda v: v[:, :, None].expand(B, groups, n // groups).reshape(shape)
+        e = torch.arange(n, device=device)
+        j = ((e // (n // groups)) * cg + (e % C) % cg).reshape(shape[1:])
+    return per_group, expand, j
+
+
+def _gn_ref(x, ga, be, dy, dx_kernel, groups=8, channel=False, relu=True):
+    """fp64 GroupNorm (+ ReLU) (the oracle, `channel`: under its channels_first semantics) and its gradients (autograd),
+    plus csum = per group (sum h, sum h*xhat) with h = dy*[y > 0]*gamma_j.
 
     The ReLU decision of an element whose pre-activation lies within fp32 resolution of 0 (|xhat*gamma + beta| below
     1e-5 of the magnitude of its terms) is not determined by the fp64 value: the kernel takes it on its fp32 value.  One
     such element changes dgamma_j by dy*xhat and dx by rstd*dy*gamma at that voxel, i.e. far more than 1e-5 of the
     result at 128^3 (a handful of such elements are expected among 33M).  For those elements the reference takes the
     decision the kernel took, read off the kernel's dx (the two candidates differ by rstd*dy*gamma there)."""
-    B, C = x.shape[0], x.shape[-1]
+    shape = tuple(x.shape)
+    per_group, expand, j = _gn_layout(shape, groups, channel, x.device)
     xd = x.double()
-    c = xd.reshape(B, 8, -1)
-    mean, var = c.mean(-1, keepdim=True), c.var(-1, unbiased=False, keepdim=True)
-    rstd = (1.0 / torch.sqrt(var + 1e-5)).expand(c.shape).reshape(x.shape)
-    xh = ((c - mean) / torch.sqrt(var + 1e-5)).reshape(x.shape)
-    # affine index of element e of chunk g (SURVEY F1, ref_model.group_norm_chunk): g*C/G + ((g*n + e) % C) % (C/G)
-    n, cg = c.shape[-1], C // 8
-    e = torch.arange(n, device=x.device)
-    j = torch.stack([g * cg + ((g * n + e) % C) % cg for g in range(8)])
-    gj, bj = ga.double()[j].reshape(1, *x.shape[1:]), be.double()[j].reshape(1, *x.shape[1:])
+    n = xd[0].numel() // groups
+    mean = expand(per_group(xd) / n)
+    rstd = expand(1.0 / torch.sqrt(per_group((xd - mean) ** 2) / n + 1e-5))
+    xh = (xd - mean) * rstd
+    gj, bj = ga.double()[j], be.double()[j]
     pre = xh * gj + bj
     dyd = dy.double()
 
+    def gn(*t):
+        with R.channels_first_semantics() if channel else contextlib.nullcontext():
+            return R.group_norm(*t, groups)
+
     def grads(mask):
         xr, gr, br = (t.double().clone().requires_grad_(True) for t in (x, ga, be))
-        return torch.autograd.grad(R.group_norm(xr, gr, br) * mask, (xr, gr, br), dyd)
-    m = (pre > 0).double()
-    dx = grads(m)[0]
-    amb = pre.abs() <= 1e-5 * ((xd.abs() + mean.abs().expand(c.shape).reshape(x.shape)) * rstd * gj.abs() + bj.abs())
-    t = rstd * dyd * gj
-    alt = dx + torch.where(m > 0, -t, t)
-    dk = dx_kernel.double()
-    flip = amb & ((dk - alt).abs() < (dk - dx).abs())
-    m = torch.where(flip, 1.0 - m, m)
+        return torch.autograd.grad(gn(xr, gr, br) * mask, (xr, gr, br), dyd)
+    m = (pre > 0).double() if relu else torch.ones_like(pre)
+    if relu:
+        dx = grads(m)[0]
+        amb = pre.abs() <= 1e-5 * ((xd.abs() + mean.abs()) * rstd * gj.abs() + bj.abs())
+        t = rstd * dyd * gj
+        alt = dx + torch.where(m > 0, -t, t)
+        dk = dx_kernel.double()
+        flip = amb & ((dk - alt).abs() < (dk - dx).abs())
+        m = torch.where(flip, 1.0 - m, m)
+        print(f"    ReLU decisions within fp32 resolution of 0: {int(amb.sum())}, taken as the kernel did: "
+              f"{int(flip.sum())}")
     dx, dga, dbe = grads(m)
-    y = torch.relu(R.group_norm(xd, ga.double(), be.double()))
+    y = gn(xd, ga.double(), be.double())
+    y = torch.relu(y) if relu else y
     h = dyd * m * gj
-    print(f"    ReLU decisions within fp32 resolution of 0: {int(amb.sum())}, taken as the kernel did: {int(flip.sum())}")
-    return y, dx, dga, dbe, xh, h, m
+    csum = torch.stack([per_group(h), per_group(h * xh)], dim=-1)
+    return y, dx, dga, dbe, csum, m
 
 
 @pytest.mark.parametrize("mean", [0.0, 3.0], ids=["zero_mean", "mean3"])
@@ -684,9 +725,7 @@ def test_group_norm_kernels_at_model_shapes(env, dev, shape, mean):
     assert has(kern, "gn_stats_kernel") and has(kern, "gn_apply"), kern
     assert has(kern, "gn_bwd_reduce8_kernel") == cells, kern       # the cell kernels, or the non-cell fallback
     xd = x.double()
-    yr, dxr, dgar, dber, xh, h, _ = _gn_ref(x, ga, be, dy, dx)
-    hc, xc = h.reshape(B, 8, -1), xh.reshape(B, 8, -1)
-    csr = torch.stack([hc.sum(-1), (hc * xc).sum(-1)], dim=-1)
+    yr, dxr, dgar, dber, csr, _ = _gn_ref(x, ga, be, dy, dx)
     checks = [K.check_sums("stats", stats, K.gn_chunk_sums(xd), K.gn_chunk_scale(xd)),
               K.check("y (gn_apply)", y0, yr, None, None, 1e-5),
               K.check("dgamma", dga, dgar, None, None, 1e-5), K.check("dbeta", dbe, dber, None, None, 1e-5),
@@ -697,14 +736,25 @@ def test_group_norm_kernels_at_model_shapes(env, dev, shape, mean):
     record(f"gn {tuple(shape)} mean {mean}", kern, checks)
 
 
-def _epilogue_ref(res, h2, ga, be, wsp, chse, dout, dgap, mask):
+def _epilogue_out(r, hh, g, b, ws, ch, mask=None):
     """fp64 restatement of the ResnetBlock epilogue (layers/resnet.py:121-137 after the pooling MLP):
-    out = res*(sigmoid(res . wsp) + chse) + relu(GN(h2)), with dgap the gradient reaching the pooling sums of res."""
+    out = r*(sigmoid(r . ws) + ch) + relu(GN(hh)); `mask`: the ReLU's decisions (default: hh's fp64 ones); g = None:
+    the form without GroupNorm (has_gn = 0), out = r*(sigmoid(r . ws) + ch) + hh."""
+    sp = torch.sigmoid((r * ws).sum(-1, keepdim=True))
+    if g is None:
+        a = hh
+    else:
+        gn = R.group_norm(hh, g, b)
+        a = torch.relu(gn) if mask is None else gn * mask
+    return r * (sp + ch[:, None, None, None, :]) + a
+
+
+def _epilogue_ref(res, h2, ga, be, wsp, chse, dout, dgap, mask):
+    """`_epilogue_out` with the kernel's ReLU decisions at 0 (mask) and its gradients, with dgap the gradient reaching
+    the pooling sums of res."""
     t = [v.double().clone().requires_grad_(True) for v in (res, h2, ga, be, wsp, chse)]
     r, hh, g, b, ws, ch = t
-    sp = torch.sigmoid((r * ws).sum(-1, keepdim=True))
-    gn = R.group_norm(hh, g, b)
-    out = r * (sp + ch[:, None, None, None, :]) + gn * mask           # the ReLU, with the kernel's decisions at 0
+    out = _epilogue_out(r, hh, g, b, ws, ch, mask)
     L = (out * dout.double()).sum() + (r.sum(dim=(1, 2, 3)) * dgap.double()).sum()
     grads = torch.autograd.grad(L, t)
     return out.detach(), grads
@@ -735,10 +785,8 @@ def test_block_epilogue_kernels_at_model_shapes(env, dev, shape, mean):
                   dh16, dbr, dbh, 8, 1e-5, 1)
     _, kern = run_profiled(run)
     assert has(kern, "b3d::block_fwd16_kernel"), kern
-    _, _, _, _, xh, h, mask = _gn_ref(h2, ga, be, dout, dh)
+    _, _, _, _, csr, mask = _gn_ref(h2, ga, be, dout, dh)
     o_r, (dres_r, dh2_r, dga_r, dbe_r, dws_r, dch_r) = _epilogue_ref(res, h2, ga, be, wsp, chse, dout, dgap, mask)
-    hc, xc = h.reshape(B, 8, -1), xh.reshape(B, 8, -1)
-    csr = torch.stack([hc.sum(-1), (hc * xc).sum(-1)], dim=-1)
     checks = [K.check("out", out, o_r, None, None, 1e-5), K.check("dchse", dch, dch_r, None, None, 1e-5),
               K.check("dwsp", dws, dws_r, None, None, 1e-5), K.check("dgamma", dga, dga_r, None, None, 1e-5),
               K.check("dbeta", dbe, dbe_r, None, None, 1e-5), K.check("csum", csum, csr, None, None, 1e-5),
@@ -747,3 +795,262 @@ def test_block_epilogue_kernels_at_model_shapes(env, dev, shape, mean):
               K.check("dbias_h2", dbh, dh2_r.sum(dim=(0, 1, 2, 3)), None, None, 1e-5)]
     record(f"block epilogue {tuple(shape)} mean {mean}", kern, checks)
 
+
+
+# ------------------------------------------------------------------------------- channel GroupNorm at model shapes
+# the channels_first model's GroupNorm inputs in the NDHWC storage the kernels see: (id, shape, groups).  At 128^3 x 16
+# one channel group spreads over ~1,184 CTAs (cgeom caps the segments at 8 x SM count, divided by B).  Edges: three
+# channels per group; C % 4 == 0 but C % 8 != 0 (the whole-volume kernels take it, the slab kernel refuses it)
+GNC_SHAPES = [("large_128c_16", (1, 128, 128, 128, 16), 8), ("large_64c_32_b2", (2, 64, 64, 64, 32), 8),
+              ("32c_64", (1, 32, 32, 32, 64), 8), ("16c_128", (1, 16, 16, 16, 128), 8), ("8c_256", (1, 8, 8, 8, 256), 8),
+              ("c24_cg3_b2", (2, 5, 9, 7, 24), 8), ("c12_g4", (1, 6, 10, 12, 12), 4)]
+
+
+@pytest.mark.parametrize("relu", [True, False], ids=["relu", "no_relu"])
+@pytest.mark.parametrize("mean", [0.0, 3.0], ids=["zero_mean", "mean3"])
+@pytest.mark.parametrize("case", GNC_SHAPES, ids=[c[0] for c in GNC_SHAPES])
+def test_channel_group_norm_kernels_at_model_shapes(env, dev, case, mean, relu):
+    """b3d_gn_channel_stats / _apply / _bwd (csrc/norm_channel.cu) against fp64 GroupNorm over true channel groups:
+    the statistics at 1e-6 of sum|terms|, y, dgamma, dbeta, csum and dx at rel-L2 <= 1e-5."""
+    ops = env.ops
+    _, shape, G = case
+    B, C = shape[0], shape[-1]
+    x = rnd(*shape, seed=101, mean=mean)
+    ga, be = 1 + 0.3 * rnd(C, seed=102), 0.3 * rnd(C, seed=103)
+    dy = rnd(*shape, seed=104)
+    stats = torch.empty(B, G, 2, dtype=torch.float64, device=dev)
+    y, dx, dga, dbe, csum = (torch.empty_like(x), torch.empty_like(x), torch.empty_like(ga), torch.empty_like(be),
+                             torch.empty_like(stats))
+
+    def run():
+        ops._call("b3d_gn_channel_stats", x, stats, G)
+        ops._call("b3d_gn_channel_apply", x, stats, ga, be, y, G, 1e-5, int(relu))
+        ops._call("b3d_gn_channel_bwd", dy, x, stats, ga, be, dga, dbe, csum, dx, G, 1e-5, int(relu))
+    _, kern = run_profiled(run)
+    r = str(relu).lower()
+    for k in ("gnc_stats_kernel", f"gnc_apply_kernel<{r}>", f"gnc_bwd_reduce_kernel<{r}>", f"gnc_bwd_apply_kernel<{r}>"):
+        assert has(kern, k), (k, kern)
+    if C % 8:
+        with pytest.raises(env._lib.B3DError, match="multiple of 8"):
+            ops._call("b3d_gn_channel_apply_slab", x, stats, ga, be, torch.empty_like(x), None, G, 1e-5, int(relu),
+                      x[0].numel() // C)
+    grp = x.double().reshape(B, -1, G, C // G)
+    sums = torch.stack([grp.sum((1, 3)), (grp * grp).sum((1, 3))], dim=-1)
+    scale = torch.stack([grp.abs().sum((1, 3)), (grp * grp).sum((1, 3))], dim=-1)
+    yr, dxr, dgar, dber, csr, _ = _gn_ref(x, ga, be, dy, dx, groups=G, channel=True, relu=relu)
+    checks = [K.check_sums("stats", stats, sums, scale), K.check("y", y, yr, None, None, 1e-5),
+              K.check("dgamma", dga, dgar, None, None, 1e-5), K.check("dbeta", dbe, dber, None, None, 1e-5),
+              K.check("csum", csum, csr, None, None, 1e-5), K.check("dx", dx, dxr, None, None, 1e-5)]
+    record(f"gn channel {tuple(shape)} G={G} mean {mean} relu {relu}", kern, checks)
+
+
+# ----------------------------------------------------------------------------------------- NCDHW <-> NDHWC re-layout
+# (id, NDHWC shape): the image / output channel counts below the 32-wide tile, voxel counts that are not a multiple of
+# 32, B = 2, and the inference volume with the four image channels
+RELAYOUT = [("c2_odd", (1, 9, 17, 11, 2)), ("c3_odd_b2", (2, 9, 17, 11, 3)), ("c4", (1, 8, 8, 8, 4)),
+            ("c16_odd", (1, 9, 17, 11, 16)), ("c256_b2", (2, 5, 6, 7, 256)), ("large_160x192x160_c4", (1, 160, 192, 160, 4))]
+
+
+@pytest.mark.parametrize("case", RELAYOUT, ids=[c[0] for c in RELAYOUT])
+def test_relayout(env, dev, case):
+    """b3d_relayout is a permutation: bit-identical to permute().contiguous() in both directions (NaN-filled outputs,
+    so an element left unwritten fails too)."""
+    ops = env.ops
+    cid, (B, D, H, W, C) = case
+    x_cf = rnd(B, C, D, H, W, seed=111)
+    z_cl = rnd(B, D, H, W, C, seed=112)          # an independent input for the inverse: not only a round trip
+    x_cl = torch.full((B, D, H, W, C), float("nan"), device=dev)
+    z_cf = torch.full((B, C, D, H, W), float("nan"), device=dev)
+
+    def run():
+        ops._call("b3d_relayout", x_cf, x_cl, 1)
+        ops._call("b3d_relayout", z_cl, z_cf, 0)
+    _, kern = run_profiled(run)
+    assert has(kern, "transpose_kernel"), kern
+    want_cl, want_cf = x_cf.permute(0, 2, 3, 4, 1).contiguous(), z_cl.permute(0, 4, 1, 2, 3).contiguous()
+    record(cid, kern, [_same("NCDHW -> NDHWC", x_cl, want_cl), _same("NDHWC -> NCDHW", z_cf, want_cf)])
+
+
+def _same(what, got, want):
+    """Bit-identity (NaN counts as a difference) as a Check."""
+    ok = got.shape == want.shape and torch.equal(got, want)
+    nbad = 0 if ok else int((got != want).sum()) if got.shape == want.shape else -1
+    return K.Check(what, 0.0 if ok else K.rel_l2(got.float(), want.float()), 0.0 if ok else float("inf"), None, ok,
+                   f"{what}: " + ("bit-identical" if ok else f"{nbad} elements differ"))
+
+
+# ---------------------------------------------------------------------------------------------------- slab windows
+def _slab_cases():
+    """(id, [D, H, W, C], windows).  The windows depth-slab inference produces: slab.slab_bounds(160, world) for 2, 4
+    and 8 ranks scaled to each encoder level, as SlabContext.geometry does (8 ranks: 24,24,24,24,16,16,16,16 slices at
+    160), given as (world, level) and cut in the test.  GroupNorm chunks (1/8 of the flat volume) hold 20 / 10 / 5 / 2.5
+    slices, so slab and chunk boundaries do not line up.  Then hand-placed windows the 8-slice alignment never
+    produces: strictly inside one chunk, across at least 3 chunks, one slice, the first and the last slice."""
+    cases = []
+    for lvl in range(4):
+        D, H, W, C = 160 >> lvl, 192 >> lvl, 160 >> lvl, 16 << lvl
+        for world in (2, 4, 8):
+            # 160x192x160 and 80x96x80 (79M and 20M elements) are real-size cases; the two deeper levels are quick
+            cases.append((f"{'large_' if lvl <= 1 else ''}{D}x{H}x{W}x{C}_world{world}", (D, H, W, C), (world, lvl)))
+    # chunk = 2.5 slices: (3, 4) inside chunk 1 = [2.5, 5); (1, 9) across chunks 0..3
+    cases.append(("hand_20x24x20x128", (20, 24, 20, 128), [(3, 4), (1, 9), (12, 13), (19, 20)]))
+    # chunk = 5 slices: (11, 14) inside chunk 2 = [10, 15); (2, 33) across chunks 0..6
+    cases.append(("hand_40x48x40x16", (40, 48, 40, 16), [(11, 14), (2, 33), (0, 1), (39, 40)]))
+    return cases
+
+
+SLAB_WINDOWS = _slab_cases()
+
+
+@pytest.fixture(scope="module")
+def slab_refs(dev):
+    """Holds the whole-volume inputs and fp64 references of one volume at a time (the cases of a volume are adjacent;
+    ~3 GB of device memory at 160x192x160), released after the module's last test."""
+    cache = {}
+    yield cache
+    cache.clear()
+    torch.cuda.empty_cache()
+
+
+def _slab_volume(cache, shape, dev):
+    """Inputs (batch 1) with a depth-dependent mean and scale, so that neighbouring chunks' statistics differ by O(1)
+    and a value normalised with the wrong chunk's statistics is far off; and their fp64 whole-volume references."""
+    if shape in cache:
+        return cache[shape]
+    cache.clear()
+    D, H, W, C = shape
+    t = torch.arange(D, device=dev, dtype=torch.float32).view(1, D, 1, 1, 1) / D
+    cm = 0.5 * torch.sin(torch.arange(C, device=dev, dtype=torch.float32))
+    x = rnd(1, D, H, W, C, seed=121, dev=dev) * (0.5 + t) + (2 * t - 1) + cm
+    res = rnd(1, D, H, W, C, seed=122, dev=dev) * (1.5 - t) + 0.5
+    ga, be = 1 + 0.3 * rnd(C, seed=123, dev=dev), 0.3 * rnd(C, seed=124, dev=dev)
+    wsp, chse = 0.3 * rnd(C, seed=125, dev=dev), torch.sigmoid(rnd(1, C, seed=126, dev=dev))
+    xd = x.double()
+    grp = xd.reshape(-1, 8, C // 8)
+    v = dict(x=x, res=res, ga=ga, be=be, wsp=wsp, chse=chse,
+             st=K.gn_chunk_sums(xd), st_scale=K.gn_chunk_scale(xd),
+             st_c=torch.stack([grp.sum((0, 2)), (grp * grp).sum((0, 2))], dim=-1)[None],
+             y=R.group_norm(xd, ga.double(), be.double()))
+    with R.channels_first_semantics():
+        v["y_c"] = R.group_norm(xd, ga.double(), be.double())
+    p64 = [t.double() for t in (res, x, ga, be, wsp, chse)]
+    v["out"] = _epilogue_out(*p64)
+    v["out_nogn"] = _epilogue_out(p64[0], p64[1], None, None, p64[4], p64[5])
+    cache[shape] = v
+    return v
+
+
+def _unpack(ops, t, shape):
+    out = torch.full(shape, float("nan"), device=t.device)
+    ops._call("b3d_p16_unpack", t, out)
+    return out
+
+
+@pytest.mark.parametrize("case", SLAB_WINDOWS, ids=[c[0] for c in SLAB_WINDOWS])
+def test_slab_window_kernels(env, dev, slab_refs, case):
+    """The depth-slab GroupNorm / block-epilogue kernels on real slab windows against fp64 of the WHOLE volume, sliced:
+      * b3d_gn_stats_slab: each window's partial (sum x, sum x^2) per whole-volume chunk (zero for the chunks it misses)
+        at 1e-6 of sum|terms|, and their sum over a partition = the whole volume's;
+      * b3d_gn_apply_slab, b3d_gn_apply_p16_slab (fp32 y + twin, and twin only), b3d_gn_channel_apply_slab (y + twin,
+        y only, twin only) and b3d_block_epilogue_fwd_p16_slab (has_gn 1 with out + twin and twin only, the form
+        sharded inference uses; has_gn 0), given the exact whole-volume statistics: the fp32 output at rel-L2 <= 1e-5;
+      * every twin (unpacked by b3d_p16_unpack) bit-identical to the fp16 / bf16 rounding of the fp32 output stored from
+        the same registers; a twin written alone within half a 16-bit ulp + 1e-5 max|ref| of the fp64 reference, and
+        bit-identical to the twin written next to y.
+    ReLU alternates with every window, the twin type (fp16 / bf16) with every second window, starting from the level's
+    parity, so each case with 4+ windows runs all four combinations and the 2-rank cases take both twin types across the
+    levels.  (The worst rel-L2 of the `[path]` line is that of a twin
+    written alone: the bf16 rounding itself, ~1.7e-3.)"""
+    ops = env.ops
+    cid, (D, H, W, C), wins = case
+    partition, lvl = isinstance(wins, tuple), 0
+    if partition:
+        world, lvl = wins
+        wins = [(a >> lvl, b >> lvl) for a, b in env.slab.slab_bounds(160, world)]
+        assert wins[0][0] == 0 and wins[-1][1] == D and all(a[1] == b[0] for a, b in zip(wins, wins[1:])), wins
+    v = _slab_volume(slab_refs, (D, H, W, C), dev)
+    x, res, ga, be, wsp, chse = (v[k] for k in ("x", "res", "ga", "be", "wsp", "chse"))
+    per, nvox = H * W * C, D * H * W
+    total, L = D * per, D * per // 8
+    nan = float("nan")
+    outs = []
+
+    def run():
+        outs.clear()
+        for i, (d0, d1) in enumerate(wins):
+            relu, td = i % 2 == 0, (torch.float16, torch.bfloat16)[(i // 2 + lvl) % 2]
+            xs, rs = x[:, d0:d1].contiguous(), res[:, d0:d1].contiguous()
+            f32 = lambda: torch.full_like(xs, nan)
+            p16 = lambda: ops.p16_empty(xs.shape, xs, td).fill_(nan)
+            o = dict(relu=relu, td=td, d0=d0, d1=d1, part=torch.full((1, 8, 2), nan, dtype=torch.float64, device=dev),
+                     part_c=torch.full((1, 8, 2), nan, dtype=torch.float64, device=dev),
+                     y_a=f32(), y_p=f32(), t_p=p16(), t_po=p16(), y_c=f32(), t_c=p16(), y_co=f32(), t_co=p16(),
+                     o_g=f32(), t_g=p16(), t_go=p16(), o_n=f32(), t_n=p16())
+            off, r = d0 * per, int(relu)
+            ops._call("b3d_gn_stats_slab", xs, o["part"], 8, off, total)
+            ops._call("b3d_gn_apply_slab", xs, v["st"], ga, be, o["y_a"], 8, 1e-5, r, off, total)
+            ops._call("b3d_gn_apply_p16_slab", xs, v["st"], ga, be, o["y_p"], o["t_p"], 8, 1e-5, r, off, total)
+            ops._call("b3d_gn_apply_p16_slab", xs, v["st"], ga, be, None, o["t_po"], 8, 1e-5, r, off, total)
+            ops._call("b3d_gn_channel_stats", xs, o["part_c"], 8)
+            ops._call("b3d_gn_channel_apply_slab", xs, v["st_c"], ga, be, o["y_c"], o["t_c"], 8, 1e-5, r, nvox)
+            ops._call("b3d_gn_channel_apply_slab", xs, v["st_c"], ga, be, o["y_co"], None, 8, 1e-5, r, nvox)
+            ops._call("b3d_gn_channel_apply_slab", xs, v["st_c"], ga, be, None, o["t_co"], 8, 1e-5, r, nvox)
+            ops._call("b3d_block_epilogue_fwd_p16_slab", rs, xs, v["st"], ga, be, wsp, chse, o["o_g"], o["t_g"], 8,
+                      1e-5, 1, d0 * H * W, nvox)
+            ops._call("b3d_block_epilogue_fwd_p16_slab", rs, xs, v["st"], ga, be, wsp, chse, None, o["t_go"], 8,
+                      1e-5, 1, d0 * H * W, nvox)
+            ops._call("b3d_block_epilogue_fwd_p16_slab", rs, xs, None, None, None, wsp, chse, o["o_n"], o["t_n"], 8,
+                      1e-5, 0, d0 * H * W, nvox)
+            outs.append(o)
+    _, kern = run_profiled(run)
+    names = [n.replace(" ", "") for n in kern]
+    for k in ("gn_stats_kernel<4>", "gn_apply_kernel<4,true>", "gn_apply_kernel<4,false>", "gn_apply16_kernel<true>",
+              "gn_apply16_kernel<false>", "gnc_stats_kernel", "gnc_apply_slab_kernel<true>",
+              "gnc_apply_slab_kernel<false>", "block_fwd16_kernel<true>", "block_fwd16_kernel<false>"):
+        assert has(names, k), (cid, k, sorted(set(kern)))
+    xflat = v["x"].double().reshape(-1)
+    tot = torch.zeros(1, 8, 2, dtype=torch.float64, device=dev)
+    checks = []
+    for i, o in enumerate(outs):
+        d0, d1, td = o["d0"], o["d1"], o["td"]
+        w = f"w{i} [{d0},{d1})"
+        act = torch.relu if o["relu"] else (lambda t: t)
+        sl = lambda t: t[:, d0:d1]
+        # partial chunk sums of the window's elements [d0*per, d1*per) of the flat volume
+        ref_p, sc_p = torch.zeros(1, 8, 2, dtype=torch.float64, device=dev), torch.zeros(1, 8, 2, dtype=torch.float64,
+                                                                                         device=dev)
+        for g in range(8):
+            lo, hi = max(g * L, d0 * per), min((g + 1) * L, d1 * per)
+            if lo < hi:
+                s = xflat[lo:hi]
+                ref_p[0, g] = torch.stack([s.sum(), (s * s).sum()])
+                sc_p[0, g] = torch.stack([s.abs().sum(), (s * s).sum()])
+        tot += o["part"]
+        grp = sl(v["x"]).double().reshape(-1, 8, C // 8)
+        shp = tuple(o["y_a"].shape)
+        y_r, yc_r = act(sl(v["y"])), act(sl(v["y_c"]))
+        checks += [
+            K.check_sums(f"{w} gn_stats_slab", o["part"], ref_p, sc_p),
+            K.check_sums(f"{w} gn_channel_stats", o["part_c"], torch.stack([grp.sum((0, 2)), (grp * grp).sum((0, 2))],
+                                                                           dim=-1)[None],
+                         torch.stack([grp.abs().sum((0, 2)), (grp * grp).sum((0, 2))], dim=-1)[None]),
+            K.check(f"{w} gn_apply_slab y", o["y_a"], y_r, None, None, 1e-5),
+            K.check(f"{w} gn_apply_p16_slab y", o["y_p"], y_r, None, None, 1e-5),
+            _same(f"{w} gn_apply_p16_slab twin = y rounded", _unpack(ops, o["t_p"], shp), o["y_p"].to(td).float()),
+            K.check_rounded(f"{w} gn_apply_p16_slab twin only", _unpack(ops, o["t_po"], shp), y_r, td),
+            _same(f"{w} gn_apply_p16_slab twin only = twin next to y", o["t_po"], o["t_p"]),
+            K.check(f"{w} gn_channel_apply_slab y", o["y_c"], yc_r, None, None, 1e-5),
+            _same(f"{w} gn_channel_apply_slab twin = y rounded", _unpack(ops, o["t_c"], shp), o["y_c"].to(td).float()),
+            _same(f"{w} gn_channel_apply_slab y only = y next to twin", o["y_co"], o["y_c"]),
+            K.check_rounded(f"{w} gn_channel_apply_slab twin only", _unpack(ops, o["t_co"], shp), yc_r, td),
+            _same(f"{w} gn_channel_apply_slab twin only = twin next to y", o["t_co"], o["t_c"]),
+            K.check(f"{w} block_epilogue_slab out", o["o_g"], sl(v["out"]), None, None, 1e-5),
+            _same(f"{w} block_epilogue_slab twin = out rounded", _unpack(ops, o["t_g"], shp), o["o_g"].to(td).float()),
+            K.check_rounded(f"{w} block_epilogue_slab twin only", _unpack(ops, o["t_go"], shp), sl(v["out"]), td),
+            _same(f"{w} block_epilogue_slab twin only = twin next to out", o["t_go"], o["t_g"]),
+            K.check(f"{w} block_epilogue_slab (no GN) out", o["o_n"], sl(v["out_nogn"]), None, None, 1e-5),
+            _same(f"{w} block_epilogue_slab (no GN) twin = out rounded", _unpack(ops, o["t_n"], shp),
+                  o["o_n"].to(td).float())]
+    if partition:
+        checks.append(K.check_sums("sum of the windows' gn_stats_slab = whole volume", tot, v["st"], v["st_scale"]))
+    record(cid, kern, checks)

@@ -4,7 +4,9 @@
    rounding of the tensor-core kernels) equal the oracle's `conv3d_same` and its autograd to 1e-12.
 2. Sensitivity: the checker accepts an fp32 computation of the same rounded operands (what a correct kernel returns)
    and rejects it once a realistic bug is applied to it — one 16-channel K chunk of one tap missing inside one edge
-   patch, one CTA's voxel range missing from a dgamma, one warp's statistics flush missing."""
+   patch, one CTA's voxel range missing from a dgamma (chunk and channel GroupNorm), one warp's statistics flush
+   missing, a depth-slab window normalising the cells past a chunk boundary with the neighbouring chunk's statistics,
+   a P16 twin whose start is one cell off."""
 import pytest
 import torch
 
@@ -117,3 +119,90 @@ def test_checker_catches_a_dropped_warp_statistics_flush():
     bad[1, 5] -= part[1, 5, 7]                 # sample 1, chunk 5: the flush of one warp (32 voxels) is lost
     c = K.check_sums("stats, one warp dropped", bad, ref, scale)
     assert not c.ok and c.where[0] == 1 and c.where[1] == 5, c
+
+
+def test_checker_catches_a_dropped_cta_range_in_channel_group_dgamma():
+    """True channel groups (norm_channel.cu): a CTA of gnc_bwd_reduce_kernel owns a contiguous voxel range of every
+    channel; at 128^3 x 16 cgeom cuts a sample into ~1,184 such ranges."""
+    B, D, H, W, C, G = 1, 16, 16, 16, 32, 8
+    x, dy = r64(B, D, H, W, C, seed=12, mean=3.0), r64(B, D, H, W, C, seed=13)
+    ga, be = 1 + 0.3 * r64(C, seed=14), 0.3 * r64(C, seed=15)
+    gr, br = ga.clone().requires_grad_(True), be.clone().requires_grad_(True)
+    with R.channels_first_semantics():
+        y = torch.relu(R.group_norm(x, gr, br, G))
+        dga, dbe = torch.autograd.grad(y, (gr, br), dy)
+        with torch.enable_grad():
+            g32, b32 = ga.float().requires_grad_(True), be.float().requires_grad_(True)
+            d32 = torch.autograd.grad(torch.relu(R.group_norm(x.float(), g32, b32, G)), (g32, b32), dy.float())
+    assert K.check("dgamma fp32", d32[0], dga, None, None, 1e-5).ok
+    assert K.check("dbeta fp32", d32[1], dbe, None, None, 1e-5).ok
+    S = D * H * W
+    per_cta = -(-S // 1184)
+    v0, v1 = 10 * per_cta, 11 * per_cta
+    grp = x.reshape(B, S, G, C // G)
+    xh = ((grp - grp.mean((1, 3), keepdim=True)) / torch.sqrt(grp.var((1, 3), unbiased=False, keepdim=True) + 1e-5))
+    xh = xh.reshape(B, S, C)
+    mask = (y.reshape(B, S, C) > 0).double()
+    lost = (dy.reshape(B, S, C) * mask * xh)[:, v0:v1].sum(dim=(0, 1))
+    c = K.check("channel dgamma, one CTA dropped", d32[0].double() - lost, dga, None, None, 1e-5)
+    assert not c.ok, c
+
+
+def _slab_x(D, H, W, C, seed):
+    """A volume whose mean and scale change with depth (as in test_slab_window_kernels): neighbouring GroupNorm chunks
+    have different statistics."""
+    t = (torch.arange(D, dtype=torch.float64) / D).view(1, D, 1, 1, 1)
+    return r64(1, D, H, W, C, seed=seed) * (0.5 + t) + (2 * t - 1)
+
+
+def _gn_apply_slab_fp32(x, stats, ga, be, d0, d1, relu, chunk_of=None):
+    """fp32 evaluation of the slab apply (gn_apply16_kernel): window [d0, d1) of the volume x, chunk statistics of the
+    whole volume (fp64 sums -> fp32 mean, rstd), y = (x - mean) * (rstd * gamma_j) + beta_j.  chunk_of(e): the chunk
+    whose statistics flat element e is normalised with (default e // L)."""
+    _, D, H, W, C = x.shape
+    L, cg = x.numel() // 8, C // 8
+    xs = x[:, d0:d1].reshape(-1).float()
+    e = d0 * H * W * C + torch.arange(xs.numel())
+    chunk = e // L if chunk_of is None else chunk_of(e)
+    m = stats[0, :, 0] / L
+    mean = m.float()
+    rstd = (1.0 / torch.sqrt(stats[0, :, 1] / L - m * m + 1e-5)).float()
+    j = (e // L) * cg + (e % C) % cg
+    y = (xs - mean[chunk]) * (rstd[chunk] * ga.float()[j]) + be.float()[j]
+    y = torch.relu(y) if relu else y
+    return y.reshape(1, d1 - d0, H, W, C)
+
+
+def test_checker_catches_a_slab_window_with_the_neighbouring_chunks_statistics():
+    D, H, W, C = 20, 6, 8, 16                  # a chunk holds 2.5 slices
+    x = _slab_x(D, H, W, C, seed=16)
+    ga, be = 1 + 0.3 * r64(C, seed=17), 0.3 * r64(C, seed=18)
+    ref = torch.relu(R.group_norm(x, ga, be))
+    stats, L = K.gn_chunk_sums(x), x.numel() // 8
+    d0, d1 = 1, 9                              # chunks 0..3
+    good = _gn_apply_slab_fp32(x, stats, ga, be, d0, d1, True)
+    c = K.check("fp32 slab apply", good, ref[:, d0:d1], None, None, 1e-5)
+    assert c.ok, c
+    # the cells of chunk 1 (past the window's first chunk boundary) normalised with chunk 0's statistics
+    bad = _gn_apply_slab_fp32(x, stats, ga, be, d0, d1, True, chunk_of=lambda e: torch.where(e // L == 1, 0, e // L))
+    c = K.check("neighbouring chunk's statistics", bad, ref[:, d0:d1], None, None, 1e-5)
+    assert not c.ok, c
+    assert L <= (d0 + c.where["d"]) * H * W * C + (c.where["h"] * W + c.where["w"]) * C + c.where["c"] < 2 * L, c
+
+
+def test_checker_catches_a_twin_shifted_by_one_cell():
+    """A P16 twin written alone (no fp32 output next to it) is checked against the rounded fp64 reference; a twin whose
+    start is one 8-channel cell off fails, in fp16 and bf16."""
+    D, H, W, C = 20, 6, 8, 16
+    x = _slab_x(D, H, W, C, seed=19)
+    ga, be = 1 + 0.3 * r64(C, seed=20), 0.3 * r64(C, seed=21)
+    ref = R.group_norm(x, ga, be)[:, 3:11]
+    y32 = _gn_apply_slab_fp32(x, K.gn_chunk_sums(x), ga, be, 3, 11, False)
+    for dt in (torch.float16, torch.bfloat16):
+        twin = y32.to(dt).float()
+        c = K.check_rounded("twin", twin, ref, dt)
+        assert c.ok, c
+        shifted = twin.clone().reshape(-1)
+        shifted[8:] = twin.reshape(-1)[:-8].clone()
+        c = K.check_rounded("twin one cell off", shifted.reshape(twin.shape), ref, dt)
+        assert not c.ok and c.ratio > 10, c
