@@ -14,11 +14,12 @@ from .layers import (GroupNormalization, ResnetBlock, ConvDownsample, MaxDownsam
                      LinearUpsample, Encoder, Decoder, VariationalAutoencoder, get_downsampling, get_upsampling)
 from .model import Model  # noqa: F401
 from .util import DiceVAELoss, DiceCoefficient, ScheduledOptim  # noqa: F401
-from . import train, infer, slab, data  # noqa: F401
+from . import train, infer, slab, data, metrics  # noqa: F401
 from .data import parse_example, VolumeDataset  # noqa: F401
 from .slab import (SlabContext, DistComm, PeerComm, ThreadComm, slab_bounds, sharded_inference,  # noqa: F401
                    GraphedInference)
 from .infer import TestTimeAugmentor, pad_to_spatial_res  # noqa: F401
+from .metrics import BRATS_REGIONS, predict_labels, segmentation_metrics  # noqa: F401
 from .train import GradientTape, train_step, GraphedTrainStep, DataParallel, reduce_sum, TrainLog  # noqa: F401
 
 __all__ = ["GroupNormalization", "ResnetBlock", "ConvDownsample", "MaxDownsample", "ConvUpsample",

@@ -30,7 +30,7 @@ class DLTensor(C.Structure):
 
 
 _DT = {torch.float32: (2, 32), torch.float64: (2, 64), torch.int64: (0, 64), torch.bfloat16: (4, 16),
-       torch.float16: (2, 16), torch.int32: (0, 32)}
+       torch.float16: (2, 16), torch.int32: (0, 32), torch.uint8: (1, 8)}
 
 P = C.POINTER(DLTensor)
 
@@ -128,6 +128,11 @@ SIGNATURES = {
     "b3d_epoch_tick": "Tv",
     "b3d_flip_normalize": "TTTTiv",
     "b3d_flip_accumulate": "TTTifiv",
+    # evaluation of one segmented volume (csrc/metrics.cu)
+    "b3d_label_map": "TTfv",
+    "b3d_region_surface": "TTTTTTv",
+    "b3d_surface_edt": "TTifffv",
+    "b3d_hd95": "TTTTTTTv",
     # P16 operand twins (csrc/p16.cu) and the entry points that produce / consume them
     "b3d_p16_pack": "TTTv",
     "b3d_p16_unpack": "TTv",

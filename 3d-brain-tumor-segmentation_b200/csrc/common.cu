@@ -20,7 +20,7 @@ int view(const DLTensor* t, int dtype, int ndim, bool allow_pitch, const char* n
               "%s: tensor must live on a CUDA device (device_type=%d); b3d has no CPU path", name,
               (int)t->device.device_type);
   static const struct { uint8_t code, bits; } kDT[] = {
-      {kDLFloat, 32}, {kDLFloat, 64}, {kDLInt, 64}, {kDLBfloat, 16}, {kDLFloat, 16}};
+      {kDLFloat, 32}, {kDLFloat, 64}, {kDLInt, 64}, {kDLBfloat, 16}, {kDLFloat, 16}, {kDLUInt, 8}};
   B3D_REQUIRE(t->dtype.code == kDT[dtype].code && t->dtype.bits == kDT[dtype].bits && t->dtype.lanes == 1,
               B3D_ERR_DTYPE, "%s: wrong dtype (code=%d bits=%d), expected code=%d bits=%d", name,
               (int)t->dtype.code, (int)t->dtype.bits, (int)kDT[dtype].code, (int)kDT[dtype].bits);

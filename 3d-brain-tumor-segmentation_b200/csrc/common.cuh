@@ -32,7 +32,7 @@ struct TView {
 };
 
 // dtype codes
-enum { DT_F32 = 0, DT_F64 = 1, DT_I64 = 2, DT_BF16 = 3, DT_F16 = 4 };
+enum { DT_F32 = 0, DT_F64 = 1, DT_I64 = 2, DT_BF16 = 3, DT_F16 = 4, DT_U8 = 5 };
 
 // Validates: CUDA device, dtype, ndim, and compact row-major strides; if allow_pitch, the last
 // dim may be a channel slice of a wider NDHWC buffer (stride[last]==1, outer strides compact

@@ -290,6 +290,27 @@ int b3d_flip_normalize(const DLTensor* x, const DLTensor* mean, const DLTensor* 
 int b3d_flip_accumulate(const DLTensor* y, DLTensor* acc, const DLTensor* mask, int flip, float scale, int first,
                         void* stream);
 
+/* ---- evaluation of one segmented volume (csrc/metrics.cu; host side metrics.py) ------------------------------------
+ * label_map: labels[d,h,w] = first argmax_c y_pred[d,h,w,c] + 1 where that maximum is > threshold, else 0 (the hard
+ *   decision of b3d_dice_coeff); y_pred fp32 [D,H,W,C], C = 1..4; labels uint8 [d,h,w], d <= D, h <= H, w <= W (the
+ *   leading corner: undoes pad_to_spatial_res).
+ * region_surface: lut (uint8 [256]) maps a label to its region bits; counts (int64 [R,4], R <= 8) receives TP, FP, FN,
+ *   TN per region; surf_pred / surf_true (uint8 [D,H,W]) get bit r where the voxel belongs to region r and has a
+ *   6-neighbour outside it (outside the volume counts as outside).
+ * surface_edt: edt (fp32 [R,D,H,W]) = squared Euclidean distance, with voxel spacing (sd, sh, sw), from every voxel to
+ *   the nearest voxel with bit r of surf set; +inf where there is none.  Exact with unit spacing.  Lines up to 1024
+ *   voxels on every axis.
+ * hd95: out (fp64 [R,4]) = dice, sensitivity, specificity and the 95th percentile (numpy 'linear') of the distances from
+ *   the prediction's surface to the truth's and back; 0 when both surfaces are empty, +inf when one is.  A ratio with a
+ *   zero denominator is 1.  workspace: uint8, 16-byte aligned, >= 4 * R * (264 + 2 * D * H * W) bytes.
+ * Each call clears what it accumulates; none allocates or synchronises, so the sequence can be graph-captured. */
+int b3d_label_map(const DLTensor* y_pred, DLTensor* labels, float threshold, void* stream);
+int b3d_region_surface(const DLTensor* pred, const DLTensor* true_labels, const DLTensor* lut, DLTensor* counts,
+                       DLTensor* surf_pred, DLTensor* surf_true, void* stream);
+int b3d_surface_edt(const DLTensor* surf, DLTensor* edt, int R, float sd, float sh, float sw, void* stream);
+int b3d_hd95(const DLTensor* edt_true, const DLTensor* surf_pred, const DLTensor* edt_pred, const DLTensor* surf_true,
+             const DLTensor* counts, DLTensor* out, DLTensor* workspace, void* stream);
+
 /* ---- P16 operand twins -------------------------------------------------------------------------------------------
  * A "P16" tensor is the 16-bit copy of an activation (fp16) or gradient (bf16) in the layout the tcgen05 conv kernels
  * consume directly: [B, D, H, C/8, W, 8] (DLPack ndim 6, dtype f16 | bf16, compact).  Channel octets are planes inside
