@@ -77,22 +77,20 @@ SIGNATURES = {
     "b3d_conv3d_wgrad": "TTTTiiTTiv",
     "b3d_conv3d_pack_weights": "TTiiiv",
     "b3d_conv3d_pack_many": "TiLv",
-    "b3d_gn_stats": "TTiv",
-    "b3d_gn_apply": "TTTTTifiv",
+    "b3d_gn_stats": "TTiLLv",
+    "b3d_gn_apply": "TTTTTTTifiLLv",
     "b3d_gn_channel_stats": "TTiv",
     "b3d_gn_channel_apply": "TTTTTifiv",
     "b3d_gn_channel_bwd": "TTTTTTTTTifiv",
     "b3d_gn_channel_apply_slab": "TTTTTTifiLv",
     "b3d_relayout": "TTiv",
-    "b3d_gn_stats_slab": "TTiLLv",
-    "b3d_gn_apply_slab": "TTTTTifiLLv",
     "b3d_gn_bwd_reduce": "TTTTTTTTifiv",
-    "b3d_gn_bwd_apply": "TTTTTTTifiv",
+    "b3d_gn_bwd_apply": "TTTTTTTTTifiv",
     "b3d_se_fc_fwd": "TTTTTfv",
     "b3d_se_fc_bwd": "TTTTTTTTTfv",
-    "b3d_block_epilogue_fwd": "TTTTTTTTifiv",
+    "b3d_block_epilogue_fwd": "TTTTTTTTTTifiLLv",
     "b3d_block_epilogue_bwd_reduce": "TTTTTTTTTTTTifiv",
-    "b3d_block_epilogue_bwd_apply": "TTTTTTTTTTTTifiv",
+    "b3d_block_epilogue_bwd_apply": "TTTTTTTTTTTTTTTTifiv",
     "b3d_loss_fwd": "TTTTTTTTv",
     "b3d_loss_dice_fwd": "TTTTTTTTTTiv",
     "b3d_loss_bwd": "TTTTTTTTTTTTv",
@@ -123,8 +121,6 @@ SIGNATURES = {
     "b3d_peer_allreduce": "TTiTTiv",
     "b3d_peer_allreduce2": "TTTiTTiv",
     "b3d_conv3d_fwd_p16_slab": "TTTTTTTiiiiiTiLLTTiv",
-    "b3d_gn_apply_p16_slab": "TTTTTTifiLLv",
-    "b3d_block_epilogue_fwd_p16_slab": "TTTTTTTTTifiLLv",
     "b3d_epoch_tick": "Tv",
     "b3d_flip_normalize": "TTTTiv",
     "b3d_flip_accumulate": "TTTifiv",
@@ -146,10 +142,6 @@ SIGNATURES = {
     "b3d_conv3d_dgrad_p16": "TTTiiiTv",
     "b3d_conv3d_wgrad_p16": "TTTTTTiiTv",
     "b3d_conv3d_wgrad_p16_block": "TTTTTTTTv",
-    "b3d_gn_apply_p16": "TTTTTTTifiv",
-    "b3d_gn_bwd_apply_p16": "TTTTTTTTTifiv",
-    "b3d_block_epilogue_fwd_p16": "TTTTTTTTTTifiv",
-    "b3d_block_epilogue_bwd_apply_p16": "TTTTTTTTTTTTTTTTifiv",
 }
 _CT = {"T": P, "i": _i, "f": _f, "v": _v, "L": _ll, "U": _ull}
 for _name, _sig in SIGNATURES.items():

@@ -6,6 +6,7 @@
 // per-voxel channel dot).  GN2 follows the contiguous-chunk semantics of norm.cu and requires
 // voxel-aligned chunks (D*H*W % groups == 0); otherwise callers use HAS_GN=0 + the norm.cu kernels.
 #include "common.cuh"
+#include "twin16.cuh"
 
 namespace b3d {
 
@@ -345,14 +346,8 @@ __global__ void __launch_bounds__(kBT)
 // ================================================================================================ P16 twin forms
 // The same forward / backward-apply passes writing the 16-bit operand twins of their results ([B, D, H, C/8, W, 8],
 // common.cuh) for the tcgen05 convs that consume them.  Lane mapping: T = F/8 lanes cooperate on one voxel and every
-// lane owns ONE 16-byte cell (8 consecutive channels): two 128-bit loads per input tensor, one 128-bit store per twin.
-struct Twin16 {
-  uint4* p;         // nullptr: no twin
-  uint4* p2;        // optional second twin, always bf16
-  unsigned W, C8;   // voxels per row, channel octets
-  unsigned rows;    // D*H rows per sample
-  int bf16;
-};
+// lane owns ONE 16-byte cell (8 consecutive channels): two 128-bit loads per input tensor, one 128-bit store per twin
+// (Twin16 and the 16-bit packing: twin16.cuh).
 struct VoxPos { unsigned row, w; };
 __device__ __forceinline__ VoxPos vox_pos(unsigned W, unsigned vox) {
   VoxPos k;
@@ -363,12 +358,6 @@ __device__ __forceinline__ VoxPos vox_pos(unsigned W, unsigned vox) {
 __device__ __forceinline__ void vox_advance(unsigned W, VoxPos& k, unsigned dv) {
   k.w += dv;
   while (k.w >= W) { k.w -= W; ++k.row; }
-}
-__device__ __forceinline__ uint32_t pk16(float lo, float hi, int bf16) {
-  uint32_t r;
-  if (bf16) asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));
-  else asm("cvt.rn.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));
-  return r;
 }
 __device__ __forceinline__ void cell_store(const Twin16& o, unsigned b, const VoxPos& k, unsigned c8, const float (&v)[8]) {
   if (o.p == nullptr) return;
@@ -795,6 +784,25 @@ static int block_geom(const TView& res, int groups, bool has_gn, BlockGeom* gm, 
   return B3D_OK;
 }
 
+// geometry of the cell kernels: T = F/8 lanes per voxel (a power of two <= 32)
+static int block_geom16(const TView& res, int groups, bool has_gn, BlockGeom* gm, int* nchunks) {
+  B3D_REQUIRE(res.ndim == 5, B3D_ERR_SHAPE, "block epilogue (P16): res must be [B, D, H, W, F]");
+  B3D_TRY(block_geom(res, groups, has_gn, gm, nchunks));
+  const int T = gm->F / 8;
+  B3D_REQUIRE(gm->F % 8 == 0 && T >= 1 && T <= 32 && (T & (T - 1)) == 0, B3D_ERR_UNSUPPORTED,
+              "block epilogue (P16): filters must be 8 * 2^k <= 256 (got %d)", gm->F);
+  B3D_REQUIRE(res.numel / res.shape[0] / gm->F < (1LL << 32), B3D_ERR_UNSUPPORTED, "block epilogue (P16): sample too large");
+  gm->T = T; gm->npl = 2;
+  const int vstep = kBT / T;
+  long long vp = (long long)vstep * 2;     // >= 2 voxel steps per thread; small tensors get many short CTAs, not a 16-step latency chain
+  const long long B = res.shape[0];
+  const long long cap = (3LL * sm_count() + B * gm->G - 1) / (B * gm->G);
+  const long long need = ((gm->vpc + cap - 1) / cap + vstep - 1) / vstep * vstep;
+  if (need > vp) vp = need;
+  gm->vox_per_cta = (int)vp;
+  return B3D_OK;
+}
+
 static inline dim3 block_grid(const BlockGeom& gm, int nchunks) {
   return dim3((unsigned)((gm.vpc + gm.vox_per_cta - 1) / gm.vox_per_cta), (unsigned)nchunks, 1);
 }
@@ -858,35 +866,74 @@ extern "C" int b3d_se_fc_bwd(const DLTensor* gap_sum_, const DLTensor* w1_, cons
   return B3D_OK;
 }
 
+// With the twin out16 (and out16b, a second, bf16 twin for the weight gradients of the consuming convs) given: the cell
+// kernel, out nullable; otherwise the float4 kernel, out required.  total_vox != 0 (cell kernel only): res / h2 / the
+// twin hold voxels [vox_offset, vox_offset + D*H*W) of a batch-1 volume of total_vox voxels (depth-slab inference);
+// `stats` = the all-reduced GroupNorm statistics of the whole volume's chunks, `chse` from the all-reduced pooling sums.
 extern "C" int b3d_block_epilogue_fwd(const DLTensor* res_, const DLTensor* h2_, const DLTensor* stats_,
                                       const DLTensor* gamma_, const DLTensor* beta_, const DLTensor* wsp_,
-                                      const DLTensor* chse_, DLTensor* out_, int groups, float eps, int has_gn,
+                                      const DLTensor* chse_, DLTensor* out_, DLTensor* out16_, DLTensor* out16b_,
+                                      int groups, float eps, int has_gn, long long vox_offset, long long total_vox,
                                       void* stream) {
+  B3D_REQUIRE(out16_ != nullptr || out16b_ == nullptr, B3D_ERR_ARG, "block epilogue: out16b without out16");
   TView res, h2, out, st, ga, be, wsp, ch;
   BlockGeom gm;
   int nchunks;
   B3D_TRY(view(res_, DT_F32, -1, false, "res", &res));
   B3D_TRY(view(h2_, DT_F32, -1, false, "h2", &h2));
-  B3D_TRY(view(out_, DT_F32, -1, false, "out", &out));
-  B3D_REQUIRE(res.numel == h2.numel && res.numel == out.numel, B3D_ERR_SHAPE, "block epilogue: size mismatch");
-  B3D_TRY(block_geom(res, groups, has_gn != 0, &gm, &nchunks));
+  if (out_ != nullptr || out16_ == nullptr) B3D_TRY(view(out_, DT_F32, -1, false, "out", &out));
+  B3D_REQUIRE(res.numel == h2.numel && (out_ == nullptr || res.numel == out.numel), B3D_ERR_SHAPE,
+              "block epilogue: size mismatch");
+  if (out16_ == nullptr) {
+    B3D_REQUIRE(total_vox == 0, B3D_ERR_UNSUPPORTED, "block epilogue: a window needs the twin kernel");
+    B3D_TRY(block_geom(res, groups, has_gn != 0, &gm, &nchunks));
+  } else {
+    B3D_REQUIRE(total_vox == 0 || (res.ndim == 5 && res.shape[0] == 1), B3D_ERR_SHAPE, "block epilogue (window): batch 1");
+    B3D_TRY(block_geom16(res, groups, has_gn != 0, &gm, &nchunks));
+  }
+  int nlaunch = nchunks;
+  if (total_vox != 0) {      // the window's CTAs keep their per-CTA voxel count, the grid covers the chunks it meets
+    const long long S_local = gm.S;
+    B3D_REQUIRE(total_vox > 0 && vox_offset >= 0 && vox_offset + S_local <= total_vox && total_vox % gm.G == 0 &&
+                    total_vox < (1LL << 32), B3D_ERR_ARG, "block epilogue (window): bad window (%lld + %lld of %lld)",
+                vox_offset, S_local, total_vox);
+    gm.S = total_vox; gm.vpc = total_vox / gm.G; gm.vshift = vox_offset; gm.S_local = S_local;
+    gm.chunk0 = (int)(vox_offset / gm.vpc);
+    nlaunch = (int)((vox_offset + S_local - 1) / gm.vpc) - gm.chunk0 + 1;
+  }
   B3D_TRY(vecF(wsp_, gm.F, "wsp", &wsp));
   B3D_TRY(vecF(chse_, res.shape[0] * gm.F, "chse", &ch));
-  cudaStream_t s = (cudaStream_t)stream;
   if (has_gn) {
     B3D_TRY(view(stats_, DT_F64, -1, false, "stats", &st));
     B3D_REQUIRE(st.numel == 2LL * nchunks, B3D_ERR_SHAPE, "stats: wrong size");
     B3D_TRY(vecF(gamma_, gm.F, "gamma", &ga));
     B3D_TRY(vecF(beta_, gm.F, "beta", &be));
-    B3D_NPL(gm.npl, (block_epilogue_fwd_kernel<true, kN><<<block_grid(gm, nchunks), kBT, 0, s>>>(
-        (const float*)res.p, (const float*)h2.p, (const double*)st.p, (const float*)ga.p, (const float*)be.p,
-        (const float*)wsp.p, (const float*)ch.p, (float*)out.p, gm, eps)));
-  } else {
-    B3D_NPL(gm.npl, (block_epilogue_fwd_kernel<false, kN><<<block_grid(gm, nchunks), kBT, 0, s>>>(
-        (const float*)res.p, (const float*)h2.p, nullptr, nullptr, nullptr, (const float*)wsp.p,
-        (const float*)ch.p, (float*)out.p, gm, eps)));
   }
-  B3D_LAUNCH_CHECK("block_epilogue_fwd");
+  cudaStream_t s = (cudaStream_t)stream;
+  const dim3 grid = block_grid(gm, nlaunch);
+  if (out16_ == nullptr) {
+    if (has_gn) {
+      B3D_NPL(gm.npl, (block_epilogue_fwd_kernel<true, kN><<<grid, kBT, 0, s>>>(
+          (const float*)res.p, (const float*)h2.p, (const double*)st.p, (const float*)ga.p, (const float*)be.p,
+          (const float*)wsp.p, (const float*)ch.p, (float*)out.p, gm, eps)));
+    } else {
+      B3D_NPL(gm.npl, (block_epilogue_fwd_kernel<false, kN><<<grid, kBT, 0, s>>>(
+          (const float*)res.p, (const float*)h2.p, nullptr, nullptr, nullptr, (const float*)wsp.p,
+          (const float*)ch.p, (float*)out.p, gm, eps)));
+    }
+    B3D_LAUNCH_CHECK("block_epilogue_fwd");
+    return B3D_OK;
+  }
+  Twin16 tw;
+  B3D_TRY(twin_view(out16_, out16b_, res, &tw));
+  if (has_gn)
+    launch_pdl(block_fwd16_kernel<true>, grid, kBT, 0, s, (const float*)res.p, (const float*)h2.p, (const double*)st.p,
+               (const float*)ga.p, (const float*)be.p, (const float*)wsp.p, (const float*)ch.p, (float*)out.p, gm, eps,
+               tw);
+  else
+    launch_pdl(block_fwd16_kernel<false>, grid, kBT, 0, s, (const float*)res.p, (const float*)h2.p, nullptr, nullptr,
+               nullptr, (const float*)wsp.p, (const float*)ch.p, (float*)out.p, gm, eps, tw);
+  B3D_LAUNCH_CHECK("block_fwd16");
   return B3D_OK;
 }
 
@@ -954,217 +1001,69 @@ extern "C" int b3d_block_epilogue_bwd_reduce(const DLTensor* dout_, const DLTens
   return B3D_OK;
 }
 
+// With a twin dres16 / dh216 given (bf16, for the data / weight gradients of the pointwise and the second 3x3x3 conv;
+// fused-GroupNorm form only): the cell kernel; every gradient needs its fp32 output or its twin, and dbias_res /
+// dbias_h2 (nullable, both or none) receive their column sums = those convs' bias gradients.  Otherwise the float4
+// kernel: dres and, with has_gn, dh2 required.
 extern "C" int b3d_block_epilogue_bwd_apply(const DLTensor* dout_, const DLTensor* res_, const DLTensor* h2_,
                                             const DLTensor* stats_, const DLTensor* gamma_,
                                             const DLTensor* beta_, const DLTensor* wsp_, const DLTensor* chse_,
                                             const DLTensor* dgap_, const DLTensor* csum_, DLTensor* dres_,
-                                            DLTensor* dh2_, int groups, float eps, int has_gn, void* stream) {
+                                            DLTensor* dh2_, DLTensor* dres16_, DLTensor* dh216_,
+                                            DLTensor* dbias_res_, DLTensor* dbias_h2_, int groups, float eps,
+                                            int has_gn, void* stream) {
+  const bool twins = dres16_ != nullptr || dh216_ != nullptr;
+  B3D_REQUIRE((dres_ != nullptr || dres16_ != nullptr) && (!has_gn || dh2_ != nullptr || dh216_ != nullptr),
+              B3D_ERR_ARG, "block epilogue bwd: every gradient needs an output");
+  B3D_REQUIRE((dbias_res_ == nullptr) == (dbias_h2_ == nullptr), B3D_ERR_ARG,
+              "block epilogue bwd: both bias gradients or none");
+  B3D_REQUIRE(twins || dbias_res_ == nullptr, B3D_ERR_ARG, "block epilogue bwd: bias gradients without a twin");
+  B3D_REQUIRE(!twins || has_gn, B3D_ERR_UNSUPPORTED, "block epilogue bwd (P16): the fused-GroupNorm form only");
   TView dout, res, h2, st, ga, be, wsp, ch, dg, cs, dres, dh2;
   BlockGeom gm;
   int nchunks;
   B3D_TRY(view(dout_, DT_F32, -1, false, "dout", &dout));
   B3D_TRY(view(res_, DT_F32, -1, false, "res", &res));
-  B3D_TRY(view(dres_, DT_F32, -1, false, "dres", &dres));
-  B3D_REQUIRE(res.numel == dout.numel && res.numel == dres.numel, B3D_ERR_SHAPE, "block epilogue bwd: size mismatch");
-  B3D_TRY(block_geom(res, groups, has_gn != 0, &gm, &nchunks));
+  if (dres_ != nullptr) B3D_TRY(view(dres_, DT_F32, -1, false, "dres", &dres));
+  B3D_REQUIRE(res.numel == dout.numel && (dres_ == nullptr || res.numel == dres.numel), B3D_ERR_SHAPE,
+              "block epilogue bwd: size mismatch");
+  if (twins)
+    B3D_TRY(block_geom16(res, groups, true, &gm, &nchunks));
+  else
+    B3D_TRY(block_geom(res, groups, has_gn != 0, &gm, &nchunks));
   B3D_TRY(vecF(wsp_, gm.F, "wsp", &wsp));
   B3D_TRY(vecF(chse_, res.shape[0] * gm.F, "chse", &ch));
   B3D_TRY(vecF(dgap_, res.shape[0] * gm.F, "dgap", &dg));
-  cudaStream_t s = (cudaStream_t)stream;
   if (has_gn) {
     B3D_TRY(view(h2_, DT_F32, -1, false, "h2", &h2));
-    B3D_TRY(view(dh2_, DT_F32, -1, false, "dh2", &dh2));
-    B3D_REQUIRE(res.numel == h2.numel && res.numel == dh2.numel, B3D_ERR_SHAPE, "block epilogue bwd: size mismatch");
+    if (dh2_ != nullptr) B3D_TRY(view(dh2_, DT_F32, -1, false, "dh2", &dh2));
+    B3D_REQUIRE(res.numel == h2.numel && (dh2_ == nullptr || res.numel == dh2.numel), B3D_ERR_SHAPE,
+                "block epilogue bwd: size mismatch");
     B3D_TRY(view(stats_, DT_F64, -1, false, "stats", &st));
     B3D_TRY(view(csum_, DT_F64, -1, false, "csum", &cs));
     B3D_REQUIRE(st.numel == 2LL * nchunks && cs.numel == 2LL * nchunks, B3D_ERR_SHAPE, "stats/csum: wrong size");
     B3D_TRY(vecF(gamma_, gm.F, "gamma", &ga));
     B3D_TRY(vecF(beta_, gm.F, "beta", &be));
-    B3D_NPL(gm.npl, (block_epilogue_bwd_apply_kernel<true, kN><<<block_grid(gm, nchunks), kBT, 0, s>>>(
-        (const float*)dout.p, (const float*)res.p, (const float*)h2.p, (const double*)st.p, (const float*)ga.p,
-        (const float*)be.p, (const float*)wsp.p, (const float*)ch.p, (const float*)dg.p, (const double*)cs.p,
-        (float*)dres.p, (float*)dh2.p, gm, eps)));
-  } else {
-    B3D_NPL(gm.npl, (block_epilogue_bwd_apply_kernel<false, kN><<<block_grid(gm, nchunks), kBT, 0, s>>>(
-        (const float*)dout.p, (const float*)res.p, nullptr, nullptr, nullptr, nullptr, (const float*)wsp.p,
-        (const float*)ch.p, (const float*)dg.p, nullptr, (float*)dres.p, nullptr, gm, eps)));
   }
-  B3D_LAUNCH_CHECK("block_epilogue_bwd_apply");
-  return B3D_OK;
-}
-
-
-// ---- P16 twin forms ---------------------------------------------------------------------------------------------
-namespace {
-int twin16(const DLTensor* t1_, const DLTensor* t2_, const TView& x, b3d::Twin16* tw) {
-  using namespace b3d;
-  tw->p = nullptr; tw->p2 = nullptr; tw->W = (unsigned)x.shape[3]; tw->C8 = (unsigned)(x.shape[4] / 8);
-  tw->rows = (unsigned)(x.shape[1] * x.shape[2]); tw->bf16 = 1;
-  if (t1_ == nullptr) return B3D_OK;
-  P16View v;
-  B3D_TRY(view_p16(t1_, "twin", &v));
-  B3D_REQUIRE(x.ndim == 5 && v.B == x.shape[0] && v.D == x.shape[1] && v.H == x.shape[2] && v.W == x.shape[3] &&
-                  8 * v.C8 == x.shape[4], B3D_ERR_SHAPE, "twin: must be the [B, D, H, C/8, W, 8] form of the fp32 tensor");
-  tw->p = (uint4*)v.p; tw->bf16 = v.bf16;
-  if (t2_ != nullptr) {
-    P16View v2;
-    B3D_TRY(view_p16(t2_, "twin (bf16)", &v2));
-    B3D_REQUIRE(v2.bf16 && v2.B == v.B && v2.D == v.D && v2.H == v.H && v2.W == v.W && v2.C8 == v.C8, B3D_ERR_SHAPE,
-                "second twin: bf16, same shape");
-    tw->p2 = (uint4*)v2.p;
-  }
-  return B3D_OK;
-}
-// geometry of the cell kernels: T = F/8 lanes per voxel (a power of two <= 32)
-int block_geom16(const TView& res, int groups, bool has_gn, b3d::BlockGeom* gm, int* nchunks) {
-  using namespace b3d;
-  B3D_REQUIRE(res.ndim == 5, B3D_ERR_SHAPE, "block epilogue (P16): res must be [B, D, H, W, F]");
-  B3D_TRY(block_geom(res, groups, has_gn, gm, nchunks));
-  const int T = gm->F / 8;
-  B3D_REQUIRE(gm->F % 8 == 0 && T >= 1 && T <= 32 && (T & (T - 1)) == 0, B3D_ERR_UNSUPPORTED,
-              "block epilogue (P16): filters must be 8 * 2^k <= 256 (got %d)", gm->F);
-  B3D_REQUIRE(res.numel / res.shape[0] / gm->F < (1LL << 32), B3D_ERR_UNSUPPORTED, "block epilogue (P16): sample too large");
-  gm->T = T; gm->npl = 2;
-  const int vstep = kBT / T;
-  long long vp = (long long)vstep * 2;     // >= 2 voxel steps per thread; small tensors get many short CTAs, not a 16-step latency chain
-  const long long B = res.shape[0];
-  const long long cap = (3LL * sm_count() + B * gm->G - 1) / (B * gm->G);
-  const long long need = ((gm->vpc + cap - 1) / cap + vstep - 1) / vstep * vstep;
-  if (need > vp) vp = need;
-  gm->vox_per_cta = (int)vp;
-  return B3D_OK;
-}
-}  // namespace
-
-// out (nullable fp32) and the P16 twin(s) of the block output: out16 in the forward operand type, out16b (nullable) a
-// second, bf16 twin for the weight gradients of the consuming convs
-extern "C" int b3d_block_epilogue_fwd_p16(const DLTensor* res_, const DLTensor* h2_, const DLTensor* stats_,
-                                          const DLTensor* gamma_, const DLTensor* beta_, const DLTensor* wsp_,
-                                          const DLTensor* chse_, DLTensor* out_, DLTensor* out16_, DLTensor* out16b_,
-                                          int groups, float eps, int has_gn, void* stream) {
-  TView res, h2, out, st, ga, be, wsp, ch;
-  BlockGeom gm;
-  int nchunks;
-  B3D_TRY(view(res_, DT_F32, -1, false, "res", &res));
-  B3D_TRY(view(h2_, DT_F32, -1, false, "h2", &h2));
-  out.p = nullptr;
-  if (out_ != nullptr) {
-    B3D_TRY(view(out_, DT_F32, -1, false, "out", &out));
-    B3D_REQUIRE(res.numel == out.numel, B3D_ERR_SHAPE, "block epilogue: size mismatch");
-  }
-  B3D_REQUIRE(res.numel == h2.numel && out16_ != nullptr, B3D_ERR_SHAPE, "block epilogue (P16): sizes / twin required");
-  B3D_TRY(block_geom16(res, groups, has_gn != 0, &gm, &nchunks));
-  B3D_TRY(vecF(wsp_, gm.F, "wsp", &wsp));
-  B3D_TRY(vecF(chse_, res.shape[0] * gm.F, "chse", &ch));
-  Twin16 tw;
-  B3D_TRY(twin16(out16_, out16b_, res, &tw));
   cudaStream_t s = (cudaStream_t)stream;
-  if (has_gn) {
-    B3D_TRY(view(stats_, DT_F64, -1, false, "stats", &st));
-    B3D_REQUIRE(st.numel == 2LL * nchunks, B3D_ERR_SHAPE, "stats: wrong size");
-    B3D_TRY(vecF(gamma_, gm.F, "gamma", &ga));
-    B3D_TRY(vecF(beta_, gm.F, "beta", &be));
-    launch_pdl(block_fwd16_kernel<true>, block_grid(gm, nchunks), kBT, 0, s, (const float*)res.p, (const float*)h2.p, (const double*)st.p, (const float*)ga.p, (const float*)be.p,
-        (const float*)wsp.p, (const float*)ch.p, (float*)out.p, gm, eps, tw);
-  } else {
-    launch_pdl(block_fwd16_kernel<false>, block_grid(gm, nchunks), kBT, 0, s, (const float*)res.p, (const float*)h2.p, nullptr, nullptr, nullptr, (const float*)wsp.p, (const float*)ch.p,
-        (float*)out.p, gm, eps, tw);
+  if (!twins) {
+    if (has_gn) {
+      B3D_NPL(gm.npl, (block_epilogue_bwd_apply_kernel<true, kN><<<block_grid(gm, nchunks), kBT, 0, s>>>(
+          (const float*)dout.p, (const float*)res.p, (const float*)h2.p, (const double*)st.p, (const float*)ga.p,
+          (const float*)be.p, (const float*)wsp.p, (const float*)ch.p, (const float*)dg.p, (const double*)cs.p,
+          (float*)dres.p, (float*)dh2.p, gm, eps)));
+    } else {
+      B3D_NPL(gm.npl, (block_epilogue_bwd_apply_kernel<false, kN><<<block_grid(gm, nchunks), kBT, 0, s>>>(
+          (const float*)dout.p, (const float*)res.p, nullptr, nullptr, nullptr, nullptr, (const float*)wsp.p,
+          (const float*)ch.p, (const float*)dg.p, nullptr, (float*)dres.p, nullptr, gm, eps)));
+    }
+    B3D_LAUNCH_CHECK("block_epilogue_bwd_apply");
+    return B3D_OK;
   }
-  B3D_LAUNCH_CHECK("block_fwd16");
-  return B3D_OK;
-}
-
-// The same for one depth slab (slab.py): res / h2 / out16 hold voxels [vox_offset, vox_offset + D*H*W) of a volume of
-// total_vox voxels; `stats` = the all-reduced GroupNorm statistics of the whole volume's chunks, `chse` from the
-// all-reduced pooling sums.
-extern "C" int b3d_block_epilogue_fwd_p16_slab(const DLTensor* res_, const DLTensor* h2_, const DLTensor* stats_,
-                                               const DLTensor* gamma_, const DLTensor* beta_, const DLTensor* wsp_,
-                                               const DLTensor* chse_, DLTensor* out_, DLTensor* out16_, int groups,
-                                               float eps, int has_gn, long long vox_offset, long long total_vox,
-                                               void* stream) {
-  TView res, h2, out, st, ga, be, wsp, ch;
-  BlockGeom gm;
-  int nchunks;
-  B3D_TRY(view(res_, DT_F32, -1, false, "res", &res));
-  B3D_TRY(view(h2_, DT_F32, -1, false, "h2", &h2));
-  out.p = nullptr;
-  if (out_ != nullptr) {
-    B3D_TRY(view(out_, DT_F32, -1, false, "out", &out));
-    B3D_REQUIRE(res.numel == out.numel, B3D_ERR_SHAPE, "block epilogue: size mismatch");
-  }
-  B3D_REQUIRE(res.numel == h2.numel && out16_ != nullptr, B3D_ERR_SHAPE, "block epilogue (P16): sizes / twin required");
-  B3D_REQUIRE(res.ndim == 5 && res.shape[0] == 1, B3D_ERR_SHAPE, "block epilogue (slab): batch 1");
-  B3D_TRY(block_geom16(res, groups, has_gn != 0, &gm, &nchunks));
-  const long long S_local = gm.S;
-  B3D_REQUIRE(total_vox > 0 && vox_offset >= 0 && vox_offset + S_local <= total_vox && total_vox % gm.G == 0 &&
-                  total_vox < (1LL << 32), B3D_ERR_ARG, "block epilogue (slab): bad window (%lld + %lld of %lld)",
-              vox_offset, S_local, total_vox);
-  gm.S = total_vox; gm.vpc = total_vox / gm.G; gm.vshift = vox_offset; gm.S_local = S_local;
-  gm.chunk0 = (int)(vox_offset / gm.vpc);
-  const int nlaunch = (int)((vox_offset + S_local - 1) / gm.vpc) - gm.chunk0 + 1;     // chunks that intersect the slab
-  B3D_TRY(vecF(wsp_, gm.F, "wsp", &wsp));
-  B3D_TRY(vecF(chse_, gm.F, "chse", &ch));
-  Twin16 tw;
-  B3D_TRY(twin16(out16_, nullptr, res, &tw));
-  cudaStream_t s = (cudaStream_t)stream;
-  if (has_gn) {
-    B3D_TRY(view(stats_, DT_F64, -1, false, "stats", &st));
-    B3D_REQUIRE(st.numel == 2LL * nchunks, B3D_ERR_SHAPE, "stats: wrong size");
-    B3D_TRY(vecF(gamma_, gm.F, "gamma", &ga));
-    B3D_TRY(vecF(beta_, gm.F, "beta", &be));
-    launch_pdl(block_fwd16_kernel<true>, block_grid(gm, nlaunch), kBT, 0, s, (const float*)res.p, (const float*)h2.p, (const double*)st.p, (const float*)ga.p, (const float*)be.p,
-        (const float*)wsp.p, (const float*)ch.p, (float*)out.p, gm, eps, tw);
-  } else {
-    launch_pdl(block_fwd16_kernel<false>, block_grid(gm, nlaunch), kBT, 0, s, (const float*)res.p, (const float*)h2.p, nullptr, nullptr, nullptr, (const float*)wsp.p, (const float*)ch.p,
-        (float*)out.p, gm, eps, tw);
-  }
-  B3D_LAUNCH_CHECK("block_fwd16 (slab)");
-  return B3D_OK;
-}
-
-// dres / dh2 (nullable fp32), their bf16 P16 twins for the data / weight gradients of the pointwise and the second 3x3x3
-// conv, and dbias_res / dbias_h2 (nullable, both or none): their column sums = those convs' bias gradients.  GN form only.
-extern "C" int b3d_block_epilogue_bwd_apply_p16(const DLTensor* dout_, const DLTensor* res_, const DLTensor* h2_,
-                                                const DLTensor* stats_, const DLTensor* gamma_,
-                                                const DLTensor* beta_, const DLTensor* wsp_, const DLTensor* chse_,
-                                                const DLTensor* dgap_, const DLTensor* csum_, DLTensor* dres_,
-                                                DLTensor* dh2_, DLTensor* dres16_, DLTensor* dh216_,
-                                                DLTensor* dbias_res_, DLTensor* dbias_h2_, int groups, float eps,
-                                                int has_gn, void* stream) {
-  TView dout, res, h2, st, ga, be, wsp, ch, dg, cs, dres, dh2;
-  BlockGeom gm;
-  int nchunks;
-  B3D_REQUIRE(has_gn, B3D_ERR_UNSUPPORTED, "block epilogue bwd (P16): the fused-GroupNorm form only");
-  B3D_TRY(view(dout_, DT_F32, -1, false, "dout", &dout));
-  B3D_TRY(view(res_, DT_F32, -1, false, "res", &res));
-  B3D_TRY(view(h2_, DT_F32, -1, false, "h2", &h2));
-  B3D_REQUIRE(res.numel == dout.numel && res.numel == h2.numel, B3D_ERR_SHAPE, "block epilogue bwd: size mismatch");
-  dres.p = nullptr; dh2.p = nullptr;
-  if (dres_ != nullptr) {
-    B3D_TRY(view(dres_, DT_F32, -1, false, "dres", &dres));
-    B3D_REQUIRE(res.numel == dres.numel, B3D_ERR_SHAPE, "block epilogue bwd: size mismatch");
-  }
-  if (dh2_ != nullptr) {
-    B3D_TRY(view(dh2_, DT_F32, -1, false, "dh2", &dh2));
-    B3D_REQUIRE(res.numel == dh2.numel, B3D_ERR_SHAPE, "block epilogue bwd: size mismatch");
-  }
-  B3D_REQUIRE((dres_ != nullptr || dres16_ != nullptr) && (dh2_ != nullptr || dh216_ != nullptr), B3D_ERR_ARG,
-              "block epilogue bwd: every gradient needs an output");
-  B3D_TRY(block_geom16(res, groups, true, &gm, &nchunks));
-  B3D_TRY(vecF(wsp_, gm.F, "wsp", &wsp));
-  B3D_TRY(vecF(chse_, res.shape[0] * gm.F, "chse", &ch));
-  B3D_TRY(vecF(dgap_, res.shape[0] * gm.F, "dgap", &dg));
-  B3D_TRY(view(stats_, DT_F64, -1, false, "stats", &st));
-  B3D_TRY(view(csum_, DT_F64, -1, false, "csum", &cs));
-  B3D_REQUIRE(st.numel == 2LL * nchunks && cs.numel == 2LL * nchunks, B3D_ERR_SHAPE, "stats/csum: wrong size");
-  B3D_TRY(vecF(gamma_, gm.F, "gamma", &ga));
-  B3D_TRY(vecF(beta_, gm.F, "beta", &be));
   Twin16 tr, th;
-  B3D_TRY(twin16(dres16_, nullptr, res, &tr));
-  B3D_TRY(twin16(dh216_, nullptr, res, &th));
-  cudaStream_t s = (cudaStream_t)stream;
+  B3D_TRY(twin_view(dres16_, nullptr, res, &tr));
+  B3D_TRY(twin_view(dh216_, nullptr, res, &th));
   float *dbr = nullptr, *dbh = nullptr;
-  B3D_REQUIRE((dbias_res_ == nullptr) == (dbias_h2_ == nullptr), B3D_ERR_ARG, "block epilogue bwd: both bias gradients or none");
   if (dbias_res_ != nullptr) {
     TView t;
     B3D_TRY(vecF(dbias_res_, gm.F, "dbias_res", &t));

@@ -99,4 +99,4 @@ int sm_count() {
 }  // namespace b3d
 
 extern "C" const char* b3d_last_error(void) { return b3d::g_err; }
-extern "C" int b3d_abi_version(void) { return 1; }
+extern "C" int b3d_abi_version(void) { return 2; }

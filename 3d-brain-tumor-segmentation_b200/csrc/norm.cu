@@ -646,118 +646,121 @@ static int check_affine(const DLTensor* t, int C, const char* name, TView* v) {
   return B3D_OK;
 }
 
+// gn_geom for x as a whole (total_vox = 0) or as the window [vox_offset, vox_offset + voxels of x) of a batch-1 volume
+// of total_vox voxels (depth-slab inference): gm then describes the chunks of the WHOLE volume, which need not line up
+// with the window, and *shift is the window's first element in the volume.
+static int gn_window(const TView& x, int groups, long long vox_offset, long long total_vox, ChunkGeom* gm,
+                     int* nchunks, long long* shift) {
+  B3D_TRY(gn_geom(x, groups, gm, nchunks));
+  *shift = 0;
+  if (total_vox == 0) return B3D_OK;
+  B3D_REQUIRE(x.shape[0] == 1, B3D_ERR_SHAPE, "GroupNorm window: batch 1");
+  B3D_REQUIRE(vox_offset >= 0 && vox_offset + x.numel / gm->C <= total_vox, B3D_ERR_SHAPE,
+              "GroupNorm window: bad offset / total (%lld, %lld voxels)", vox_offset, total_vox);
+  gm->L = total_vox * gm->C / groups;
+  gm->inv_L = 1.0f / (float)gm->L;
+  *shift = vox_offset * gm->C;
+  return B3D_OK;
+}
+
+// the cell kernels need whole cells per chunk, power-of-two octet counts dividing the thread block (so that a thread
+// keeps its channel octet over the grid-stride loop) and affine indices that repeat within a cell stride
+static int cell_ok(const ChunkGeom& gm, const TView& x) {
+  const int C8 = gm.C / 8;
+  B3D_REQUIRE(gm.C % 8 == 0 && gm.L % 8 == 0 && (C8 & (C8 - 1)) == 0 && C8 <= kThreads &&
+                  ((kThreads * kCell) % gm.cg == 0) && (gm.cg % 8 == 0 || 8 % gm.cg == 0) &&
+                  (x.numel / x.shape[0]) / 8 < (1LL << 32) && ((uintptr_t)x.p & 15) == 0,
+              B3D_ERR_UNSUPPORTED, "GroupNorm twin kernels: C = 8 * 2^k channels, 8 | chunk length (C=%d, L=%lld)", gm.C,
+              (long long)gm.L);
+  return B3D_OK;
+}
+
 }  // namespace b3d
 
 using namespace b3d;
 
-extern "C" int b3d_gn_stats(const DLTensor* x_, DLTensor* stats_, int groups, void* stream) {
+// total_vox = 0: x is the whole tensor; otherwise the window [vox_offset, vox_offset + voxels of x) of a batch-1 volume
+// of total_vox voxels, and `stats` receives the window's PARTIAL sums per chunk of the whole volume (see gn_window)
+extern "C" int b3d_gn_stats(const DLTensor* x_, DLTensor* stats_, int groups, long long vox_offset, long long total_vox,
+                            void* stream) {
   TView x, st;
   ChunkGeom gm;
   int nchunks;
+  long long shift;
   B3D_TRY(view(x_, DT_F32, -1, false, "x", &x));
-  B3D_TRY(gn_geom(x, groups, &gm, &nchunks));
+  B3D_TRY(gn_window(x, groups, vox_offset, total_vox, &gm, &nchunks, &shift));
   B3D_TRY(check_stats(stats_, nchunks, "stats", &st));
   cudaStream_t s = (cudaStream_t)stream;
   B3D_TRY(cuda_ok(cudaMemsetAsync(st.p, 0, sizeof(double) * 2 * nchunks, s), "memset stats"));
-  const bool v4 = (gm.L % 4 == 0) && (((uintptr_t)x.p & 15) == 0);
+  const bool v4 = (gm.L % 4 == 0) && (shift % 4 == 0) && (((uintptr_t)x.p & 15) == 0);
   if (v4)
-    gn_stats_kernel<4><<<gn_grid(gm, nchunks, 4, true), kThreads, 0, s>>>((const float*)x.p, (double*)st.p, gm.L, 0,
+    gn_stats_kernel<4><<<gn_grid(gm, nchunks, 4, true), kThreads, 0, s>>>((const float*)x.p, (double*)st.p, gm.L, shift,
                                                                           x.numel);
   else
-    gn_stats_kernel<1><<<gn_grid(gm, nchunks, 1, true), kThreads, 0, s>>>((const float*)x.p, (double*)st.p, gm.L, 0,
+    gn_stats_kernel<1><<<gn_grid(gm, nchunks, 1, true), kThreads, 0, s>>>((const float*)x.p, (double*)st.p, gm.L, shift,
                                                                           x.numel);
   B3D_LAUNCH_CHECK("gn_stats");
   return B3D_OK;
 }
 
-extern "C" int b3d_gn_apply(const DLTensor* x_, const DLTensor* stats_, const DLTensor* gamma_,
-                            const DLTensor* beta_, DLTensor* y_, int groups, float eps, int relu, void* stream) {
+// With the twin y16 (and y16b) given: the cell kernel, y nullable; otherwise the element kernel, y required.  The
+// window as in b3d_gn_stats, with `stats` the (all-reduced) statistics of the whole volume.
+extern "C" int b3d_gn_apply(const DLTensor* x_, const DLTensor* stats_, const DLTensor* gamma_, const DLTensor* beta_,
+                            DLTensor* y_, DLTensor* y16_, DLTensor* y16b_, int groups, float eps, int relu,
+                            long long vox_offset, long long total_vox, void* stream) {
+  B3D_REQUIRE(y16_ != nullptr || y16b_ == nullptr, B3D_ERR_ARG, "gn_apply: y16b without y16");
   TView x, y, st, ga, be;
   ChunkGeom gm;
   int nchunks;
+  long long shift;
   B3D_TRY(view(x_, DT_F32, -1, false, "x", &x));
-  B3D_TRY(view(y_, DT_F32, -1, false, "y", &y));
-  B3D_REQUIRE(x.numel == y.numel, B3D_ERR_SHAPE, "gn_apply: x/y size mismatch");
-  B3D_TRY(gn_geom(x, groups, &gm, &nchunks));
+  if (y_ != nullptr || y16_ == nullptr) {
+    B3D_TRY(view(y_, DT_F32, -1, false, "y", &y));
+    B3D_REQUIRE(x.numel == y.numel, B3D_ERR_SHAPE, "gn_apply: x/y size mismatch");
+  }
+  B3D_TRY(gn_window(x, groups, vox_offset, total_vox, &gm, &nchunks, &shift));
   B3D_TRY(check_stats(stats_, nchunks, "stats", &st));
   B3D_TRY(check_affine(gamma_, gm.C, "gamma", &ga));
   B3D_TRY(check_affine(beta_, gm.C, "beta", &be));
   cudaStream_t s = (cudaStream_t)stream;
-  const bool v4 = (gm.L % 4 == 0) && ((((uintptr_t)x.p | (uintptr_t)y.p) & 15) == 0);
+  if (y16_ == nullptr) {
+    const bool v4 = (gm.L % 4 == 0) && (shift % 4 == 0) && ((((uintptr_t)x.p | (uintptr_t)y.p) & 15) == 0);
 #define LAUNCH(V, R)                                                                                     \
   gn_apply_kernel<V, R><<<gn_grid(gm, nchunks, V), kThreads, 0, s>>>(                                    \
-      (const float*)x.p, (const double*)st.p, (const float*)ga.p, (const float*)be.p, (float*)y.p, gm, eps, 0,   \
+      (const float*)x.p, (const double*)st.p, (const float*)ga.p, (const float*)be.p, (float*)y.p, gm, eps, shift, \
       x.numel)
-  if (v4) {
-    if (relu) LAUNCH(4, true); else LAUNCH(4, false);
-  } else {
-    if (relu) LAUNCH(1, true); else LAUNCH(1, false);
-  }
+    if (v4) {
+      if (relu) LAUNCH(4, true); else LAUNCH(4, false);
+    } else {
+      if (relu) LAUNCH(1, true); else LAUNCH(1, false);
+    }
 #undef LAUNCH
-  B3D_LAUNCH_CHECK("gn_apply");
-  return B3D_OK;
-}
-
-// ---- depth-slab forms (whole-volume inference sharded along D; batch 1): x is this rank's contiguous part
-// [elem_offset, elem_offset + numel) of a sample with total_elems elements.  gn_stats_slab writes this slab's
-// PARTIAL (sum, sum^2) per chunk of the WHOLE sample (the caller all-reduces them); gn_apply_slab normalises the
-// slab with the reduced statistics.  Chunk boundaries need not coincide with slab boundaries.
-static int slab_geom(const TView& x, int groups, long long elem_offset, long long total_elems, ChunkGeom* gm) {
-  const int C = (int)x.shape[x.ndim - 1];
-  B3D_REQUIRE(groups >= 1 && C >= groups && C % groups == 0, B3D_ERR_SHAPE,
-              "Number of groups (%d) must be a multiple of the number of channels (%d).", groups, C);
-  B3D_REQUIRE(total_elems % groups == 0 && elem_offset >= 0 && elem_offset + x.numel <= total_elems &&
-                  elem_offset % C == 0 && total_elems % C == 0,
-              B3D_ERR_SHAPE, "gn slab: bad offset / total (%lld, %lld)", elem_offset, total_elems);
-  gm->L = total_elems / groups; gm->C = C; gm->cg = C / groups; gm->G = groups; gm->inv_L = 1.0f / (float)gm->L;
-  return B3D_OK;
-}
-
-extern "C" int b3d_gn_stats_slab(const DLTensor* x_, DLTensor* stats_, int groups, long long elem_offset,
-                                 long long total_elems, void* stream) {
-  TView x, st;
-  ChunkGeom gm;
-  B3D_TRY(view(x_, DT_F32, -1, false, "x", &x));
-  B3D_TRY(slab_geom(x, groups, elem_offset, total_elems, &gm));
-  B3D_TRY(check_stats(stats_, groups, "stats", &st));
-  cudaStream_t s = (cudaStream_t)stream;
-  B3D_TRY(cuda_ok(cudaMemsetAsync(st.p, 0, sizeof(double) * 2 * groups, s), "memset stats"));
-  const bool v4 = (gm.L % 4 == 0) && (elem_offset % 4 == 0) && (((uintptr_t)x.p & 15) == 0);
-  if (v4)
-    gn_stats_kernel<4><<<gn_grid(gm, groups, 4, true), kThreads, 0, s>>>((const float*)x.p, (double*)st.p, gm.L,
-                                                                         elem_offset, x.numel);
+    B3D_LAUNCH_CHECK("gn_apply");
+    return B3D_OK;
+  }
+  B3D_REQUIRE(((uintptr_t)y.p & 15) == 0, B3D_ERR_SHAPE, "gn_apply: y must be 16-byte aligned");
+  B3D_TRY(cell_ok(gm, x));
+  B3D_REQUIRE(shift % kCell == 0 && x.numel % kCell == 0, B3D_ERR_LAYOUT, "gn_apply: window not cell-aligned");
+  Twin16 tw;
+  B3D_TRY(twin_view(y16_, y16b_, x, &tw));
+  dim3 grid = gn_grid16(gm, nchunks);
+  long long n_local = -1;
+  int c0 = 0;
+  if (total_vox != 0) {      // only the chunks that intersect the window, each CTA row sized for the part it can hold
+    c0 = (int)(shift / gm.L);
+    const int nc = (int)((shift + x.numel - 1) / gm.L) - c0 + 1;
+    ChunkGeom gl = gm;
+    if (x.numel < gl.L) gl.L = (x.numel + kCell - 1) / kCell * kCell;
+    grid = gn_grid16(gl, nc);
+    n_local = x.numel;
+  }
+  if (relu)
+    launch_pdl(gn_apply16_kernel<true>, grid, kThreads, 0, s, (const float*)x.p, (const double*)st.p, (const float*)ga.p,
+               (const float*)be.p, (float*)y.p, gm, eps, tw, shift, n_local, c0);
   else
-    gn_stats_kernel<1><<<gn_grid(gm, groups, 1, true), kThreads, 0, s>>>((const float*)x.p, (double*)st.p, gm.L,
-                                                                         elem_offset, x.numel);
-  B3D_LAUNCH_CHECK("gn_stats_slab");
-  return B3D_OK;
-}
-
-extern "C" int b3d_gn_apply_slab(const DLTensor* x_, const DLTensor* stats_, const DLTensor* gamma_,
-                                 const DLTensor* beta_, DLTensor* y_, int groups, float eps, int relu,
-                                 long long elem_offset, long long total_elems, void* stream) {
-  TView x, y, st, ga, be;
-  ChunkGeom gm;
-  B3D_TRY(view(x_, DT_F32, -1, false, "x", &x));
-  B3D_TRY(view(y_, DT_F32, -1, false, "y", &y));
-  B3D_REQUIRE(x.numel == y.numel, B3D_ERR_SHAPE, "gn_apply_slab: x/y size mismatch");
-  B3D_TRY(slab_geom(x, groups, elem_offset, total_elems, &gm));
-  B3D_TRY(check_stats(stats_, groups, "stats", &st));
-  B3D_TRY(check_affine(gamma_, gm.C, "gamma", &ga));
-  B3D_TRY(check_affine(beta_, gm.C, "beta", &be));
-  cudaStream_t s = (cudaStream_t)stream;
-  const bool v4 = (gm.L % 4 == 0) && (elem_offset % 4 == 0) && ((((uintptr_t)x.p | (uintptr_t)y.p) & 15) == 0);
-#define LAUNCH(V, R)                                                                                     \
-  gn_apply_kernel<V, R><<<gn_grid(gm, groups, V), kThreads, 0, s>>>(                                     \
-      (const float*)x.p, (const double*)st.p, (const float*)ga.p, (const float*)be.p, (float*)y.p, gm, eps,     \
-      elem_offset, x.numel)
-  if (v4) {
-    if (relu) LAUNCH(4, true); else LAUNCH(4, false);
-  } else {
-    if (relu) LAUNCH(1, true); else LAUNCH(1, false);
-  }
-#undef LAUNCH
-  B3D_LAUNCH_CHECK("gn_apply_slab");
+    launch_pdl(gn_apply16_kernel<false>, grid, kThreads, 0, s, (const float*)x.p, (const double*)st.p, (const float*)ga.p,
+               (const float*)be.p, (float*)y.p, gm, eps, tw, shift, n_local, c0);
+  B3D_LAUNCH_CHECK("gn_apply16");
   return B3D_OK;
 }
 
@@ -811,148 +814,49 @@ extern "C" int b3d_gn_bwd_reduce(const DLTensor* dy_, const DLTensor* x_, const 
   return B3D_OK;
 }
 
+// With the twin dx16 given: the cell kernel, dx nullable, and dbias (nullable, fp32 [C]) = column sums of dx = the bias
+// gradient of the conv that produced x; otherwise the element kernel, dx required.
 extern "C" int b3d_gn_bwd_apply(const DLTensor* dy_, const DLTensor* x_, const DLTensor* stats_,
                                 const DLTensor* gamma_, const DLTensor* beta_, const DLTensor* csum_,
-                                DLTensor* dx_, int groups, float eps, int relu, void* stream) {
+                                DLTensor* dx_, DLTensor* dx16_, DLTensor* dbias_, int groups, float eps, int relu,
+                                void* stream) {
+  B3D_REQUIRE(dx_ != nullptr || dx16_ != nullptr, B3D_ERR_ARG, "gn_bwd_apply: neither dx nor dx16 given");
+  B3D_REQUIRE(dbias_ == nullptr || dx16_ != nullptr, B3D_ERR_ARG, "gn_bwd_apply: dbias without dx16");
   TView x, dy, dx, st, ga, be, cs;
   ChunkGeom gm;
   int nchunks;
   B3D_TRY(view(x_, DT_F32, -1, false, "x", &x));
   B3D_TRY(view(dy_, DT_F32, -1, false, "dy", &dy));
-  B3D_TRY(view(dx_, DT_F32, -1, false, "dx", &dx));
-  B3D_REQUIRE(x.numel == dy.numel && x.numel == dx.numel, B3D_ERR_SHAPE, "gn_bwd_apply: size mismatch");
+  if (dx_ != nullptr) B3D_TRY(view(dx_, DT_F32, -1, false, "dx", &dx));
+  B3D_REQUIRE(x.numel == dy.numel && (dx_ == nullptr || x.numel == dx.numel), B3D_ERR_SHAPE,
+              "gn_bwd_apply: size mismatch");
   B3D_TRY(gn_geom(x, groups, &gm, &nchunks));
   B3D_TRY(check_stats(stats_, nchunks, "stats", &st));
   B3D_TRY(check_stats(csum_, nchunks, "csum", &cs));
   B3D_TRY(check_affine(gamma_, gm.C, "gamma", &ga));
   B3D_TRY(check_affine(beta_, gm.C, "beta", &be));
   cudaStream_t s = (cudaStream_t)stream;
-  const bool v4 =
-      (gm.L % 4 == 0) && ((((uintptr_t)x.p | (uintptr_t)dy.p | (uintptr_t)dx.p) & 15) == 0);
+  if (dx16_ == nullptr) {
+    const bool v4 =
+        (gm.L % 4 == 0) && ((((uintptr_t)x.p | (uintptr_t)dy.p | (uintptr_t)dx.p) & 15) == 0);
 #define LAUNCH(V, R)                                                                                       \
   gn_bwd_apply_kernel<V, R><<<gn_grid(gm, nchunks, V), kThreads, 0, s>>>(                                  \
       (const float*)dy.p, (const float*)x.p, (const double*)st.p, (const float*)ga.p, (const float*)be.p, \
       (const double*)cs.p, (float*)dx.p, gm, eps)
-  if (v4) {
-    if (relu) LAUNCH(4, true); else LAUNCH(4, false);
-  } else {
-    if (relu) LAUNCH(1, true); else LAUNCH(1, false);
-  }
+    if (v4) {
+      if (relu) LAUNCH(4, true); else LAUNCH(4, false);
+    } else {
+      if (relu) LAUNCH(1, true); else LAUNCH(1, false);
+    }
 #undef LAUNCH
-  B3D_LAUNCH_CHECK("gn_bwd_apply");
-  return B3D_OK;
-}
-
-
-// ---- P16 twin forms (see the kernels above) ----------------------------------------------------------------------
-namespace {
-// the cell kernels need whole cells per chunk, power-of-two octet counts dividing the thread block (so that a thread
-// keeps its channel octet over the grid-stride loop) and affine indices that repeat within a cell stride
-int cell_ok(const b3d::ChunkGeom& gm, const TView& x) {
-  using namespace b3d;
-  const int C8 = gm.C / 8;
-  B3D_REQUIRE(gm.C % 8 == 0 && gm.L % 8 == 0 && (C8 & (C8 - 1)) == 0 && C8 <= kThreads &&
-                  ((kThreads * kCell) % gm.cg == 0) && (gm.cg % 8 == 0 || 8 % gm.cg == 0) &&
-                  (x.numel / x.shape[0]) / 8 < (1LL << 32) && ((uintptr_t)x.p & 15) == 0,
-              B3D_ERR_UNSUPPORTED, "GroupNorm twin kernels: C = 8 * 2^k channels, 8 | chunk length (C=%d, L=%lld)", gm.C,
-              (long long)gm.L);
-  return B3D_OK;
-}
-}  // namespace
-
-// y (nullable fp32) and the P16 twin(s) of GroupNorm(+ReLU): y16 in the forward operand type, y16b (nullable) a second,
-// bf16 twin for the weight gradient of the consuming conv
-extern "C" int b3d_gn_apply_p16(const DLTensor* x_, const DLTensor* stats_, const DLTensor* gamma_,
-                                const DLTensor* beta_, DLTensor* y_, DLTensor* y16_, DLTensor* y16b_, int groups,
-                                float eps, int relu, void* stream) {
-  TView x, y, st, ga, be;
-  ChunkGeom gm;
-  int nchunks;
-  B3D_TRY(view(x_, DT_F32, 5, false, "x", &x));
-  y.p = nullptr;
-  if (y_ != nullptr) {
-    B3D_TRY(view(y_, DT_F32, -1, false, "y", &y));
-    B3D_REQUIRE(x.numel == y.numel && ((uintptr_t)y.p & 15) == 0, B3D_ERR_SHAPE, "gn_apply: x/y size mismatch");
+    B3D_LAUNCH_CHECK("gn_bwd_apply");
+    return B3D_OK;
   }
-  B3D_TRY(gn_geom(x, groups, &gm, &nchunks));
-  B3D_TRY(check_stats(stats_, nchunks, "stats", &st));
-  B3D_TRY(check_affine(gamma_, gm.C, "gamma", &ga));
-  B3D_TRY(check_affine(beta_, gm.C, "beta", &be));
-  B3D_TRY(cell_ok(gm, x));
-  Twin16 tw;
-  B3D_TRY(twin_view(y16_, y16b_, x, &tw));
-  cudaStream_t s = (cudaStream_t)stream;
-  if (relu)
-    launch_pdl(gn_apply16_kernel<true>, gn_grid16(gm, nchunks), kThreads, 0, s, (const float*)x.p, (const double*)st.p, (const float*)ga.p, (const float*)be.p, (float*)y.p, gm, eps, tw, 0, -1, 0);
-  else
-    launch_pdl(gn_apply16_kernel<false>, gn_grid16(gm, nchunks), kThreads, 0, s, (const float*)x.p, (const double*)st.p, (const float*)ga.p, (const float*)be.p, (float*)y.p, gm, eps, tw, 0, -1, 0);
-  B3D_LAUNCH_CHECK("gn_apply16");
-  return B3D_OK;
-}
-
-// The same for one depth slab (slab.py): x / y / y16 hold the flat elements [elem_offset, elem_offset + numel) of a
-// volume of total_elems elements per sample, `stats` the (all-reduced) chunk statistics of the WHOLE volume.
-extern "C" int b3d_gn_apply_p16_slab(const DLTensor* x_, const DLTensor* stats_, const DLTensor* gamma_,
-                                     const DLTensor* beta_, DLTensor* y_, DLTensor* y16_, int groups, float eps,
-                                     int relu, long long elem_offset, long long total_elems, void* stream) {
-  TView x, y, st, ga, be;
-  ChunkGeom gm;
-  B3D_TRY(view(x_, DT_F32, 5, false, "x", &x));
-  B3D_REQUIRE(x.shape[0] == 1, B3D_ERR_SHAPE, "gn_apply (slab): batch 1");
-  y.p = nullptr;
-  if (y_ != nullptr) {
-    B3D_TRY(view(y_, DT_F32, -1, false, "y", &y));
-    B3D_REQUIRE(x.numel == y.numel && ((uintptr_t)y.p & 15) == 0, B3D_ERR_SHAPE, "gn_apply: x/y size mismatch");
-  }
-  B3D_TRY(slab_geom(x, groups, elem_offset, total_elems, &gm));
-  B3D_TRY(check_stats(stats_, groups, "stats", &st));
-  B3D_TRY(check_affine(gamma_, gm.C, "gamma", &ga));
-  B3D_TRY(check_affine(beta_, gm.C, "beta", &be));
-  B3D_TRY(cell_ok(gm, x));
-  B3D_REQUIRE(elem_offset % kCell == 0 && x.numel % kCell == 0, B3D_ERR_LAYOUT, "gn_apply (slab): window not cell-aligned");
-  Twin16 tw;
-  B3D_TRY(twin_view(y16_, nullptr, x, &tw));
-  cudaStream_t s = (cudaStream_t)stream;
-  const int c0 = (int)(elem_offset / gm.L), nc = (int)((elem_offset + x.numel - 1) / gm.L) - c0 + 1;
-  ChunkGeom gl = gm;                               // grid sized for the part of a chunk a slab can hold
-  if (x.numel < gl.L) gl.L = (x.numel + kCell - 1) / kCell * kCell;
-  const dim3 grid = gn_grid16(gl, nc);
-  if (relu)
-    launch_pdl(gn_apply16_kernel<true>, grid, kThreads, 0, s, (const float*)x.p, (const double*)st.p, (const float*)ga.p, (const float*)be.p, (float*)y.p, gm, eps, tw,
-        elem_offset, x.numel, c0);
-  else
-    launch_pdl(gn_apply16_kernel<false>, grid, kThreads, 0, s, (const float*)x.p, (const double*)st.p, (const float*)ga.p, (const float*)be.p, (float*)y.p, gm, eps, tw,
-        elem_offset, x.numel, c0);
-  B3D_LAUNCH_CHECK("gn_apply16 (slab)");
-  return B3D_OK;
-}
-
-// dx (nullable fp32), its bf16 P16 twin for the data / weight gradient of the conv that produced x, and dbias (nullable,
-// fp32 [C]) = column sums of dx = that conv's bias gradient
-extern "C" int b3d_gn_bwd_apply_p16(const DLTensor* dy_, const DLTensor* x_, const DLTensor* stats_,
-                                    const DLTensor* gamma_, const DLTensor* beta_, const DLTensor* csum_,
-                                    DLTensor* dx_, DLTensor* dx16_, DLTensor* dbias_, int groups, float eps, int relu,
-                                    void* stream) {
-  TView x, dy, dx, st, ga, be, cs;
-  ChunkGeom gm;
-  int nchunks;
-  B3D_TRY(view(x_, DT_F32, 5, false, "x", &x));
-  B3D_TRY(view(dy_, DT_F32, -1, false, "dy", &dy));
-  dx.p = nullptr;
-  if (dx_ != nullptr) {
-    B3D_TRY(view(dx_, DT_F32, -1, false, "dx", &dx));
-    B3D_REQUIRE(x.numel == dx.numel && ((uintptr_t)dx.p & 15) == 0, B3D_ERR_SHAPE, "gn_bwd_apply: size mismatch");
-  }
-  B3D_REQUIRE(x.numel == dy.numel && ((uintptr_t)dy.p & 15) == 0, B3D_ERR_SHAPE, "gn_bwd_apply: size mismatch");
-  B3D_TRY(gn_geom(x, groups, &gm, &nchunks));
-  B3D_TRY(check_stats(stats_, nchunks, "stats", &st));
-  B3D_TRY(check_stats(csum_, nchunks, "csum", &cs));
-  B3D_TRY(check_affine(gamma_, gm.C, "gamma", &ga));
-  B3D_TRY(check_affine(beta_, gm.C, "beta", &be));
+  B3D_REQUIRE((((uintptr_t)dy.p | (uintptr_t)dx.p) & 15) == 0, B3D_ERR_SHAPE,
+              "gn_bwd_apply: dy / dx must be 16-byte aligned");
   B3D_TRY(cell_ok(gm, x));
   Twin16 tw;
   B3D_TRY(twin_view(dx16_, nullptr, x, &tw));
-  cudaStream_t s = (cudaStream_t)stream;
   float* db = nullptr;
   if (dbias_ != nullptr) {
     TView dbv;

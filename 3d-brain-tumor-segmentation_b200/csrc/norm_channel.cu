@@ -376,11 +376,8 @@ extern "C" int b3d_gn_channel_apply_slab(const DLTensor* x_, const DLTensor* sta
   B3D_TRY(vecn(stats_, DT_F64, 2LL * groups, "stats", &st));
   B3D_TRY(vecn(gamma_, DT_F32, C, "gamma", &ga));
   B3D_TRY(vecn(beta_, DT_F32, C, "beta", &be));
-  // the cell position is advanced for y-only calls too, so its geometry is that of x
   Twin16 tw;
-  tw.p = nullptr; tw.p2 = nullptr; tw.bf16 = 0;
-  tw.W = (unsigned)x.shape[3]; tw.C8 = (unsigned)(C / 8); tw.rows = (unsigned)(x.shape[1] * x.shape[2]);
-  if (y16_ != nullptr) B3D_TRY(twin_view(y16_, nullptr, x, &tw));
+  B3D_TRY(twin_view(y16_, nullptr, x, &tw));
   const int q = C / 8;
   const int threads = q >= 256 ? q : (256 / q) * q;
   long long blocks = (ncells + (long long)threads * kSlabIter - 1) / ((long long)threads * kSlabIter);

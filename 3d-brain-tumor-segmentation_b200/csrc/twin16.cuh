@@ -1,7 +1,8 @@
 // b3d — the store side of a P16 operand twin ([B, D, H, C/8, W, 8], common.cuh) for kernels that stream a fp32 NDHWC
 // tensor one 16-byte CELL (8 consecutive channels of a voxel) per thread and step: the twin position of a thread's
 // first cell, its advance by a loop stride without a division, the 16-bit packing and the store.  Shared by the
-// GroupNorm apply kernels of both semantics (norm.cu, norm_channel.cu).
+// GroupNorm apply kernels of both semantics (norm.cu, norm_channel.cu); the block epilogue (block.cu) uses the twin
+// struct, the packing and twin_view with its own per-voxel position.
 #pragma once
 #include "common.cuh"
 
@@ -55,14 +56,18 @@ __device__ __forceinline__ void cell_store(const Twin16& o, const CellPos& k, co
     o.p2[idx] = make_uint4(pk16(v[0], v[1], 1), pk16(v[2], v[3], 1), pk16(v[4], v[5], 1), pk16(v[6], v[7], 1));
 }
 
-// Twin16 of the twin tensor(s) t1_ (and the optional bf16 t2_) of the fp32 NDHWC tensor x
+// Twin16 of the twin tensor(s) t1_ (and the optional bf16 t2_) of the fp32 NDHWC tensor x.  t1_ == nullptr: no twin
+// (p = nullptr), but the row geometry is x's all the same: kernels advance their twin position for twin-less calls too.
 inline int twin_view(const DLTensor* t1_, const DLTensor* t2_, const TView& x, Twin16* tw) {
-  tw->p = nullptr; tw->p2 = nullptr;
+  B3D_REQUIRE(x.ndim == 5, B3D_ERR_SHAPE, "twin: the fp32 tensor must be [B, D, H, W, C]");
+  tw->p = nullptr; tw->p2 = nullptr; tw->W = (unsigned)x.shape[3]; tw->C8 = (unsigned)(x.shape[4] / 8);
+  tw->rows = (unsigned)(x.shape[1] * x.shape[2]); tw->bf16 = 1;
+  if (t1_ == nullptr) return B3D_OK;
   P16View v;
   B3D_TRY(view_p16(t1_, "twin", &v));
-  B3D_REQUIRE(x.ndim == 5 && v.B == x.shape[0] && v.D == x.shape[1] && v.H == x.shape[2] && v.W == x.shape[3] &&
+  B3D_REQUIRE(v.B == x.shape[0] && v.D == x.shape[1] && v.H == x.shape[2] && v.W == x.shape[3] &&
                   8 * v.C8 == x.shape[4], B3D_ERR_SHAPE, "twin: must be the [B, D, H, C/8, W, 8] form of the fp32 tensor");
-  tw->p = (uint4*)v.p; tw->W = (unsigned)v.W; tw->C8 = (unsigned)v.C8; tw->rows = (unsigned)(v.D * v.H); tw->bf16 = v.bf16;
+  tw->p = (uint4*)v.p; tw->bf16 = v.bf16;
   if (t2_ != nullptr) {
     P16View v2;
     B3D_TRY(view_p16(t2_, "twin (bf16)", &v2));

@@ -762,17 +762,14 @@ class GroupNormFn(Function):
             raise ValueError(f"Number of groups ({groups}) must be a multiple of the number of channels ({C}).")
         if stats is None:
             stats = _new((x.shape[0], groups, 2), x, torch.float64)
-            _call("b3d_gn_stats", x, stats, groups)
+            _call("b3d_gn_stats", x, stats, groups, 0, 0)
         td = twin_dtype(False)
         L = x.numel() // x.shape[0] // groups
         twin = td is not None and p16_ok(x.shape) and L % 4 == 0
         y16 = p16_empty(x.shape, x, td) if twin else None
         y16b = p16_empty(x.shape, x, torch.bfloat16) if twin and want_wgrad_twin(td, grad_enabled) else None
         y = None if (twin and operand_only) else torch.empty_like(x)
-        if twin:
-            _call("b3d_gn_apply_p16", x, stats, gamma, beta, y, y16, y16b, groups, float(eps), int(relu))
-        else:
-            _call("b3d_gn_apply", x, stats, gamma, beta, y, groups, float(eps), int(relu))
+        _call("b3d_gn_apply", x, stats, gamma, beta, y, y16, y16b, groups, float(eps), int(relu), 0, 0)
         if y is None:
             y = virtual(x.shape, x, [y16], [y16b] if y16b is not None else None)
         ctx.save_for_backward(x, gamma, beta, stats)
@@ -802,6 +799,7 @@ class GroupNormFn(Function):
         L = x.numel() // x.shape[0] // groups
         mb = ctx.mb
         twin = td is not None and p16_ok(x.shape) and L % 4 == 0 and mb is not None
+        dx16 = dbias = None
         if twin:
             dx16 = p16_empty(x.shape, x, td)
             bias = mb["bias"]
@@ -809,14 +807,14 @@ class GroupNormFn(Function):
             dbias = _grad_target(bias) if fused_bias else None
             # the producing conv takes its weight gradient through the fp32 entry point (narrow layers): keep fp32 too
             dx = torch.empty_like(x) if mb["f32_grad"] else None
-            _call("b3d_gn_bwd_apply_p16", dy, x, stats, gamma, beta, csum, dx, dx16, dbias[0] if fused_bias else None,
-                  groups, eps, relu)
+        else:
+            dx = torch.empty_like(x)
+        _call("b3d_gn_bwd_apply", dy, x, stats, gamma, beta, csum, dx, dx16, None if dbias is None else dbias[0],
+              groups, eps, relu)
+        if twin:
             mb["dy16"], mb["dbias"], mb["dy_real"] = dx16, dbias, dx is not None
             if dx is None:
                 dx = _grad_placeholder(x)
-        else:
-            dx = torch.empty_like(x)
-            _call("b3d_gn_bwd_apply", dy, x, stats, gamma, beta, csum, dx, groups, eps, relu)
         return dx, (None if dg_direct else dgamma), (None if db_direct else dbeta), None, None, None, None, None, None
 
 
@@ -926,15 +924,13 @@ class BlockEpilogueFn(Function):
             out16 = p16_empty(res.shape, res, td)
             out16b = p16_empty(res.shape, res, torch.bfloat16) if want_wgrad_twin(td, grad_enabled) else None
             out = None if operand_only else torch.empty_like(res)
-            _call("b3d_block_epilogue_fwd_p16", res, h2, stats2, gamma2 if has_gn else None, beta2 if has_gn else None,
-                  wsp_v, chse, out, out16, out16b, groups, float(eps), int(has_gn))
-            if out is None:
-                out = virtual(res.shape, res, [out16], [out16b] if out16b is not None else None)
         else:
             out16 = out16b = None
             out = _new_act(res.shape, res)
-            _call("b3d_block_epilogue_fwd", res, h2, stats2, gamma2 if has_gn else None, beta2 if has_gn else None,
-                  wsp_v, chse, out, groups, float(eps), int(has_gn))
+        _call("b3d_block_epilogue_fwd", res, h2, stats2, gamma2 if has_gn else None, beta2 if has_gn else None,
+              wsp_v, chse, out, out16, out16b, groups, float(eps), int(has_gn), 0, 0)
+        if out is None:
+            out = virtual(res.shape, res, [out16], [out16b] if out16b is not None else None)
         ctx.save_for_backward(res, h2, stats2, gamma2, beta2, wsp, gap_sum, w1, w2, hidden, chse)
         ctx.cfg = (groups, float(eps), has_gn, inv)
         ctx.params = (gamma2, beta2, wsp, w1, w2)
@@ -968,6 +964,7 @@ class BlockEpilogueFn(Function):
         td = twin_dtype(True)
         mb_res, mb_h2 = ctx.mbs
         twin = td is not None and p16_ok(res.shape) and has_gn and mb_res is not None and mb_h2 is not None
+        dres16 = dh216 = tb_res = tb_h2 = None
         if twin:
             b_res, b_h2 = mb_res["bias"], mb_h2["bias"]
             fused_bias = b_res is not None and b_h2 is not None
@@ -977,23 +974,21 @@ class BlockEpilogueFn(Function):
             dh2 = torch.empty_like(res) if mb_h2["f32_grad"] else None
             tb_res = _grad_target(b_res) if fused_bias else None
             tb_h2 = _grad_target(b_h2) if fused_bias else None
-            _call("b3d_block_epilogue_bwd_apply_p16", dout, res, h2, stats2, gamma2, beta2, wsp_v, chse, dgap, csum,
-                  dres, dh2, dres16, dh216, tb_res[0] if fused_bias else None, tb_h2[0] if fused_bias else None,
-                  groups, eps, 1)
+        else:
+            dres = torch.empty_like(res)
+            dh2 = torch.empty_like(h2) if has_gn else None
+        _call("b3d_block_epilogue_bwd_apply", dout, res, h2 if has_gn else None, stats2,
+              gamma2 if has_gn else None, beta2 if has_gn else None, wsp_v, chse, dgap, csum, dres, dh2, dres16, dh216,
+              None if tb_res is None else tb_res[0], None if tb_h2 is None else tb_h2[0], groups, eps, int(has_gn))
+        if twin:
             mb_res["dy16"], mb_res["dbias"], mb_res["dy_real"] = dres16, tb_res, dres is not None
             mb_h2["dy16"], mb_h2["dbias"], mb_h2["dy_real"] = dh216, tb_h2, dh2 is not None
             if dres is None:
                 dres = _grad_placeholder(res)
             if dh2 is None:
                 dh2 = _grad_placeholder(res)
-        else:
-            dres = torch.empty_like(res)
-            dh2 = torch.empty_like(h2) if has_gn else None
-            _call("b3d_block_epilogue_bwd_apply", dout, res, h2 if has_gn else None, stats2,
-                  gamma2 if has_gn else None, beta2 if has_gn else None, wsp_v, chse, dgap, csum, dres, dh2,
-                  groups, eps, int(has_gn))
-            if not has_gn:
-                dh2 = dout
+        elif not has_gn:
+            dh2 = dout
         return (dres, dh2, None, None if dg_direct else dgamma, None if db_direct else dbeta,
                 None if dwsp_direct else dwsp.reshape(wsp.shape), None, None if dw1_direct else dw1,
                 None if dw2_direct else dw2, None, None, None, None)

@@ -11,7 +11,8 @@ its slab while a `SlabContext` reroutes the three operations whose result depend
       (`b3d_conv3d_fwd_halo`), the output holds only this slab's slices.
   * GroupNormalization (group_norm.py:83-124): its "groups" are contiguous 1/G chunks of the WHOLE flat volume
       (SURVEY F1) and do not line up with slabs => every rank reduces partial (sum, sum^2) per global chunk
-      (`b3d_gn_stats_slab`), one all-reduce of 2*G doubles, then `b3d_gn_apply_slab`.
+      (`b3d_gn_stats` on the slab's voxel window of the volume), one all-reduce of 2*G doubles, then `b3d_gn_apply`
+      on the same window.
       A channels_first model's groups are true channel groups (a fixed set of channels over every voxel of the
       volume): the slab's own `b3d_gn_channel_stats` are the partial sums, all-reduced the same way, then
       `b3d_gn_channel_apply_slab`.  Such a model takes and returns NCDHW tensors, so the drivers below cut and
@@ -455,8 +456,8 @@ class SlabContext:
         out = torch.empty_like(res) if keep_f32 else None
         g0, dg = self.geometry(res)
         hw = res.shape[2] * res.shape[3]
-        ops._call("b3d_block_epilogue_fwd_p16_slab", res.contiguous(), ops.materialize(h2), stats2,
-                  gamma2 if has_gn else None, beta2 if has_gn else None, wsp.reshape(F), chse, out, out16, groups,
+        ops._call("b3d_block_epilogue_fwd", res.contiguous(), ops.materialize(h2), stats2,
+                  gamma2 if has_gn else None, beta2 if has_gn else None, wsp.reshape(F), chse, out, out16, None, groups,
                   float(eps), int(has_gn), g0 * hw, dg * hw)
         if out is None:
             return ops.virtual(res.shape, res, [out16], None)
@@ -509,24 +510,25 @@ class SlabContext:
         if C % groups != 0:
             raise ValueError(f"Number of groups ({groups}) must be a multiple of the number of channels ({C}).")
         g0, dg = self.geometry(x)
-        per_slice = x.shape[2] * x.shape[3] * C
-        off, total = g0 * per_slice, dg * per_slice
+        hw = x.shape[2] * x.shape[3]
+        off, total = g0 * hw, dg * hw          # the slab's voxel window of the volume
         if stats is None:
             stats = torch.empty((1, groups, 2), dtype=torch.float64, device=x.device)
-            ops._call("b3d_gn_stats_slab", x, stats, groups, off, total)
+            ops._call("b3d_gn_stats", x, stats, groups, off, total)
             self._pending.append(stats)
         self.flush()             # the conv epilogue's (or the kernel's above) partial sums -> whole-volume statistics
-        L = total // groups
-        if self.p16 is not None and ops.p16_ok(x.shape) and L % 8 == 0 and per_slice % 8 == 0:
+        L = total * C // groups
+        if self.p16 is not None and ops.p16_ok(x.shape) and L % 8 == 0 and hw * C % 8 == 0:
             y16 = self.new_p16(x.shape, x)
             y = None if operand_only else torch.empty_like(x)
-            ops._call("b3d_gn_apply_p16_slab", x, stats, gamma, beta, y, y16, groups, float(eps), int(relu), off, total)
-            if y is None:
-                return ops.virtual(x.shape, x, [y16], None)
-            ops._attach(y, y16, None)
+        else:
+            y16, y = None, self.new_activation(x.shape, x)
+        ops._call("b3d_gn_apply", x, stats, gamma, beta, y, y16, None, groups, float(eps), int(relu), off, total)
+        if y16 is None:
             return y
-        y = self.new_activation(x.shape, x)
-        ops._call("b3d_gn_apply_slab", x, stats, gamma, beta, y, groups, float(eps), int(relu), off, total)
+        if y is None:
+            return ops.virtual(x.shape, x, [y16], None)
+        ops._attach(y, y16, None)
         return y
 
     def group_norm_channel(self, x, gamma, beta, groups, eps, relu, operand_only=False):

@@ -112,23 +112,29 @@ int b3d_conv3d_pack_many(const DLTensor* jobs /*int64 table*/, int njobs, long l
  * "group" g = g-th contiguous 1/G chunk of each sample's flat buffer; eps inside sqrt; population
  * variance.  stats: fp64 [B, G, 2] = (sum x, sum x^2).  relu=1 fuses the following Activation('relu')
  * (resnet.py:95,111; downsample.py:39; upsample.py:37).  Errors (B3D_ERR_SHAPE, reference
- * ValueError text) when C < groups or C % groups != 0 (group_norm.py:51-59). */
-int b3d_gn_stats(const DLTensor* x, DLTensor* stats, int groups, void* stream);
+ * ValueError text) when C < groups or C % groups != 0 (group_norm.py:51-59).
+ *   Window (stats, apply): total_vox = 0 => x is the whole tensor, any batch.  total_vox > 0 => x is the window
+ *     [vox_offset, vox_offset + voxels of x) of a batch-1 volume of total_vox voxels (depth-slab inference; chunk
+ *     boundaries need not coincide with the window's): gn_stats writes the window's PARTIAL (sum, sum^2) per chunk of
+ *     the WHOLE volume (fp64 [1, G, 2]; the caller all-reduces them), gn_apply normalises the window with the reduced
+ *     statistics.
+ *   P16 twins (see "P16 operand twins" below): gn_apply with y16 (fp16 | bf16) given writes it, y16b (nullable) a
+ *     second, bf16 twin for the weight gradient of the consuming conv, and y becomes nullable (NULL = twin only);
+ *     needs C = 8 * 2^k and a cell-aligned window, else B3D_ERR_UNSUPPORTED / B3D_ERR_LAYOUT.  gn_bwd_apply with dx16
+ *     (bf16) given writes the twin for the data / weight gradient of the conv that produced x, dx becomes nullable and
+ *     dbias (nullable, fp32 [C]) receives the column sums of dx = that conv's bias gradient.  Without twins y / dx
+ *     are required.  B3D_ERR_ARG: y16b without y16, dbias without dx16, neither dx nor dx16. */
+int b3d_gn_stats(const DLTensor* x, DLTensor* stats, int groups, long long vox_offset, long long total_vox,
+                 void* stream);
 int b3d_gn_apply(const DLTensor* x, const DLTensor* stats, const DLTensor* gamma, const DLTensor* beta,
-                 DLTensor* y, int groups, float eps, int relu, void* stream);
-/* depth-slab forms (batch 1): x = this rank's contiguous part [elem_offset, elem_offset + numel) of a sample of
- * total_elems elements.  stats_slab writes the slab's PARTIAL (sum, sum^2) per chunk of the WHOLE sample (fp64
- * [groups, 2]; the caller all-reduces over ranks); apply_slab normalises the slab with the reduced statistics. */
-int b3d_gn_stats_slab(const DLTensor* x, DLTensor* stats, int groups, long long elem_offset, long long total_elems,
-                      void* stream);
-int b3d_gn_apply_slab(const DLTensor* x, const DLTensor* stats, const DLTensor* gamma, const DLTensor* beta,
-                      DLTensor* y, int groups, float eps, int relu, long long elem_offset, long long total_elems,
-                      void* stream);
+                 DLTensor* y /*nullable*/, DLTensor* y16 /*nullable*/, DLTensor* y16b /*nullable*/, int groups,
+                 float eps, int relu, long long vox_offset, long long total_vox, void* stream);
 int b3d_gn_bwd_reduce(const DLTensor* dy, const DLTensor* x, const DLTensor* stats, const DLTensor* gamma,
                       const DLTensor* beta, DLTensor* dgamma, DLTensor* dbeta, DLTensor* csum /*fp64 [B,G,2]*/,
                       int groups, float eps, int relu, void* stream);
 int b3d_gn_bwd_apply(const DLTensor* dy, const DLTensor* x, const DLTensor* stats, const DLTensor* gamma,
-                     const DLTensor* beta, const DLTensor* csum, DLTensor* dx, int groups, float eps, int relu,
+                     const DLTensor* beta, const DLTensor* csum, DLTensor* dx /*nullable*/,
+                     DLTensor* dx16 /*nullable*/, DLTensor* dbias /*nullable*/, int groups, float eps, int relu,
                      void* stream);
 
 /* ---- GroupNormalization with TRUE channel groups — the reference's data_format='channels_first' semantics
@@ -151,15 +157,27 @@ int b3d_relayout(const DLTensor* src, DLTensor* dst, int to_channels_last, void*
 
 /* ---- ResnetBlock epilogue (resnet.py:121-137) --------------------------------------------------
  * chse = sigmoid(relu(gap_sum*inv_vox . W1) . W2);  out = res*(sigmoid(res.w_sp)+chse) + relu(GN2(h2)).
- * has_gn=0: h2 is already normalised+activated (stats/gamma/beta NULL). */
+ * has_gn=0: h2 is already normalised+activated (stats/gamma/beta NULL).
+ *   P16 twins (see "P16 operand twins" below): block_epilogue_fwd with out16 (fp16 | bf16) given writes it, out16b
+ *     (nullable) a second, bf16 twin for the weight gradients of the consuming convs, and out becomes nullable (NULL =
+ *     twin only).  Only then may it take a window: total_vox > 0 => res / h2 / out16 hold voxels [vox_offset,
+ *     vox_offset + D*H*W) of a batch-1 volume of total_vox voxels, stats = the all-reduced GroupNorm statistics of the
+ *     whole volume, chse from the all-reduced pooling sums; total_vox = 0 => the tensors are the whole volume.
+ *     block_epilogue_bwd_apply with dres16 / dh216 (bf16) given (has_gn = 1 only) writes the twins for the data / weight
+ *     gradients of the pointwise and the second 3x3x3 conv, dres / dh2 become nullable (each gradient needs its fp32
+ *     output or its twin) and dbias_res / dbias_h2 (nullable, both or none, fp32 [F]) receive their column sums =
+ *     those convs' bias gradients.  Without twins out, dres and (has_gn) dh2 are required.  The twin kernels need
+ *     F = 8 * 2^k <= 256 (else B3D_ERR_UNSUPPORTED).  B3D_ERR_ARG: out16b without out16, bias gradients without a twin,
+ *     a gradient with neither output. */
 int b3d_se_fc_fwd(const DLTensor* gap_sum, const DLTensor* w1, const DLTensor* w2, DLTensor* hidden,
                   DLTensor* chse, float inv_vox, void* stream);
 int b3d_se_fc_bwd(const DLTensor* gap_sum, const DLTensor* w1, const DLTensor* w2, const DLTensor* hidden,
                   const DLTensor* chse, const DLTensor* dchse, DLTensor* dw1, DLTensor* dw2, DLTensor* dgap,
                   float inv_vox, void* stream);
 int b3d_block_epilogue_fwd(const DLTensor* res, const DLTensor* h2, const DLTensor* stats, const DLTensor* gamma,
-                           const DLTensor* beta, const DLTensor* wsp, const DLTensor* chse, DLTensor* out,
-                           int groups, float eps, int has_gn, void* stream);
+                           const DLTensor* beta, const DLTensor* wsp, const DLTensor* chse, DLTensor* out /*nullable*/,
+                           DLTensor* out16 /*nullable*/, DLTensor* out16b /*nullable*/, int groups, float eps,
+                           int has_gn, long long vox_offset, long long total_vox, void* stream);
 int b3d_block_epilogue_bwd_reduce(const DLTensor* dout, const DLTensor* res, const DLTensor* h2,
                                   const DLTensor* stats, const DLTensor* gamma, const DLTensor* beta,
                                   const DLTensor* wsp, DLTensor* dchse, DLTensor* dwsp, DLTensor* dgamma,
@@ -168,8 +186,10 @@ int b3d_block_epilogue_bwd_reduce(const DLTensor* dout, const DLTensor* res, con
 int b3d_block_epilogue_bwd_apply(const DLTensor* dout, const DLTensor* res, const DLTensor* h2,
                                  const DLTensor* stats, const DLTensor* gamma, const DLTensor* beta,
                                  const DLTensor* wsp, const DLTensor* chse, const DLTensor* dgap,
-                                 const DLTensor* csum, DLTensor* dres, DLTensor* dh2, int groups, float eps,
-                                 int has_gn, void* stream);
+                                 const DLTensor* csum, DLTensor* dres /*nullable*/, DLTensor* dh2 /*nullable*/,
+                                 DLTensor* dres16 /*nullable*/, DLTensor* dh216 /*nullable*/,
+                                 DLTensor* dbias_res /*nullable*/, DLTensor* dbias_h2 /*nullable*/, int groups,
+                                 float eps, int has_gn, void* stream);
 
 /* ---- VAE bottleneck (vae.py:9-13, :119-129): Dense, reparameterisation -------------------------*/
 int b3d_dense_fwd(const DLTensor* x, const DLTensor* w, const DLTensor* bias, DLTensor* y, int act /*1 relu*/,
@@ -264,23 +284,16 @@ int b3d_peer_allreduce2(DLTensor* a /*fp64*/, DLTensor* b /*fp32*/, const DLTens
                         const DLTensor* epoch, int seq, void* stream);
 int b3d_epoch_tick(DLTensor* epoch, void* stream);
 
-/* Depth-slab forms of the P16 forward kernels (whole-volume inference sharded along D; /root/reference/test.py:133 on one
+/* Depth-slab form of the P16 forward conv (whole-volume inference sharded along D; /root/reference/test.py:133 on one
  * slab per GPU): the conv reads P16 sources that carry halo_before / halo_after extra depth slices and emits this slab's
  * PARTIAL GroupNorm statistics over the chunks of the whole volume (stat_total output voxels per sample, this slab's
- * first = stat_off; /root/reference/layers/group_norm.py:83-124 reshapes the whole volume); GroupNorm apply and the
- * block epilogue take the all-reduced statistics and the window [offset, offset + local size) of the volume. */
+ * first = stat_off; /root/reference/layers/group_norm.py:83-124 reshapes the whole volume); b3d_gn_apply and
+ * b3d_block_epilogue_fwd take the all-reduced statistics and the same voxel window. */
 int b3d_conv3d_fwd_p16_slab(const DLTensor* x0, const DLTensor* x1, const DLTensor* x2, const DLTensor* x3,
                             const DLTensor* w, const DLTensor* bias /*nullable*/, DLTensor* y, int stride,
                             int transposed, int act, int halo_before, int halo_after, DLTensor* gn_stats /*nullable*/,
                             int groups, long long stat_off, long long stat_total, DLTensor* gap /*nullable*/,
                             const DLTensor* wpacked, int prezeroed /*gn_stats / gap are already zero*/, void* stream);
-int b3d_gn_apply_p16_slab(const DLTensor* x, const DLTensor* stats, const DLTensor* gamma, const DLTensor* beta,
-                          DLTensor* y /*nullable*/, DLTensor* y16, int groups, float eps, int relu,
-                          long long elem_offset, long long total_elems, void* stream);
-int b3d_block_epilogue_fwd_p16_slab(const DLTensor* res, const DLTensor* h2, const DLTensor* stats,
-                                    const DLTensor* gamma, const DLTensor* beta, const DLTensor* wsp,
-                                    const DLTensor* chse, DLTensor* out /*nullable*/, DLTensor* out16, int groups,
-                                    float eps, int has_gn, long long vox_offset, long long total_vox, void* stream);
 
 /* ---- test-time augmentation (test.py:105-161): flip bits 1=D 2=H 4=W on one [D,H,W,C] volume ------------
  * flip_normalize: out = (flip(x) - mean)/std (test.py:107,128; mean/std nullable).
@@ -316,7 +329,7 @@ int b3d_hd95(const DLTensor* edt_true, const DLTensor* surf_pred, const DLTensor
  * consume directly: [B, D, H, C/8, W, 8] (DLPack ndim 6, dtype f16 | bf16, compact).  Channel octets are planes inside
  * every (d, h) row: a voxel's 8 channels are one 16-byte UMMA cell and a halo row of one plane is W*16 contiguous bytes,
  * so whole halos are fetched as wide TMA rows.  The twins are written by the kernels that PRODUCE conv operands (the
- * *_p16 forms of GroupNorm apply / block epilogue and their backward kernels below) — there is no cast pass on the
+ * twin outputs of b3d_gn_apply / b3d_block_epilogue_fwd and their backward-apply passes) — there is no cast pass on the
  * training step, and a channel concatenation (encoder.py:85,91; decoder.py:75) is a list of up to 4 sources. */
 int b3d_p16_pack(const DLTensor* x /*fp32 NDHWC, C % 8 == 0, may be a channel slice*/, DLTensor* dst /*P16*/,
                  DLTensor* colsum /*nullable fp32 [C]: per-channel sums of x*/, void* stream);
@@ -333,8 +346,8 @@ int b3d_unfold_dup(const DLTensor* dwf, DLTensor* dw, int F, void* stream);
  * wpacked is required).  x0..x3: the sources whose channels are concatenated (x1..x3 nullable), all of the pass's MMA
  * operand type (forward: fp16 by default; data gradient: bf16).  The weight gradient takes bf16 twins of BOTH operands
  * (tcgen05 kind::f16 has one operand type for A and B; mixing f16 with bf16 is an illegal instruction), which is why
- * forward activations carry a second, bf16 twin (y16b / out16b below) when the forward type is fp16.  The weight gradient does NOT produce the bias gradient on this path: it is emitted
- * by the kernel that writes dy (`dbias` of b3d_gn_bwd_apply_p16 / b3d_block_epilogue_bwd_apply_p16, `colsum` of
+ * forward activations carry a second, bf16 twin (y16b / out16b above) when the forward type is fp16.  The weight gradient does NOT produce the bias gradient on this path: it is emitted
+ * by the kernel that writes dy (`dbias` of b3d_gn_bwd_apply / b3d_block_epilogue_bwd_apply, `colsum` of
  * b3d_p16_pack).  scratch (nullable, 16-bit, 1-D): see b3d_conv3d_wgrad_p16_plan. */
 int b3d_conv3d_fwd_p16(const DLTensor* x0, const DLTensor* x1, const DLTensor* x2, const DLTensor* x3, const DLTensor* w,
                        const DLTensor* bias /*nullable*/, DLTensor* y, int stride, int transposed, int act,
@@ -365,25 +378,6 @@ int b3d_conv3d_wgrad_p16_block_ok(int cin, int cout, int h_sp, int w_sp);
 /* 0: the layer's weight gradient is not on the P16 path; 1: straight from the operands; 2: needs a 16-bit scratch of
  * numel(big tensor) elements (stride-2 family); 3: of numel(dy) elements (TS-mode kernel).  w_sp = W of dy. */
 int b3d_conv3d_wgrad_p16_plan(int k, int stride, int transposed, int cin, int cout, int w_sp);
-/* GroupNorm apply / backward-apply and block epilogue forward / backward-apply with twin outputs.  The fp32 outputs
- * (y, dx, out, dres, dh2) are nullable: NULL = only the twin is written (every consumer is a conv).  dbias* (nullable,
- * fp32 [C]): column sums of the gradient written = the bias gradient of the conv that produced the kernel's input. */
-int b3d_gn_apply_p16(const DLTensor* x, const DLTensor* stats, const DLTensor* gamma, const DLTensor* beta, DLTensor* y,
-                     DLTensor* y16, DLTensor* y16b /*nullable: second, bf16 twin*/, int groups, float eps, int relu,
-                     void* stream);
-int b3d_gn_bwd_apply_p16(const DLTensor* dy, const DLTensor* x, const DLTensor* stats, const DLTensor* gamma,
-                         const DLTensor* beta, const DLTensor* csum, DLTensor* dx, DLTensor* dx16, DLTensor* dbias,
-                         int groups, float eps, int relu, void* stream);
-int b3d_block_epilogue_fwd_p16(const DLTensor* res, const DLTensor* h2, const DLTensor* stats, const DLTensor* gamma,
-                               const DLTensor* beta, const DLTensor* wsp, const DLTensor* chse, DLTensor* out,
-                               DLTensor* out16, DLTensor* out16b /*nullable: second, bf16 twin*/, int groups, float eps,
-                               int has_gn, void* stream);
-int b3d_block_epilogue_bwd_apply_p16(const DLTensor* dout, const DLTensor* res, const DLTensor* h2,
-                                     const DLTensor* stats, const DLTensor* gamma, const DLTensor* beta,
-                                     const DLTensor* wsp, const DLTensor* chse, const DLTensor* dgap,
-                                     const DLTensor* csum, DLTensor* dres, DLTensor* dh2, DLTensor* dres16,
-                                     DLTensor* dh216, DLTensor* dbias_res, DLTensor* dbias_h2, int groups, float eps,
-                                     int has_gn, void* stream);
 
 #ifdef __cplusplus
 }

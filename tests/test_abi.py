@@ -1,5 +1,5 @@
 """CPU suite, part 2 — the C-ABI library loads, exports every symbol include/b3d.h declares, and rejects
-host tensors loudly (there is no CPU fallback).  No compute is launched here."""
+host tensors (there is no CPU fallback) and contradictory optional arguments loudly.  No compute is launched here."""
 import ctypes
 import os
 import re
@@ -22,7 +22,7 @@ def test_header_symbols_exported(b3d):
     assert len(names) >= 30
     for n in names:
         assert hasattr(lib, n), f"{n} declared in include/b3d.h but not exported"
-    assert lib.b3d_abi_version() == 1
+    assert lib.b3d_abi_version() == 2
 
 
 def test_python_signatures_cover_header(b3d):
@@ -54,9 +54,23 @@ def test_cpu_tensors_are_rejected(b3d):
     x = torch.zeros(1, 4, 4, 4, 8)
     st = torch.zeros(1, 8, 2, dtype=torch.float64)
     with pytest.raises(b3d._lib.B3DError, match="CUDA device"):
-        b3d._lib.call("b3d_gn_stats", x, st, 8)
+        b3d._lib.call("b3d_gn_stats", x, st, 8, 0, 0)
     with pytest.raises(RuntimeError, match="no CPU path"):
         b3d.ops.group_norm(x, torch.ones(8), torch.zeros(8))
+    # optional outputs that contradict each other are B3D_ERR_ARG (-1) before any tensor is looked at: a second twin
+    # without the first, bias gradients without a twin (only the twin kernels sum them), a gradient without any output
+    v, t = torch.ones(8), torch.zeros(1, 4, 4, 1, 4, 8, dtype=torch.bfloat16)
+    for name, args in (
+            ("b3d_gn_apply", (x, st, v, v, x, None, t, 8, 1e-5, 0, 0, 0)),
+            ("b3d_gn_bwd_apply", (x, x, st, v, v, st, x, None, v, 8, 1e-5, 0)),
+            ("b3d_gn_bwd_apply", (x, x, st, v, v, st, None, None, None, 8, 1e-5, 0)),
+            ("b3d_block_epilogue_fwd", (x, x, st, v, v, v, v, x, None, t, 8, 1e-5, 1, 0, 0)),
+            ("b3d_block_epilogue_bwd_apply", (x, x, x, st, v, v, v, v, v, st, x, x, None, None, v, v, 8, 1e-5, 1)),
+            ("b3d_block_epilogue_bwd_apply", (x, x, x, st, v, v, v, v, v, st, x, None, None, None, None, None, 8, 1e-5,
+                                              1)),
+            ("b3d_block_epilogue_bwd_apply", (x, x, x, st, v, v, v, v, v, st, None, None, t, t, v, None, 8, 1e-5, 1))):
+        with pytest.raises(b3d._lib.B3DError, match=r"failed \(-1\)"):
+            b3d._lib.call(name, *args)
 
 
 def test_dlpack_struct_matches_torch_capsule(b3d):

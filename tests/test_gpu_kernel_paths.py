@@ -711,16 +711,16 @@ def test_group_norm_kernels_at_model_shapes(env, dev, shape, mean):
     cells = (C // 8) & (C // 8 - 1) == 0        # power-of-two channels per group: the cell kernels (norm.cu)
 
     def run():
-        ops._call("b3d_gn_stats", x, stats, 8)
-        ops._call("b3d_gn_apply", x, stats, ga, be, y0, 8, 1e-5, 1)
+        ops._call("b3d_gn_stats", x, stats, 8, 0, 0)
+        ops._call("b3d_gn_apply", x, stats, ga, be, y0, None, None, 8, 1e-5, 1, 0, 0)
         ops._call("b3d_gn_bwd_reduce", dy, x, stats, ga, be, dga, dbe, csum, 8, 1e-5, 1)
         if cells:
             y16 = ops.p16_empty(shape, x, torch.float16)
-            ops._call("b3d_gn_apply_p16", x, stats, ga, be, y1, y16, None, 8, 1e-5, 1)
+            ops._call("b3d_gn_apply", x, stats, ga, be, y1, y16, None, 8, 1e-5, 1, 0, 0)
             dx16 = ops.p16_empty(shape, x, torch.bfloat16)
-            ops._call("b3d_gn_bwd_apply_p16", dy, x, stats, ga, be, csum, dx, dx16, dbias, 8, 1e-5, 1)
+            ops._call("b3d_gn_bwd_apply", dy, x, stats, ga, be, csum, dx, dx16, dbias, 8, 1e-5, 1)
         else:
-            ops._call("b3d_gn_bwd_apply", dy, x, stats, ga, be, csum, dx, 8, 1e-5, 1)
+            ops._call("b3d_gn_bwd_apply", dy, x, stats, ga, be, csum, dx, None, None, 8, 1e-5, 1)
     _, kern = run_profiled(run)
     assert has(kern, "gn_stats_kernel") and has(kern, "gn_apply"), kern
     assert has(kern, "gn_bwd_reduce8_kernel") == cells, kern       # the cell kernels, or the non-cell fallback
@@ -731,7 +731,7 @@ def test_group_norm_kernels_at_model_shapes(env, dev, shape, mean):
               K.check("dgamma", dga, dgar, None, None, 1e-5), K.check("dbeta", dbe, dber, None, None, 1e-5),
               K.check("csum", csum, csr, None, None, 1e-5), K.check("dx", dx, dxr, None, None, 1e-5)]
     if cells:
-        checks += [K.check("y (gn_apply_p16)", y1, yr, None, None, 1e-5),
+        checks += [K.check("y (gn_apply, twin kernel)", y1, yr, None, None, 1e-5),
                    K.check("dbias", dbias, dxr.sum(dim=(0, 1, 2, 3)), None, None, 1e-5)]
     record(f"gn {tuple(shape)} mean {mean}", kern, checks)
 
@@ -776,12 +776,12 @@ def test_block_epilogue_kernels_at_model_shapes(env, dev, shape, mean):
     dr, dh, dbr, dbh = torch.empty_like(res), torch.empty_like(res), torch.empty(F, device=dev), torch.empty(F, device=dev)
 
     def run():
-        ops._call("b3d_gn_stats", h2, stats, 8)
+        ops._call("b3d_gn_stats", h2, stats, 8, 0, 0)
         o16 = ops.p16_empty(shape, res, torch.float16)
-        ops._call("b3d_block_epilogue_fwd_p16", res, h2, stats, ga, be, wsp, chse, out, o16, None, 8, 1e-5, 1)
+        ops._call("b3d_block_epilogue_fwd", res, h2, stats, ga, be, wsp, chse, out, o16, None, 8, 1e-5, 1, 0, 0)
         ops._call("b3d_block_epilogue_bwd_reduce", dout, res, h2, stats, ga, be, wsp, dch, dws, dga, dbe, csum, 8, 1e-5, 1)
         dr16, dh16 = ops.p16_empty(shape, res, torch.bfloat16), ops.p16_empty(shape, res, torch.bfloat16)
-        ops._call("b3d_block_epilogue_bwd_apply_p16", dout, res, h2, stats, ga, be, wsp, chse, dgap, csum, dr, dh, dr16,
+        ops._call("b3d_block_epilogue_bwd_apply", dout, res, h2, stats, ga, be, wsp, chse, dgap, csum, dr, dh, dr16,
                   dh16, dbr, dbh, 8, 1e-5, 1)
     _, kern = run_profiled(run)
     assert has(kern, "b3d::block_fwd16_kernel"), kern
@@ -949,11 +949,11 @@ def _unpack(ops, t, shape):
 @pytest.mark.parametrize("case", SLAB_WINDOWS, ids=[c[0] for c in SLAB_WINDOWS])
 def test_slab_window_kernels(env, dev, slab_refs, case):
     """The depth-slab GroupNorm / block-epilogue kernels on real slab windows against fp64 of the WHOLE volume, sliced:
-      * b3d_gn_stats_slab: each window's partial (sum x, sum x^2) per whole-volume chunk (zero for the chunks it misses)
-        at 1e-6 of sum|terms|, and their sum over a partition = the whole volume's;
-      * b3d_gn_apply_slab, b3d_gn_apply_p16_slab (fp32 y + twin, and twin only), b3d_gn_channel_apply_slab (y + twin,
-        y only, twin only) and b3d_block_epilogue_fwd_p16_slab (has_gn 1 with out + twin and twin only, the form
-        sharded inference uses; has_gn 0), given the exact whole-volume statistics: the fp32 output at rel-L2 <= 1e-5;
+      * b3d_gn_stats on a window: each window's partial (sum x, sum x^2) per whole-volume chunk (zero for the chunks it
+        misses) at 1e-6 of sum|terms|, and their sum over a partition = the whole volume's;
+      * b3d_gn_apply on a window (y only, y + twin, and twin only), b3d_gn_channel_apply_slab (y + twin, y only, twin
+        only) and b3d_block_epilogue_fwd on a window (has_gn 1 with out + twin and twin only, the form sharded
+        inference uses; has_gn 0), given the exact whole-volume statistics: the fp32 output at rel-L2 <= 1e-5;
       * every twin (unpacked by b3d_p16_unpack) bit-identical to the fp16 / bf16 rounding of the fp32 output stored from
         the same registers; a twin written alone within half a 16-bit ulp + 1e-5 max|ref| of the fp64 reference, and
         bit-identical to the twin written next to y.
@@ -971,7 +971,7 @@ def test_slab_window_kernels(env, dev, slab_refs, case):
     v = _slab_volume(slab_refs, (D, H, W, C), dev)
     x, res, ga, be, wsp, chse = (v[k] for k in ("x", "res", "ga", "be", "wsp", "chse"))
     per, nvox = H * W * C, D * H * W
-    total, L = D * per, D * per // 8
+    L = D * per // 8
     nan = float("nan")
     outs = []
 
@@ -986,21 +986,21 @@ def test_slab_window_kernels(env, dev, slab_refs, case):
                      part_c=torch.full((1, 8, 2), nan, dtype=torch.float64, device=dev),
                      y_a=f32(), y_p=f32(), t_p=p16(), t_po=p16(), y_c=f32(), t_c=p16(), y_co=f32(), t_co=p16(),
                      o_g=f32(), t_g=p16(), t_go=p16(), o_n=f32(), t_n=p16())
-            off, r = d0 * per, int(relu)
-            ops._call("b3d_gn_stats_slab", xs, o["part"], 8, off, total)
-            ops._call("b3d_gn_apply_slab", xs, v["st"], ga, be, o["y_a"], 8, 1e-5, r, off, total)
-            ops._call("b3d_gn_apply_p16_slab", xs, v["st"], ga, be, o["y_p"], o["t_p"], 8, 1e-5, r, off, total)
-            ops._call("b3d_gn_apply_p16_slab", xs, v["st"], ga, be, None, o["t_po"], 8, 1e-5, r, off, total)
+            off, r = d0 * H * W, int(relu)
+            ops._call("b3d_gn_stats", xs, o["part"], 8, off, nvox)
+            ops._call("b3d_gn_apply", xs, v["st"], ga, be, o["y_a"], None, None, 8, 1e-5, r, off, nvox)
+            ops._call("b3d_gn_apply", xs, v["st"], ga, be, o["y_p"], o["t_p"], None, 8, 1e-5, r, off, nvox)
+            ops._call("b3d_gn_apply", xs, v["st"], ga, be, None, o["t_po"], None, 8, 1e-5, r, off, nvox)
             ops._call("b3d_gn_channel_stats", xs, o["part_c"], 8)
             ops._call("b3d_gn_channel_apply_slab", xs, v["st_c"], ga, be, o["y_c"], o["t_c"], 8, 1e-5, r, nvox)
             ops._call("b3d_gn_channel_apply_slab", xs, v["st_c"], ga, be, o["y_co"], None, 8, 1e-5, r, nvox)
             ops._call("b3d_gn_channel_apply_slab", xs, v["st_c"], ga, be, None, o["t_co"], 8, 1e-5, r, nvox)
-            ops._call("b3d_block_epilogue_fwd_p16_slab", rs, xs, v["st"], ga, be, wsp, chse, o["o_g"], o["t_g"], 8,
-                      1e-5, 1, d0 * H * W, nvox)
-            ops._call("b3d_block_epilogue_fwd_p16_slab", rs, xs, v["st"], ga, be, wsp, chse, None, o["t_go"], 8,
-                      1e-5, 1, d0 * H * W, nvox)
-            ops._call("b3d_block_epilogue_fwd_p16_slab", rs, xs, None, None, None, wsp, chse, o["o_n"], o["t_n"], 8,
-                      1e-5, 0, d0 * H * W, nvox)
+            ops._call("b3d_block_epilogue_fwd", rs, xs, v["st"], ga, be, wsp, chse, o["o_g"], o["t_g"], None, 8,
+                      1e-5, 1, off, nvox)
+            ops._call("b3d_block_epilogue_fwd", rs, xs, v["st"], ga, be, wsp, chse, None, o["t_go"], None, 8,
+                      1e-5, 1, off, nvox)
+            ops._call("b3d_block_epilogue_fwd", rs, xs, None, None, None, wsp, chse, o["o_n"], o["t_n"], None, 8,
+                      1e-5, 0, off, nvox)
             outs.append(o)
     _, kern = run_profiled(run)
     names = [n.replace(" ", "") for n in kern]
@@ -1030,15 +1030,15 @@ def test_slab_window_kernels(env, dev, slab_refs, case):
         shp = tuple(o["y_a"].shape)
         y_r, yc_r = act(sl(v["y"])), act(sl(v["y_c"]))
         checks += [
-            K.check_sums(f"{w} gn_stats_slab", o["part"], ref_p, sc_p),
+            K.check_sums(f"{w} gn_stats", o["part"], ref_p, sc_p),
             K.check_sums(f"{w} gn_channel_stats", o["part_c"], torch.stack([grp.sum((0, 2)), (grp * grp).sum((0, 2))],
                                                                            dim=-1)[None],
                          torch.stack([grp.abs().sum((0, 2)), (grp * grp).sum((0, 2))], dim=-1)[None]),
-            K.check(f"{w} gn_apply_slab y", o["y_a"], y_r, None, None, 1e-5),
-            K.check(f"{w} gn_apply_p16_slab y", o["y_p"], y_r, None, None, 1e-5),
-            _same(f"{w} gn_apply_p16_slab twin = y rounded", _unpack(ops, o["t_p"], shp), o["y_p"].to(td).float()),
-            K.check_rounded(f"{w} gn_apply_p16_slab twin only", _unpack(ops, o["t_po"], shp), y_r, td),
-            _same(f"{w} gn_apply_p16_slab twin only = twin next to y", o["t_po"], o["t_p"]),
+            K.check(f"{w} gn_apply y", o["y_a"], y_r, None, None, 1e-5),
+            K.check(f"{w} gn_apply y next to twin", o["y_p"], y_r, None, None, 1e-5),
+            _same(f"{w} gn_apply twin = y rounded", _unpack(ops, o["t_p"], shp), o["y_p"].to(td).float()),
+            K.check_rounded(f"{w} gn_apply twin only", _unpack(ops, o["t_po"], shp), y_r, td),
+            _same(f"{w} gn_apply twin only = twin next to y", o["t_po"], o["t_p"]),
             K.check(f"{w} gn_channel_apply_slab y", o["y_c"], yc_r, None, None, 1e-5),
             _same(f"{w} gn_channel_apply_slab twin = y rounded", _unpack(ops, o["t_c"], shp), o["y_c"].to(td).float()),
             _same(f"{w} gn_channel_apply_slab y only = y next to twin", o["y_co"], o["y_c"]),
@@ -1052,5 +1052,5 @@ def test_slab_window_kernels(env, dev, slab_refs, case):
             _same(f"{w} block_epilogue_slab (no GN) twin = out rounded", _unpack(ops, o["t_n"], shp),
                   o["o_n"].to(td).float())]
     if partition:
-        checks.append(K.check_sums("sum of the windows' gn_stats_slab = whole volume", tot, v["st"], v["st_scale"]))
+        checks.append(K.check_sums("sum of the windows' gn_stats = whole volume", tot, v["st"], v["st_scale"]))
     record(cid, kern, checks)

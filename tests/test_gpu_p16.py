@@ -249,27 +249,27 @@ def test_group_norm_twin_outputs(b3d, dev, shape, relu):
     x = rnd(*shape, seed=1, dev=dev)
     ga, be = 1 + 0.3 * rnd(shape[-1], seed=2, dev=dev), 0.3 * rnd(shape[-1], seed=3, dev=dev)
     stats = torch.empty(shape[0], 8, 2, dtype=torch.float64, device=dev)
-    ops._call("b3d_gn_stats", x, stats, 8)
+    ops._call("b3d_gn_stats", x, stats, 8, 0, 0)
     y0, y1 = torch.empty_like(x), torch.empty_like(x)
-    ops._call("b3d_gn_apply", x, stats, ga, be, y0, 8, 1e-5, int(relu))
+    ops._call("b3d_gn_apply", x, stats, ga, be, y0, None, None, 8, 1e-5, int(relu), 0, 0)
     y16 = ops.p16_empty(shape, x, torch.float16)
     yw = ops.p16_empty(shape, x, torch.bfloat16)
-    ops._call("b3d_gn_apply_p16", x, stats, ga, be, y1, y16, yw, 8, 1e-5, int(relu))
+    ops._call("b3d_gn_apply", x, stats, ga, be, y1, y16, yw, 8, 1e-5, int(relu), 0, 0)
     # separate kernels (one 16-byte cell per thread): same formula, fused-multiply-add grouping may differ in the last bit
     assert rel(y1, y0) < 1e-6 and torch.equal(y16, to_p16_ref(y1, torch.float16))
     assert torch.equal(yw, to_p16_ref(y1, torch.bfloat16))
     y16b = ops.p16_empty(shape, x, torch.float16)
-    ops._call("b3d_gn_apply_p16", x, stats, ga, be, None, y16b, None, 8, 1e-5, int(relu))       # one twin only
+    ops._call("b3d_gn_apply", x, stats, ga, be, None, y16b, None, 8, 1e-5, int(relu), 0, 0)     # one twin only
     assert torch.equal(y16b, y16)
     # backward
     dy = rnd(*shape, seed=4, dev=dev)
     dga, dbe, csum = torch.empty_like(ga), torch.empty_like(be), torch.empty_like(stats)
     ops._call("b3d_gn_bwd_reduce", dy, x, stats, ga, be, dga, dbe, csum, 8, 1e-5, int(relu))
     dx0, dx1 = torch.empty_like(x), torch.empty_like(x)
-    ops._call("b3d_gn_bwd_apply", dy, x, stats, ga, be, csum, dx0, 8, 1e-5, int(relu))
+    ops._call("b3d_gn_bwd_apply", dy, x, stats, ga, be, csum, dx0, None, None, 8, 1e-5, int(relu))
     dx16 = ops.p16_empty(shape, x, torch.bfloat16)
     db = torch.empty(shape[-1], device=dev)
-    ops._call("b3d_gn_bwd_apply_p16", dy, x, stats, ga, be, csum, dx1, dx16, db, 8, 1e-5, int(relu))
+    ops._call("b3d_gn_bwd_apply", dy, x, stats, ga, be, csum, dx1, dx16, db, 8, 1e-5, int(relu))
     assert rel(dx1, dx0) < 1e-6 and torch.equal(dx16, to_p16_ref(dx1, torch.bfloat16))
     ref = dx0.double().sum(dim=(0, 1, 2, 3))
     assert float((db.double() - ref).abs().max()) < 1e-4 * float(dx0.abs().sum(dim=(0, 1, 2, 3)).max()) + 1e-6
@@ -283,16 +283,16 @@ def test_block_epilogue_twin_outputs(b3d, dev, shape):
     ga, be = 1 + 0.3 * rnd(F, seed=3, dev=dev), 0.3 * rnd(F, seed=4, dev=dev)
     wsp, chse = 0.3 * rnd(F, seed=5, dev=dev), torch.sigmoid(rnd(shape[0], F, seed=6, dev=dev))
     stats = torch.empty(shape[0], 8, 2, dtype=torch.float64, device=dev)
-    ops._call("b3d_gn_stats", h2, stats, 8)
+    ops._call("b3d_gn_stats", h2, stats, 8, 0, 0)
     o0, o1 = torch.empty_like(res), torch.empty_like(res)
-    ops._call("b3d_block_epilogue_fwd", res, h2, stats, ga, be, wsp, chse, o0, 8, 1e-5, 1)
+    ops._call("b3d_block_epilogue_fwd", res, h2, stats, ga, be, wsp, chse, o0, None, None, 8, 1e-5, 1, 0, 0)
     o16 = ops.p16_empty(shape, res, torch.float16)
     ow = ops.p16_empty(shape, res, torch.bfloat16)
-    ops._call("b3d_block_epilogue_fwd_p16", res, h2, stats, ga, be, wsp, chse, o1, o16, ow, 8, 1e-5, 1)
+    ops._call("b3d_block_epilogue_fwd", res, h2, stats, ga, be, wsp, chse, o1, o16, ow, 8, 1e-5, 1, 0, 0)
     assert rel(o1, o0) < 1e-6 and torch.equal(o16, to_p16_ref(o1, torch.float16))
     assert torch.equal(ow, to_p16_ref(o1, torch.bfloat16))
     o16b = ops.p16_empty(shape, res, torch.float16)
-    ops._call("b3d_block_epilogue_fwd_p16", res, h2, stats, ga, be, wsp, chse, None, o16b, None, 8, 1e-5, 1)
+    ops._call("b3d_block_epilogue_fwd", res, h2, stats, ga, be, wsp, chse, None, o16b, None, 8, 1e-5, 1, 0, 0)
     assert torch.equal(o16b, o16)
     # backward apply
     dout = rnd(*shape, seed=7, dev=dev)
@@ -301,16 +301,17 @@ def test_block_epilogue_twin_outputs(b3d, dev, shape):
     dga, dbe, csum = torch.empty_like(ga), torch.empty_like(be), torch.empty_like(stats)
     ops._call("b3d_block_epilogue_bwd_reduce", dout, res, h2, stats, ga, be, wsp, dch, dws, dga, dbe, csum, 8, 1e-5, 1)
     dr0, dh0 = torch.empty_like(res), torch.empty_like(res)
-    ops._call("b3d_block_epilogue_bwd_apply", dout, res, h2, stats, ga, be, wsp, chse, dgap, csum, dr0, dh0, 8, 1e-5, 1)
+    ops._call("b3d_block_epilogue_bwd_apply", dout, res, h2, stats, ga, be, wsp, chse, dgap, csum, dr0, dh0, None, None,
+              None, None, 8, 1e-5, 1)
     dr16, dh16 = ops.p16_empty(shape, res, torch.bfloat16), ops.p16_empty(shape, res, torch.bfloat16)
     dbr, dbh = torch.empty(F, device=dev), torch.empty(F, device=dev)
     dr1, dh1 = torch.empty_like(res), torch.empty_like(res)
-    ops._call("b3d_block_epilogue_bwd_apply_p16", dout, res, h2, stats, ga, be, wsp, chse, dgap, csum, dr1, dh1, dr16,
+    ops._call("b3d_block_epilogue_bwd_apply", dout, res, h2, stats, ga, be, wsp, chse, dgap, csum, dr1, dh1, dr16,
               dh16, dbr, dbh, 8, 1e-5, 1)
     assert rel(dr1, dr0) < 1e-6 and rel(dh1, dh0) < 1e-6
     assert torch.equal(dr16, to_p16_ref(dr1, torch.bfloat16)) and torch.equal(dh16, to_p16_ref(dh1, torch.bfloat16))
     dr16b, dh16b = ops.p16_empty(shape, res, torch.bfloat16), ops.p16_empty(shape, res, torch.bfloat16)
-    ops._call("b3d_block_epilogue_bwd_apply_p16", dout, res, h2, stats, ga, be, wsp, chse, dgap, csum, None, None, dr16b,
+    ops._call("b3d_block_epilogue_bwd_apply", dout, res, h2, stats, ga, be, wsp, chse, dgap, csum, None, None, dr16b,
               dh16b, None, None, 8, 1e-5, 1)                                        # twins only, no bias gradients
     assert torch.equal(dr16b, dr16) and torch.equal(dh16b, dh16)
     for got, full in ((dbr, dr0), (dbh, dh0)):

@@ -55,20 +55,21 @@ for n, C in ((128, 16), (64, 32), (32, 64)):
     st = torch.empty(1, 8, 2, dtype=torch.float64, device=dev)
     cs = torch.empty_like(st)
     tag = f"{n}^3x{C}"
-    report(f"gn_stats {tag}", 4 * E, lambda: ops._call("b3d_gn_stats", x, st, 8))
-    report(f"gn_apply+relu {tag}", 8 * E, lambda: ops._call("b3d_gn_apply", x, st, ga, be, y, 8, 1e-5, 1))
+    report(f"gn_stats {tag}", 4 * E, lambda: ops._call("b3d_gn_stats", x, st, 8, 0, 0))
+    report(f"gn_apply+relu {tag}", 8 * E, lambda: ops._call("b3d_gn_apply", x, st, ga, be, y, None, None, 8, 1e-5, 1, 0, 0))
     report(f"gn_bwd_reduce {tag}", 8 * E,
            lambda: ops._call("b3d_gn_bwd_reduce", dy, x, st, ga, be, dga, dbe, cs, 8, 1e-5, 1))
     report(f"gn_bwd_apply {tag}", 12 * E,
-           lambda: ops._call("b3d_gn_bwd_apply", dy, x, st, ga, be, cs, dx, 8, 1e-5, 1))
+           lambda: ops._call("b3d_gn_bwd_apply", dy, x, st, ga, be, cs, dx, None, None, 8, 1e-5, 1))
     # ResnetBlock epilogue (GN2 + ReLU + scSE + add)
     F, R = C, C // 2
     res, h2, out = torch.randn(shp, device=dev), torch.randn(shp, device=dev), torch.empty(shp, device=dev)
     wsp = torch.randn(F, device=dev) * 0.1
     chse = torch.rand(1, F, device=dev)
-    ops._call("b3d_gn_stats", h2, st, 8)
+    ops._call("b3d_gn_stats", h2, st, 8, 0, 0)
     report(f"block_epilogue_fwd {tag}", 12 * E,
-           lambda: ops._call("b3d_block_epilogue_fwd", res, h2, st, ga, be, wsp, chse, out, 8, 1e-5, 1))
+           lambda: ops._call("b3d_block_epilogue_fwd", res, h2, st, ga, be, wsp, chse, out, None, None, 8, 1e-5, 1,
+                             0, 0))
     dchse, dwsp, dgap = torch.empty(1, F, device=dev), torch.empty(F, device=dev), torch.randn(1, F, device=dev) * 1e-3
     dres, dh2 = torch.empty(shp, device=dev), torch.empty(shp, device=dev)
     report(f"block_epilogue_bwd_reduce {tag}", 12 * E,
@@ -76,28 +77,29 @@ for n, C in ((128, 16), (64, 32), (32, 64)):
                              8, 1e-5, 1))
     report(f"block_epilogue_bwd_apply {tag}", 20 * E,
            lambda: ops._call("b3d_block_epilogue_bwd_apply", dy, res, h2, st, ga, be, wsp, chse, dgap, cs, dres, dh2,
-                             8, 1e-5, 1))
+                             None, None, None, None, 8, 1e-5, 1))
     # ---- the P16 twin forms the training step actually runs (fp32 outputs not materialised)
     t16, t16b = ops.p16_empty(shp, x, torch.float16), ops.p16_empty(shp, x, torch.bfloat16)
     u16b = ops.p16_empty(shp, x, torch.bfloat16)
     dbias, dbias2 = torch.empty(C, device=dev), torch.empty(C, device=dev)
-    report(f"gn_apply_p16 fp16 twin only (inference) {tag}", 6 * E,
-           lambda: ops._call("b3d_gn_apply_p16", x, st, ga, be, None, t16, None, 8, 1e-5, 1))
-    report(f"gn_apply_p16 fp16+bf16 twins (training) {tag}", 8 * E,
-           lambda: ops._call("b3d_gn_apply_p16", x, st, ga, be, None, t16, t16b, 8, 1e-5, 1))
-    report(f"gn_apply_p16 fp32 + both twins {tag}", 12 * E,
-           lambda: ops._call("b3d_gn_apply_p16", x, st, ga, be, y, t16, t16b, 8, 1e-5, 1))
-    report(f"gn_bwd_apply_p16 bf16 twin + dbias {tag}", 10 * E,
-           lambda: ops._call("b3d_gn_bwd_apply_p16", dy, x, st, ga, be, cs, None, t16b, dbias, 8, 1e-5, 1))
-    report(f"gn_bwd_apply_p16 bf16 twin, no dbias {tag}", 10 * E,
-           lambda: ops._call("b3d_gn_bwd_apply_p16", dy, x, st, ga, be, cs, None, t16b, None, 8, 1e-5, 1))
-    report(f"block_epilogue_fwd_p16 twins only {tag}", 12 * E,
-           lambda: ops._call("b3d_block_epilogue_fwd_p16", res, h2, st, ga, be, wsp, chse, None, t16, t16b, 8, 1e-5, 1))
-    report(f"block_epilogue_bwd_apply_p16 twins + dbias {tag}", 16 * E,
-           lambda: ops._call("b3d_block_epilogue_bwd_apply_p16", dy, res, h2, st, ga, be, wsp, chse, dgap, cs, None, None,
+    report(f"gn_apply fp16 twin only (inference) {tag}", 6 * E,
+           lambda: ops._call("b3d_gn_apply", x, st, ga, be, None, t16, None, 8, 1e-5, 1, 0, 0))
+    report(f"gn_apply fp16+bf16 twins (training) {tag}", 8 * E,
+           lambda: ops._call("b3d_gn_apply", x, st, ga, be, None, t16, t16b, 8, 1e-5, 1, 0, 0))
+    report(f"gn_apply fp32 + both twins {tag}", 12 * E,
+           lambda: ops._call("b3d_gn_apply", x, st, ga, be, y, t16, t16b, 8, 1e-5, 1, 0, 0))
+    report(f"gn_bwd_apply bf16 twin + dbias {tag}", 10 * E,
+           lambda: ops._call("b3d_gn_bwd_apply", dy, x, st, ga, be, cs, None, t16b, dbias, 8, 1e-5, 1))
+    report(f"gn_bwd_apply bf16 twin, no dbias {tag}", 10 * E,
+           lambda: ops._call("b3d_gn_bwd_apply", dy, x, st, ga, be, cs, None, t16b, None, 8, 1e-5, 1))
+    report(f"block_epilogue_fwd twins only {tag}", 12 * E,
+           lambda: ops._call("b3d_block_epilogue_fwd", res, h2, st, ga, be, wsp, chse, None, t16, t16b, 8, 1e-5, 1,
+                             0, 0))
+    report(f"block_epilogue_bwd_apply twins + dbias {tag}", 16 * E,
+           lambda: ops._call("b3d_block_epilogue_bwd_apply", dy, res, h2, st, ga, be, wsp, chse, dgap, cs, None, None,
                              t16b, u16b, dbias, dbias2, 8, 1e-5, 1))
-    report(f"block_epilogue_bwd_apply_p16 twins, no dbias {tag}", 16 * E,
-           lambda: ops._call("b3d_block_epilogue_bwd_apply_p16", dy, res, h2, st, ga, be, wsp, chse, dgap, cs, None, None,
+    report(f"block_epilogue_bwd_apply twins, no dbias {tag}", 16 * E,
+           lambda: ops._call("b3d_block_epilogue_bwd_apply", dy, res, h2, st, ga, be, wsp, chse, dgap, cs, None, None,
                              t16b, u16b, None, None, 8, 1e-5, 1))
     del res, h2, out, dres, dh2, t16, t16b, u16b
 
