@@ -142,6 +142,7 @@ SIGNATURES = {
     "b3d_conv3d_dgrad_p16": "TTTiiiTv",
     "b3d_conv3d_wgrad_p16": "TTTTTTiiTv",
     "b3d_conv3d_wgrad_p16_block": "TTTTTTTTv",
+    "b3d_conv3d_wgrad_narrow": "TTTTTTv",
 }
 _CT = {"T": P, "i": _i, "f": _f, "v": _v, "L": _ll, "U": _ull}
 for _name, _sig in SIGNATURES.items():
@@ -168,6 +169,8 @@ lib.b3d_conv3d_wgrad_p16_plan.argtypes = [_i] * 6
 lib.b3d_conv3d_wgrad_p16_plan.restype = _i
 lib.b3d_conv3d_wgrad_p16_block_ok.argtypes = [_i] * 4
 lib.b3d_conv3d_wgrad_p16_block_ok.restype = _i
+lib.b3d_conv3d_wgrad_narrow_ok.argtypes = [_i] * 4
+lib.b3d_conv3d_wgrad_narrow_ok.restype = _i
 
 
 class B3DError(RuntimeError):

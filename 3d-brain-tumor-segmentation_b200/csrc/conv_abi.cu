@@ -683,6 +683,54 @@ extern "C" int b3d_conv3d_wgrad_p16_block(const DLTensor* x0_, const DLTensor* x
   return launch_conv_wgrad_kdf(wg, (float*)dw.p, (cudaStream_t)stream, wp, dres.p, (float*)dwp.p);
 }
 
+extern "C" int b3d_conv3d_wgrad_narrow_ok(int k, int cin, int cout, int pair) {
+  return tc_wgrad_narrow_supported(k, cin, cout, pair) ? 1 : 0;
+}
+
+extern "C" int b3d_conv3d_wgrad_narrow(const DLTensor* nar_, const DLTensor* wide_, const DLTensor* wide2_, DLTensor* dw_,
+                                       DLTensor* dw2_, DLTensor* dbias_, void* stream) {
+  TView nar, dw;
+  P16View wide;
+  int k;
+  B3D_TRY(view(nar_, DT_F32, 5, true, "narrow tensor", &nar));
+  B3D_TRY(view_p16(wide_, "wide tensor (P16)", &wide));
+  B3D_TRY(weight_view(dw_, &dw, &k));
+  B3D_REQUIRE(wide.bf16, B3D_ERR_DTYPE, "wgrad (narrow): the wide operand is a bf16 twin");
+  NarrowWgrad a;
+  memset(&a, 0, sizeof(a));
+  a.nar = (const float*)nar.p; a.pitch = nar.pitch;
+  a.B = (int)nar.shape[0]; a.D = (int)nar.shape[1]; a.H = (int)nar.shape[2]; a.W = (int)nar.shape[3];
+  a.Cn = (int)nar.shape[4]; a.k = k; a.Cw = 8 * wide.C8;
+  a.wide = wide.p; a.dw = (float*)dw.p;
+  B3D_REQUIRE(wide.B == a.B && wide.D == a.D && wide.H == a.H && wide.W == a.W, B3D_ERR_SHAPE,
+              "wgrad (narrow): spatial dims of the two operands differ");
+  if (dw.shape[3] == a.Cn && dw.shape[4] == a.Cw) a.tr = 0;
+  else if (dw.shape[3] == a.Cw && dw.shape[4] == a.Cn) a.tr = 1;
+  else B3D_REQUIRE(false, B3D_ERR_SHAPE, "wgrad (narrow): dw channel dims match neither operand order");
+  if (wide2_ != nullptr || dw2_ != nullptr) {
+    P16View w2;
+    TView dw2;
+    int k2;
+    B3D_REQUIRE(wide2_ != nullptr && dw2_ != nullptr && a.tr == 0, B3D_ERR_ARG,
+                "wgrad (narrow): dres and dw_pw go together, with a narrow layer input");
+    B3D_TRY(view_p16(wide2_, "dres (P16)", &w2));
+    B3D_TRY(weight_view(dw2_, &dw2, &k2));
+    B3D_REQUIRE(w2.bf16 && w2.B == wide.B && w2.D == wide.D && w2.H == wide.H && w2.W == wide.W && w2.C8 == wide.C8,
+                B3D_ERR_SHAPE, "wgrad (narrow): dres must match dy");
+    B3D_REQUIRE(k2 == 1 && dw2.shape[3] == a.Cn && dw2.shape[4] == a.Cw, B3D_ERR_SHAPE,
+                "wgrad (narrow): dw_pw is the (1,1,1,Cin,Cout) kernel gradient");
+    a.wide2 = w2.p; a.dw2 = (float*)dw2.p;
+  }
+  if (dbias_ != nullptr) {
+    TView db;
+    B3D_TRY(view(dbias_, DT_F32, 1, false, "dbias", &db));
+    B3D_REQUIRE(a.tr == 1 && db.numel == a.Cn, B3D_ERR_ARG,
+                "wgrad (narrow): the bias gradient is the column sums of a narrow dy (%d values)", a.Cn);
+    a.dbias = (float*)db.p;
+  }
+  return launch_conv_wgrad_narrow(a, (cudaStream_t)stream);
+}
+
 // dw of a Conv3D (x = layer input, up to 4 concatenated P16 sources; dy = P16 gradient of the output) or of a
 // Conv3DTranspose (transposed = 1: single source).  The bias gradient is NOT produced here: on this path it is emitted
 // by the kernel that writes dy (b3d_gn_bwd_apply / b3d_block_epilogue_bwd_apply, `dbias`).

@@ -134,6 +134,22 @@ int launch_conv_wgrad_ts(const WgradGeom& wg, const void* x_bf16, const void* dy
 bool tc_wgrad_kdf_supported(const WgradGeom& wg, const WgP16* p16);
 int launch_conv_wgrad_kdf(const WgradGeom& wg, float* dw, cudaStream_t s, const WgP16& p16,
                           const void* dres = nullptr, float* dw2 = nullptr);
+// weight gradient of a stride-1 k in {1, 3} layer with Cn < 8 channels on one side, the tap-stacked operand of the
+// narrow fp32 tensor built in shared memory (conv_tc_wgrad.cu); the wide side is a bf16 P16 twin
+struct NarrowWgrad {
+  const float* nar;                // fp32 [B, D, H, W, pitch], Cn channels
+  long long pitch;
+  int B, D, H, W, Cn, k;
+  int tr;                          // 0: nar = layer input x, dw [k,k,k,Cn,Cw]; 1: nar = dy, dw [k,k,k,Cw,Cn]
+  const void* wide;                // P16 bf16 twin, Cw channels: dy (tr = 0) or x (tr = 1)
+  const void* wide2;               // nullable (tr = 0): dres of the pointwise conv reading the same x
+  int Cw;
+  float* dw;
+  float* dw2;                      // with wide2: the pointwise conv's dw [Cn][Cw]
+  float* dbias;                    // nullable (tr = 1): column sums of dy
+};
+bool tc_wgrad_narrow_supported(int k, int cin, int cout, int pair);
+int launch_conv_wgrad_narrow(const NarrowWgrad& a, cudaStream_t s);
 int launch_cast_bf16_t8(const float* src, void* dst, long long nvox, int C, float* colsum, cudaStream_t s);
 int launch_cast_stack_bf16(const float* src, void* dst, int B, int D, int H, int W, int Cn, long long pitch, int k,
                            int sgn, int nA, cudaStream_t s);

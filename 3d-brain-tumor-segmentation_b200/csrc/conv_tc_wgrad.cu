@@ -386,6 +386,296 @@ int launch_conv_wgrad_tc(const WgradGeom& wg, const void* x, const void* dy, flo
   return B3D_OK;
 }
 
+// ================================================== narrow layers: the tap-stacked operand built in shared memory
+// Weight gradient of a stride-1 k in {1, 3} layer with Cn < 8 channels on one side (the 2-channel input volume, the
+// 2-3 channel gradients of the output convs): the GEMM of the KS = 1 kernel above over the stacked operand of
+// cast_stack_bf16_kernel (rows (tap, c) = the narrow tensor shifted by sgn * (tap - pad), zero-padded to a multiple of 8
+// rows; K = voxels), but the stacked operand never goes through global memory.  Per stage:
+//   * warp 0 fetches the B planes (the wide tensor's bf16 P16 twin) by TMA;
+//   * warps 2..7 read the fp32 narrow tensor (a few bytes per voxel; the tile's halo stays in L1) and store the stacked
+//     bf16 cells straight into the MN-major plane layout of the A operand, then arrive on the stage's barrier.  A thread
+//     builds every row of one voxel; K and Cn are template parameters, so each row's tap, channel and shift are
+//     compile-time constants (rows in the order of cast_stack_bf16_kernel, the same RN rounding to bf16);
+//   * warp 1 issues the MMAs (M = 64 | 128 stacked rows, N = the wide channels), warps 4..7 reduce the partial dw.
+// Roles of the narrow tensor:
+//   * layer input x (sgn = +1): rows (tap, ci), columns co -> dw[tap][ci][co].  A second B tile (dres, the gradient of
+//     the pointwise conv reading the same x) doubles N; its columns against the centre-tap rows are that layer's dw;
+//   * output gradient dy (sgn = -1, dw[t][ci][co] = sum_u x[u][ci] dy[u - (t - pad)][co]): rows (tap, co), columns ci,
+//     written transposed to dw[tap][ci][co]; the column sums of dy (bias gradient) come out of the tile build.
+struct NwParams {
+  const float* nar;                // fp32 narrow tensor [B, D, H, W, pitch]
+  long long pitch;
+  float* dw;
+  float* dw2;                      // != nullptr: dw [Cn][Cw] of the pointwise conv (B columns Cw..2Cw-1 = dres)
+  float* dbias;                    // != nullptr (narrow dy): += column sums of dy
+  int B, D, H, W;
+  int Cn, sgn, rows, planes;       // rows = k^3 * Cn real stacked rows in `planes` octets
+  int tr;                          // 1: the narrow tensor is dy
+  int Cw, NT, M, tmem_cols, centre;
+  int TD, TH, TW, px, stage_bytes, nstages;
+  int ntd, nth, ntw, ntiles, nsplit;
+};
+
+constexpr int kNwBuilders = 6;                       // warps 2..7
+
+template <int K, int CN>
+__global__ void __launch_bounds__(256, 1)
+    conv_wgrad_narrow_kernel(const __grid_constant__ WgMaps maps, const NwParams prm) {
+  constexpr int ROWS = K * K * K * CN, PLANES = (ROWS + 7) / 8, PAD = K / 2, CENTRE = (K * K * K) / 2;
+  pdl_trigger();
+  extern __shared__ __align__(1024) uint8_t smem[];
+  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + kWgSmem - 128);
+  uint64_t* full = bars;        // [4]
+  uint64_t* empty = bars + 4;   // [4]
+  uint64_t* done = bars + 8;
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 9);
+
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int vox = prm.TD * prm.TH * prm.TW;
+  if (threadIdx.x == 0) {
+    for (int i = 0; i < prm.nstages; ++i) {
+      mbar_init(smem_u32(&full[i]), 1 + kNwBuilders);
+      mbar_init(smem_u32(&empty[i]), 1);
+    }
+    mbar_init(smem_u32(done), 1);
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+  }
+  if (warp == 2) {
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)),
+                 "r"(prm.tmem_cols));
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
+  }
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem_base = *tmem_slot;
+  const int yplanes = prm.NT / 8, wplanes = prm.Cw / 8;
+
+  if (warp == 0) {
+    if (lane == 0) {
+      int s = 0, ph = 0;
+      for (int tile = blockIdx.x; tile < prm.ntiles; tile += prm.nsplit) {
+        int t = tile;
+        const int w0 = (t % prm.ntw) * prm.TW; t /= prm.ntw;
+        const int h0 = (t % prm.nth) * prm.TH; t /= prm.nth;
+        const int d0 = (t % prm.ntd) * prm.TD;
+        const int b = t / prm.ntd;
+        mbar_wait(smem_u32(&empty[s]), ph ^ 1);
+        const uint32_t fb = smem_u32(&full[s]);
+        mbar_expect_tx(fb, (uint32_t)(yplanes * vox * 16));
+        const uint32_t ydst = smem_u32(smem + (size_t)s * prm.stage_bytes + (size_t)prm.planes * prm.px);
+        for (int q = 0; q < yplanes; ++q)
+          tma_load_5d(ydst + q * vox * 16, q < wplanes ? &maps.y : &maps.y2, 4 * w0, q < wplanes ? q : q - wplanes, h0,
+                      d0, b, fb);
+        if (++s == prm.nstages) { s = 0; ph ^= 1; }
+      }
+    }
+  } else if (warp == 1) {
+    const bool leader = elect_one();
+    // D=f32, A=B=bf16, both MN-major
+    const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | (1u << 15) | (1u << 16) |
+                           ((uint32_t)(prm.NT >> 3) << 17) | (((uint32_t)prm.M >> 4) << 24);
+    int s = 0, ph = 0;
+    uint32_t acc = 0;
+    for (int tile = blockIdx.x; tile < prm.ntiles; tile += prm.nsplit) {
+      mbar_wait(smem_u32(&full[s]), ph);
+      tc_fence_after();
+      const uint32_t xaddr = smem_u32(smem) + (uint32_t)s * (uint32_t)prm.stage_bytes;
+      // K = 16 voxels per MMA: 8 along w (16 B apart) x 2 h rows (LBO = row pitch)
+      const uint64_t adesc0 = make_desc(xaddr, (uint32_t)prm.TW * 16, (uint32_t)prm.px);
+      const uint64_t bdesc0 = make_desc(xaddr + (uint32_t)(prm.planes * prm.px), (uint32_t)prm.TW * 16, (uint32_t)vox * 16);
+      for (int cell = 0; cell < vox; cell += 2 * prm.TW)
+        for (int w8 = 0; w8 < prm.TW; w8 += 8) {
+          if (leader) tc_mma_bf16(tmem_base, adesc0 + cell + w8, bdesc0 + cell + w8, idesc, acc);
+          acc = 1;
+        }
+      if (leader) tc_commit(smem_u32(&empty[s]));
+      __syncwarp();
+      if (++s == prm.nstages) { s = 0; ph ^= 1; }
+    }
+    if (leader) tc_commit(smem_u32(done));
+    __syncwarp();
+  } else {
+    // builders: thread -> voxel (all its rows), consecutive lanes on consecutive voxels (16-byte stores side by side)
+    const int bt = threadIdx.x - 64;
+    const long long sw = prm.pitch, sh = sw * prm.W, sd = sh * prm.H;
+    float bsum[CN];
+#pragma unroll
+    for (int c = 0; c < CN; ++c) bsum[c] = 0.f;
+    int s = 0, ph = 0;
+    for (int tile = blockIdx.x; tile < prm.ntiles; tile += prm.nsplit) {
+      int t = tile;
+      const int w0 = (t % prm.ntw) * prm.TW; t /= prm.ntw;
+      const int h0 = (t % prm.nth) * prm.TH; t /= prm.nth;
+      const int d0 = (t % prm.ntd) * prm.TD;
+      const int b = t / prm.ntd;
+      mbar_wait(smem_u32(&empty[s]), ph ^ 1);
+      uint8_t* xs = smem + (size_t)s * prm.stage_bytes;
+      for (int vl = bt; vl < vox; vl += 32 * kNwBuilders) {
+        const int d = d0 + vl / (prm.TW * prm.TH), h = h0 + (vl / prm.TW) % prm.TH, w = w0 + vl % prm.TW;
+        const bool in = d < prm.D && h < prm.H && w < prm.W;
+        // per dimension and tap index j: the element offset of the shift sgn * (j - PAD), and whether it stays inside
+        long long od[K], oh[K], ow[K];
+        bool okd[K], okh[K], okw[K];
+#pragma unroll
+        for (int j = 0; j < K; ++j) {
+          const int q = prm.sgn * (j - PAD);
+          od[j] = q * sd; oh[j] = q * sh; ow[j] = q * sw;
+          okd[j] = in && d + q >= 0 && d + q < prm.D;
+          okh[j] = h + q >= 0 && h + q < prm.H;
+          okw[j] = w + q >= 0 && w + q < prm.W;
+        }
+        const float* base = prm.nar + ((((long long)b * prm.D + d) * prm.H + h) * prm.W + w) * sw;
+#pragma unroll
+        for (int p = 0; p < PLANES; ++p) {
+          float v[8];
+#pragma unroll
+          for (int e = 0; e < 8; ++e) {
+            const int row = p * 8 + e, tap = row / CN, c = row % CN;
+            const int kd = tap / (K * K), kh = (tap / K) % K, kw = tap % K;
+            v[e] = 0.f;
+            if (row < ROWS && okd[kd] && okh[kh] && okw[kw]) v[e] = __ldg(base + od[kd] + oh[kh] + ow[kw] + c);
+            if (row < ROWS && tap == CENTRE) bsum[c] += v[e];      // the voxel itself (0 outside the volume)
+          }
+          uint4 o;
+          asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(o.x) : "f"(v[1]), "f"(v[0]));
+          asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(o.y) : "f"(v[3]), "f"(v[2]));
+          asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(o.z) : "f"(v[5]), "f"(v[4]));
+          asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(o.w) : "f"(v[7]), "f"(v[6]));
+          *reinterpret_cast<uint4*>(xs + (size_t)p * prm.px + (size_t)vl * 16) = o;
+        }
+      }
+      asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // generic-proxy stores -> UMMA reads
+      __syncwarp();
+      if (lane == 0) mbar_arrive(smem_u32(&full[s]));
+      if (++s == prm.nstages) { s = 0; ph ^= 1; }
+    }
+    if (prm.dbias != nullptr) {
+#pragma unroll
+      for (int c = 0; c < CN; ++c) {
+        float x = bsum[c];
+        for (int o = 16; o > 0; o >>= 1) x += __shfl_xor_sync(0xffffffffu, x, o);
+        if (lane == 0 && blockIdx.x < prm.ntiles) atomicAdd(prm.dbias + c, x);
+      }
+    }
+    if (warp >= 4) {
+      // final reduction of this CTA's partial dw (rows: see the KS = 1 kernel above; one tap, all taps are rows here)
+      const int q = warp - 4;
+      mbar_wait(smem_u32(done), 0);
+      tc_fence_after();
+      const int pitch = prm.NT + 4, c4n = prm.NT / 4;
+      float* stg = reinterpret_cast<float*>(smem) + q * 32 * pitch;
+      for (int j = 0; j < prm.NT; j += 16) {
+        float r[16];
+        tc_ld16(tmem_base + ((uint32_t)(q * 32) << 16) + j, r);
+#pragma unroll
+        for (int i = 0; i < 16; i += 4)
+          *reinterpret_cast<float4*>(stg + lane * pitch + j + i) = make_float4(r[i], r[i + 1], r[i + 2], r[i + 3]);
+      }
+      __syncwarp();
+      const int nel = prm.tr ? 32 * prm.NT : 32 * c4n;
+      for (int e = lane; blockIdx.x < prm.ntiles && e < nel; e += 32) {
+        const int rl = prm.tr ? e / prm.NT : e / c4n, c = prm.tr ? e - rl * prm.NT : (e - rl * c4n) * 4;
+        const int row = prm.M == 128 ? q * 32 + rl : (rl < 16 ? q * 16 + rl : prm.rows);
+        if (row >= prm.rows) continue;
+        const int t = row / prm.Cn, cc = row - t * prm.Cn;
+        const float* src = stg + rl * pitch + c;
+        if (prm.tr) {
+          atomicAdd(prm.dw + ((size_t)t * prm.Cw + c) * prm.Cn + cc, *src);
+        } else if (c < prm.Cw) {
+          atomicAdd(reinterpret_cast<float4*>(prm.dw + (size_t)row * prm.Cw + c), *reinterpret_cast<const float4*>(src));
+        } else if (t == prm.centre) {
+          atomicAdd(reinterpret_cast<float4*>(prm.dw2 + (size_t)cc * prm.Cw + c - prm.Cw),
+                    *reinterpret_cast<const float4*>(src));
+        }
+      }
+    }
+  }
+  tc_fence_before();
+  __syncthreads();
+  if (warp == 2) {
+    tc_fence_after();
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(prm.tmem_cols));
+  }
+}
+
+bool tc_wgrad_narrow_supported(int k, int cin, int cout, int pair) {
+  const bool nx = cin >= 1 && cin < 8 && cout >= 16 && cout % 16 == 0;
+  const bool ny = cout >= 1 && cout < 8 && cin >= 16 && cin % 16 == 0;
+  if ((k != 1 && k != 3) || !(nx || ny) || (pair && !nx)) return false;
+  const int cn = nx ? cin : cout, cw = nx ? cout : cin;
+  return (k * k * k * cn + 7) / 8 * 8 <= 128 && (pair ? 2 : 1) * cw <= 256;
+}
+
+int launch_conv_wgrad_narrow(const NarrowWgrad& a, cudaStream_t s) {
+  const int cin = a.tr ? a.Cw : a.Cn, cout = a.tr ? a.Cn : a.Cw;
+  B3D_REQUIRE(tc_wgrad_narrow_supported(a.k, cin, cout, a.wide2 != nullptr), B3D_ERR_UNSUPPORTED,
+              "wgrad (narrow): layer not on this path (k=%d %d->%d)", a.k, cin, cout);
+  B3D_REQUIRE((((uintptr_t)a.wide | (uintptr_t)a.wide2 | (uintptr_t)a.dw | (uintptr_t)a.dw2) & 15) == 0, B3D_ERR_LAYOUT,
+              "wgrad (narrow): 16-byte alignment");
+  NwParams p;
+  memset(&p, 0, sizeof(p));
+  p.nar = a.nar; p.pitch = a.pitch; p.dw = a.dw; p.dw2 = a.dw2; p.dbias = a.dbias;
+  p.B = a.B; p.D = a.D; p.H = a.H; p.W = a.W;
+  p.Cn = a.Cn; p.sgn = a.tr ? -1 : 1; p.tr = a.tr; p.Cw = a.Cw;
+  p.rows = a.k * a.k * a.k * a.Cn; p.planes = (p.rows + 7) / 8;
+  p.M = p.planes <= 8 ? 64 : 128;
+  p.NT = a.wide2 != nullptr ? 2 * a.Cw : a.Cw;
+  p.tmem_cols = 32;
+  while (p.tmem_cols < p.NT) p.tmem_cols *= 2;
+  p.centre = (a.k * a.k * a.k) / 2;
+  // tile planner (as launch_conv_wgrad_tc): largest tile whose stages fit, with M/8 MN groups readable from every stage
+  static const int cand[][3] = {{1, 4, 8},  {2, 4, 8},  {2, 4, 16}, {2, 8, 16},
+                                {4, 8, 16}, {4, 8, 32}, {4, 16, 32}};
+  const int budget = kWgSmem - 128;
+  bool found = false;
+  for (int i = 0; i < (int)(sizeof(cand) / sizeof(cand[0])); ++i) {
+    const int TD = cand[i][0], TH = cand[i][1], TW = cand[i][2];
+    if (found && (TD > a.D * 2 || TH > a.H * 2 || TW > a.W * 2)) continue;
+    const int px = TD * TH * TW * 16;
+    const long long stage = (long long)(p.planes + p.NT / 8) * px;
+    for (int ns = 3; ns >= 2; --ns) {
+      if (ns * stage <= budget && (ns - 1) * stage + (long long)(p.M / 8) * px <= budget) {
+        p.TD = TD; p.TH = TH; p.TW = TW; p.px = px; p.stage_bytes = (int)stage; p.nstages = ns;
+        found = true;
+        break;
+      }
+    }
+  }
+  B3D_REQUIRE(found, B3D_ERR_UNSUPPORTED, "wgrad (narrow): no tile fits shared memory");
+  p.ntd = (a.D + p.TD - 1) / p.TD; p.nth = (a.H + p.TH - 1) / p.TH; p.ntw = (a.W + p.TW - 1) / p.TW;
+  p.ntiles = a.B * p.ntd * p.nth * p.ntw;
+  p.nsplit = sm_count() < p.ntiles ? sm_count() : p.ntiles;
+  WgMaps maps;
+  memset(&maps, 0, sizeof(maps));
+  B3D_TRY(make_p16_map(&maps.y, a.wide, 1, a.B, a.D, a.H, a.W, a.Cw / 8, p.TW, 1, p.TH, p.TD));
+  if (a.wide2 != nullptr) B3D_TRY(make_p16_map(&maps.y2, a.wide2, 1, a.B, a.D, a.H, a.W, a.Cw / 8, p.TW, 1, p.TH, p.TD));
+  B3D_TRY(cuda_ok(cudaMemsetAsync(a.dw, 0, sizeof(float) * (size_t)p.rows * a.Cw, s), "memset dw"));
+  if (a.dw2 != nullptr) B3D_TRY(cuda_ok(cudaMemsetAsync(a.dw2, 0, sizeof(float) * (size_t)a.Cn * a.Cw, s), "memset dw2"));
+  if (a.dbias != nullptr) B3D_TRY(cuda_ok(cudaMemsetAsync(a.dbias, 0, sizeof(float) * (size_t)a.Cn, s), "memset dbias"));
+  const dim3 grid((unsigned)p.nsplit);
+#define LAUNCH(K, CN)                                                                                          \
+  case K * 8 + CN: {                                                                                           \
+    static bool attr = false;                                                                                  \
+    if (!attr) {                                                                                               \
+      B3D_TRY(cuda_ok(cudaFuncSetAttribute(conv_wgrad_narrow_kernel<K, CN>,                                     \
+                                           cudaFuncAttributeMaxDynamicSharedMemorySize, kWgSmem),             \
+                      "cudaFuncSetAttribute(wgrad_narrow)"));                                                  \
+      attr = true;                                                                                             \
+    }                                                                                                          \
+    conv_wgrad_narrow_kernel<K, CN><<<grid, 256, kWgSmem, s>>>(maps, p);                                       \
+    break;                                                                                                     \
+  }
+  switch (a.k * 8 + a.Cn) {   // tc_wgrad_narrow_supported: k = 3 takes Cn <= 4 (27 Cn rows <= 128), k = 1 any Cn < 8
+    LAUNCH(1, 1) LAUNCH(1, 2) LAUNCH(1, 3) LAUNCH(1, 4) LAUNCH(1, 5) LAUNCH(1, 6) LAUNCH(1, 7)
+    LAUNCH(3, 1) LAUNCH(3, 2) LAUNCH(3, 3) LAUNCH(3, 4)
+    default: B3D_REQUIRE(false, B3D_ERR_UNSUPPORTED, "wgrad (narrow): k=%d Cn=%d", a.k, a.Cn);
+  }
+#undef LAUNCH
+  B3D_LAUNCH_CHECK("conv_wgrad_narrow");
+  return B3D_OK;
+}
+
 
 // ================================================================================ kd folded into M, kw folded into N
 // For Cin = 32 / 64 the kernel above computes M = 64 / 128 rows per MMA of which Cin are real, 27 MMAs per K step.  Here

@@ -39,7 +39,6 @@ class Decoder(Layer):
             conv = ResnetBlock(filters=base_filters * (2 ** i), groups=groups, reduction=reduction,
                                data_format=data_format, l2_scale=l2_scale)
             self.levels.append([upsample, res, conv])
-        self.levels[-1][2].keep_f32_output = True      # feeds the out_ch-channel output conv
 
         # 1x1x1 conv to the class channels + sigmoid (glorot_normal, L2)
         self.out = Conv3D(filters=out_ch, kernel_size=1, strides=1, padding='same', activation='sigmoid',

@@ -36,9 +36,6 @@ class ResnetBlock(Layer):
                             'groups': groups})
         self.filters, self.groups = filters, groups
         self.data_format = data_format
-        # set by Decoder / VariationalAutoencoder on the block whose output feeds a narrow (2-3 channel) output conv: that
-        # conv's weight gradient takes fp32 operands, so the output is kept in fp32 next to its 16-bit twin
-        self.keep_f32_output = False
         self._fused_stats = data_format == 'channels_last'     # chunk statistics from the conv epilogue (F1 only)
 
         self.conv3d_ptwise = Conv3D(filters=filters, kernel_size=1, strides=1, padding='same',
@@ -99,11 +96,9 @@ class ResnetBlock(Layer):
         if st2 is None:                                   # chunk boundaries not voxel-aligned: unfused GN2
             a2 = norm2.call(h2, relu=True)
             return ops.block_epilogue(res, a2, None, None, None, self.spatial.kernel, gap,
-                                      self.dense_relu.kernel, self.dense_sigmoid.kernel, self.groups, norm2.epsilon,
-                                      keep_f32=self.keep_f32_output)
+                                      self.dense_relu.kernel, self.dense_sigmoid.kernel, self.groups, norm2.epsilon)
         return ops.block_epilogue(res, h2, st2, norm2.gamma, norm2.beta, self.spatial.kernel, gap,
-                                  self.dense_relu.kernel, self.dense_sigmoid.kernel, self.groups, norm2.epsilon,
-                                  keep_f32=self.keep_f32_output)
+                                  self.dense_relu.kernel, self.dense_sigmoid.kernel, self.groups, norm2.epsilon)
 
     def get_config(self):
         return self.config

@@ -62,7 +62,6 @@ class VariationalAutoencoder(Layer):
             conv = ResnetBlock(filters=base_filters * (2 ** i), groups=groups, reduction=reduction,
                                data_format=data_format, l2_scale=l2_scale)
             self.levels.append([upsample, conv])
-        self.levels[-1][1].keep_f32_output = True      # feeds the out_ch-channel output conv
 
         self.out = Conv3D(filters=out_ch, kernel_size=3, strides=1, padding='same', data_format=data_format,
                           kernel_regularizer=L2(l2_scale), kernel_initializer='he_normal')

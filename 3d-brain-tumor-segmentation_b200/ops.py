@@ -497,12 +497,18 @@ class Conv3dFn(Function):
         # it tells that kernel's backward which bias to write the column sums of dy into and whether this conv's
         # backward can work from a bf16 twin of dy alone, and carries the twin / bias gradient back to this conv's
         # backward.  (Python attributes on the gradient tensors themselves do not survive the autograd engine.)
-        f32_grad = not (ctx.srcs_w is not None and twin_dtype(True) == torch.bfloat16 and lib.b3d_conv3d_wgrad_p16_plan(
-            k, stride, int(transposed), Cin, Cout, od[2]) != 0)
+        # narrow layers (fewer than 8 channels on one side): weight gradient from the fp32 narrow tensor and the bf16
+        # twin of the wide one (b3d_conv3d_wgrad_narrow); a narrow output needs the input's twin, a narrow input has none
+        ctx.narrow = bool(stride == 1 and not transposed and twin_dtype(True) == torch.bfloat16 and
+                          lib.b3d_conv3d_wgrad_narrow_ok(k, Cin, Cout, 0) and
+                          (Cin < 8 or (ctx.srcs_w is not None and len(ctx.srcs_w) == 1)))
+        f32_grad = not (ctx.narrow or (ctx.srcs_w is not None and twin_dtype(True) == torch.bfloat16 and
+                                       lib.b3d_conv3d_wgrad_p16_plan(k, stride, int(transposed), Cin, Cout, od[2]) != 0))
         ctx.mb = y._b3d_mb = {"bias": bias, "f32_grad": f32_grad}
         if grad_box is not None and k == 1 and stride == 1 and not transposed:
             # the block's pointwise conv: the 3x3x3 conv reading the same x may compute its dx and dw (backward below)
-            grad_box["pw"] = {"mb": ctx.mb, "w": w, "srcs_w": ctx.srcs_w}
+            grad_box["pw"] = {"mb": ctx.mb, "w": w, "srcs_w": ctx.srcs_w,
+                              "x": (x.data_ptr(), tuple(x.shape)) if ctx.narrow and Cin < 8 else None}
         outs = (y, stats, gap)
         ctx.mark_non_differentiable(*[t for t in (stats, gap) if t is not None])
         return outs
@@ -544,7 +550,8 @@ class Conv3dFn(Function):
             else:
                 db, db_direct = _grad_target(pb)
         bias_done = dbias is not None
-        if dy16 is None and td is not None and p16_ok(dy.shape) and (plan or (tcd and is_virtual(dy))):
+        narrow = bool(need_dw and ctx.narrow and td == torch.bfloat16)
+        if dy16 is None and td is not None and p16_ok(dy.shape) and (plan or (narrow and cin < 8) or (tcd and is_virtual(dy))):
             # no twin came with the gradient (several consumers were summed by autograd, or a fp32 producer): one packing
             # pass serves the data gradient and the weight gradient and yields the bias gradient on the way
             dy16 = to_p16(materialize(dy), td, db if (need_dw and has_bias and not bias_done) else None)
@@ -625,7 +632,14 @@ class Conv3dFn(Function):
             # (csrc/conv_tc_wgrad.cu) the pointwise layer's dw is one more MMA per K step over the x tile already in
             # shared memory (b3d_conv3d_wgrad_p16_block) instead of a second pass over x
             fuse_w = None
-            if (plan and dy16 is not None and pwbox is not None and pwbox["mb"] is not mb
+            if (narrow and cin < 8 and dy16 is not None and pwbox is not None and pwbox["mb"] is not mb
+                    and not pwbox.get("done") and k == 3 and pwbox["w"].requires_grad
+                    and pwbox.get("x") == (x.data_ptr(), tuple(x.shape))):
+                dres16 = pwbox["mb"].get("dy16")
+                if dres16 is not None and dres16.dtype == dy16.dtype and tuple(dres16.shape) == tuple(dy16.shape) and \
+                        lib.b3d_conv3d_wgrad_narrow_ok(k, cin, cout, 1):
+                    fuse_w = dres16
+            elif (plan and dy16 is not None and pwbox is not None and pwbox["mb"] is not mb
                     and not pwbox.get("done") and k == 3 and stride == 1 and not transposed
                     and pwbox["w"].requires_grad and _same_sources(pwbox.get("srcs_w"), srcs_w)):
                 dres16 = pwbox["mb"].get("dy16")
@@ -635,10 +649,25 @@ class Conv3dFn(Function):
             if fuse_w is not None:
                 dwp, dwp_direct = _grad_target(pwbox["w"])
                 _tag_conv(w, ctx.nv, stride, transposed)
-                _call("b3d_conv3d_wgrad_p16_block", *_pad4(srcs_w), dy16, fuse_w, dw, dwp)
+                if narrow:
+                    _call("b3d_conv3d_wgrad_narrow", x, dy16, fuse_w, dw, dwp, None)
+                else:
+                    _call("b3d_conv3d_wgrad_p16_block", *_pad4(srcs_w), dy16, fuse_w, dw, dwp)
                 pwbox["dw"] = (dwp, dwp_direct)
                 if has_bias and not bias_done:
                     _call("b3d_colsum", materialize(dy), db)
+            elif narrow and cin < 8 and dy16 is not None:
+                # narrow input (the image): x is the real fp32 tensor, dy comes as its bf16 twin
+                _tag_conv(w, ctx.nv, stride, transposed)
+                _call("b3d_conv3d_wgrad_narrow", x, dy16, None, dw, None, None)
+                if has_bias and not bias_done:
+                    _call("b3d_colsum", materialize(dy), db)
+            elif narrow and cout < 8:
+                # narrow output (the output convs): dy is fp32 and yields the bias gradient in the same pass
+                _tag_conv(w, ctx.nv, stride, transposed)
+                _call("b3d_conv3d_wgrad_narrow", materialize(dy), srcs_w[0], None, dw, None,
+                      db if (has_bias and not bias_done) else None)
+                bias_done = True
             elif plan and dy16 is not None:
                 scratch = None
                 if plan == 2:
@@ -994,12 +1023,11 @@ class BlockEpilogueFn(Function):
                 None if dw2_direct else dw2, None, None, None, None)
 
 
-def block_epilogue(res, h2, stats2, gamma2, beta2, wsp, gap_sum, w1, w2, groups=8, eps=1e-5, keep_f32=False):
+def block_epilogue(res, h2, stats2, gamma2, beta2, wsp, gap_sum, w1, w2, groups=8, eps=1e-5):
     sctx = _slab.current()
     if sctx is not None and sctx.p16 is not None and p16_ok(res.shape):
-        return sctx.block_epilogue(res, h2, stats2, gamma2, beta2, wsp, gap_sum, w1, w2, groups, eps,
-                                   keep_f32 or not FUSED["on"])
-    operand_only = FUSED["on"] and sctx is None and not keep_f32
+        return sctx.block_epilogue(res, h2, stats2, gamma2, beta2, wsp, gap_sum, w1, w2, groups, eps, not FUSED["on"])
+    operand_only = FUSED["on"] and sctx is None
     out, out16, out16b = BlockEpilogueFn.apply(res, h2, stats2, gamma2, beta2, wsp, gap_sum, w1, w2, groups, eps,
                                                operand_only, torch.is_grad_enabled())
     if out16 is not None and not is_virtual(out):

@@ -375,6 +375,17 @@ int b3d_conv3d_wgrad_p16_block(const DLTensor* x0, const DLTensor* x1, const DLT
                                const DLTensor* dy /*P16*/, const DLTensor* dres /*P16*/, DLTensor* dw, DLTensor* dw_pw,
                                void* stream);
 int b3d_conv3d_wgrad_p16_block_ok(int cin, int cout, int h_sp, int w_sp);
+/* weight gradient of a stride-1 k in {1, 3} conv with fewer than 8 channels on one side, the tap-stacked operand of the
+ * narrow fp32 tensor built in shared memory (no staged copy in global memory).  nar: fp32 NDHWC, Cn < 8 channels;
+ * wide: bf16 P16 twin with Cw channels.  Which tensor is which follows from dw:
+ *   dw (k,k,k,Cn,Cw): nar = the layer input x, wide = dy.  dres / dw_pw (nullable, together): the gradient of the
+ *     pointwise conv reading the same x and that conv's dw (1,1,1,Cn,Cw), computed in the same pass;
+ *   dw (k,k,k,Cw,Cn): nar = dy, wide = x.  dbias (nullable) receives the column sums of dy.
+ * Layers it takes (else B3D_ERR_UNSUPPORTED): k in {1, 3}; Cn in 1..7 with pad8(k^3 * Cn) <= 128; Cw a multiple of 16
+ * with Cw (2 Cw with dres) <= 256.  The library also exports the host-side query of these rules,
+ *   int b3d_conv3d_wgrad_narrow_ok(int k, int cin, int cout, int pair)   (1: taken; pair: with dres / dw_pw). */
+int b3d_conv3d_wgrad_narrow(const DLTensor* nar, const DLTensor* wide /*P16*/, const DLTensor* dres /*P16*/,
+                            DLTensor* dw, DLTensor* dw_pw, DLTensor* dbias, void* stream);
 /* 0: the layer's weight gradient is not on the P16 path; 1: straight from the operands; 2: needs a 16-bit scratch of
  * numel(big tensor) elements (stride-2 family); 3: of numel(dy) elements (TS-mode kernel).  w_sp = W of dy. */
 int b3d_conv3d_wgrad_p16_plan(int k, int stride, int transposed, int cin, int cout, int w_sp);
